@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port, host cores)
     python bench.py --config {1,2,3,4,5} ...                 # pick the BASELINE.json configuration
+    python bench.py ... --dump-outputs DIR                   # also save the main line's last timed step (.npy)
 
 Default workload = BASELINE.json configs[2] ("config3", the largest single-GPU configuration):
 LENS architecture I=100 -> F=200 -> P=10 000 places, random-init weights with trained statistics,
@@ -70,7 +71,14 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="main configuration only")
     ap.add_argument("--extras", default="1,2,4,5", help="configurations measured beside the main one")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the main line's last timed step returned as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm times a bounded sample on the host)")
+    return args
 
 
 def resolve(args, config=None, world=1):
@@ -297,6 +305,41 @@ def emit(line):
     out.flush()
 
 
+DUMP_BYTES = 60 << 20          # array data of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(directory, arrays, budget=DUMP_BYTES):
+    """Write the tensors one step of the timed path returned (name -> tensor) as DIR/<name>.npy, so that two
+    builds run with the same arguments can be compared output for output.
+
+    Values are float32 where that is exact (float32, integers of up to 16 bits, bool) and float64 otherwise.
+    Arrays of two or more dimensions share their leading dimension (streams, or event windows); when they do
+    not fit in `budget` bytes, the same fixed, seeded sample of those rows is written for each of them.
+    DIR/sample_rows.npy lists the rows written."""
+    import math
+    import torch
+    exact32 = (torch.float32, torch.uint8, torch.int8, torch.int16, torch.bool)
+
+    def dtype(t):
+        return np.dtype(np.float32 if t.dtype in exact32 else np.float64)
+    whole = {k: t for k, t in arrays.items() if t.dim() < 2}
+    rowed = {k: t for k, t in arrays.items() if t.dim() >= 2}
+    lead = {t.shape[0] for t in rowed.values()}
+    assert len(lead) <= 1, "arrays of two or more dimensions must share their leading dimension"
+    n = lead.pop() if lead else 0
+    fixed = sum(t.numel() * dtype(t).itemsize for t in whole.values())
+    per_row = 8 + sum(math.prod(t.shape[1:]) * dtype(t).itemsize for t in rowed.values())
+    keep = min(n, (budget - fixed) // per_row)
+    rows = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    for k, t in whole.items():
+        np.save(os.path.join(directory, k + ".npy"), t.cpu().numpy().astype(dtype(t)))
+    for k, t in rowed.items():
+        picked = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        np.save(os.path.join(directory, k + ".npy"), picked.cpu().numpy().astype(dtype(t)))
+    np.save(os.path.join(directory, "sample_rows.npy"), rows.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 class Ctx:
     """torch / distributed state shared by the measurements."""
@@ -324,16 +367,18 @@ class Ctx:
         self.torch.cuda.synchronize()
 
     def timed(self, fn, steps):
-        """CUDA events on the launching (current) stream around every call; L2 flushed in between."""
+        """CUDA events on the launching (current) stream around every call; L2 flushed in between.
+        -> (ms per call, what the last call returned)."""
         torch = self.torch
-        evs = []
+        evs, out = [], None
         for _ in range(steps):
+            out = None                  # free the previous call's outputs before this call allocates its own
             self.flush.zero_()
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            a.record(); fn(); b.record()
+            a.record(); out = fn(); b.record()
             evs.append((a, b))
         torch.cuda.synchronize()
-        return [a.elapsed_time(b) for a, b in evs]
+        return [a.elapsed_time(b) for a, b in evs], out
 
     def max_over_ranks(self, *vals):
         t = self.torch.tensor(list(vals), dtype=self.torch.float64, device=self.dev)
@@ -342,8 +387,9 @@ class Ctx:
         return t.tolist()
 
 
-def measure_snn(ctx, c, steps, warmup, W_out_sharded=False, want_e2e=True):
-    """One SNN + matching configuration: resident and host-fed throughput, per-kernel rooflines."""
+def measure_snn(ctx, c, steps, warmup, W_out_sharded=False, want_e2e=True, dump=None):
+    """One SNN + matching configuration: resident and host-fed throughput, per-kernel rooflines.
+    `dump`: directory for what the last timed resident step returned (this rank's streams)."""
     torch, dist = ctx.torch, ctx.dist
     from lens_b200 import synth, _lib
     from lens_b200.pipeline import InferencePipeline
@@ -361,7 +407,7 @@ def measure_snn(ctx, c, steps, warmup, W_out_sharded=False, want_e2e=True):
         for _ in range(2):
             dist.all_gather_into_tensor(full, shard)
         ctx.barrier()
-        ag = ctx.timed(lambda: dist.all_gather_into_tensor(full, shard), 5)
+        ag, _ = ctx.timed(lambda: dist.all_gather_into_tensor(full, shard), 5)
         ag_ms, = ctx.max_over_ranks(float(np.mean(ag)))
         res["all_gather"] = dict(bytes=int(full.numel() * 4), ms=ag_ms,
                                  algbw_GBps=full.numel() * 4 / (ag_ms / 1e3) / 1e9, collective="ncclAllGather (W_out rows)")
@@ -401,17 +447,20 @@ def measure_snn(ctx, c, steps, warmup, W_out_sharded=False, want_e2e=True):
     pipe.stage_timing = True
     launches0 = _lib.launch_count()
     ctx.barrier()
-    ms = ctx.timed(step_resident, steps)
+    ms, out = ctx.timed(step_resident, steps)
     ctx.barrier()
     launches = _lib.launch_count() - launches0
     ktime = pipe.net.get_timing()
     stage = pipe.pop_stage_timing()
     pipe.net.set_timing(False)
     pipe.stage_timing = False
+    if dump:
+        dump_outputs(dump, {k: v for k, v in out.items() if v is not None})
+    del out
     ms_e2e = [0.0]
     if want_e2e:
         ctx.barrier()
-        ms_e2e = ctx.timed(step_e2e, steps)
+        ms_e2e, _ = ctx.timed(step_e2e, steps)
         ctx.barrier()
     last = step_resident()
     recall = pipe.recall(last["hits"], last["n_valid"])
@@ -422,7 +471,7 @@ def measure_snn(ctx, c, steps, warmup, W_out_sharded=False, want_e2e=True):
         allti = torch.empty((world,) + tuple(ti.shape), dtype=ti.dtype, device=dev)
         dist.all_gather_into_tensor(allti, ti)
         ctx.barrier()
-        tg = ctx.timed(lambda: dist.all_gather_into_tensor(allti, ti), 5)
+        tg, _ = ctx.timed(lambda: dist.all_gather_into_tensor(allti, ti), 5)
         tg_ms, = ctx.max_over_ranks(float(np.mean(tg)))
         res["topn_gather"] = dict(bytes=int(allti.numel() * 4), ms=tg_ms, collective="ncclAllGather (top-N indices)")
     del last
@@ -493,7 +542,7 @@ def measure_place_sharded(ctx, c, steps):
     for _ in range(3):
         out = pipe.step(frames=frames, gt_center=gt, gt_tol=2)
     ctx.barrier()
-    ms = ctx.timed(lambda: pipe.step(frames=frames, gt_center=gt, gt_tol=2), steps)
+    ms, _ = ctx.timed(lambda: pipe.step(frames=frames, gt_center=gt, gt_tol=2), steps)
     ctx.barrier()
     # the exchange alone: all-gather of (value, index) lists + merge
     tv, ti = out["top_val"].contiguous(), out["top_idx"].contiguous()
@@ -510,7 +559,7 @@ def measure_place_sharded(ctx, c, steps):
     for _ in range(3):
         exchange()
     ctx.barrier()
-    xms = ctx.timed(exchange, 5)
+    xms, _ = ctx.timed(exchange, 5)
     tot, xt = ctx.max_over_ranks(sum(ms), float(np.mean(xms)))
     del pipe, frames
     torch.cuda.empty_cache()
@@ -522,8 +571,9 @@ def measure_place_sharded(ctx, c, steps):
                 recall_at_n=dict(zip(map(str, NS), (out["hits"].double() / max(int(out["n_valid"].item()), 1)).tolist())))
 
 
-def measure_latency(ctx, c, reps=5):
-    """Config 1: ONE stream, serial chain of Q*T steps through the public batched call; us per step."""
+def measure_latency(ctx, c, reps=5, dump=None):
+    """Config 1: ONE stream, serial chain of Q*T steps through the public batched call; us per step.
+    `dump`: directory for what the last timed pass returned."""
     torch = ctx.torch
     from lens_b200 import synth
     from lens_b200.pipeline import InferencePipeline
@@ -536,15 +586,18 @@ def measure_latency(ctx, c, reps=5):
     # reduce=False: a single stream is "replicas only" (no collective; other ranks may not even be here)
     for _ in range(3):
         pipe.step(frames=frames, gt_center=gt, gt_tol=2, reduce=False)
-    ms = ctx.timed(lambda: pipe.step(frames=frames, gt_center=gt, gt_tol=2, reduce=False), reps)
+    ms, out = ctx.timed(lambda: pipe.step(frames=frames, gt_center=gt, gt_tol=2, reduce=False), reps)
+    if dump:
+        dump_outputs(dump, {k: v for k, v in out.items() if v is not None})
     best = float(np.min(ms))
     return dict(workload="%s: %s" % (c["name"], c["what"]), ms_per_pass=float(np.mean(ms)), ms_best=best,
                 serial_steps=Q * T_STEPS, us_per_step=float(np.mean(ms)) * 1e3 / (Q * T_STEPS),
                 value=Q * T_STEPS / (float(np.mean(ms)) / 1e3), unit="query_timesteps/s")
 
 
-def measure_binning(ctx, c, steps):
-    """Config 4: this rank's window-aligned shard of the event stream -> frames + pooled (K1)."""
+def measure_binning(ctx, c, steps, dump=None):
+    """Config 4: this rank's window-aligned shard of the event stream -> frames + pooled (K1).
+    `dump`: directory for what the last timed call returned."""
     torch = ctx.torch
     from lens_b200 import synth, ops
     world, dev, peaks = ctx.world, ctx.dev, ctx.peaks
@@ -557,8 +610,11 @@ def measure_binning(ctx, c, steps):
     for _ in range(3):
         bin_step()
     ctx.barrier()
-    bms = ctx.timed(bin_step, max(3, min(steps, 10)))
+    bms, out = ctx.timed(bin_step, steps)
     ctx.barrier()
+    if dump:
+        dump_outputs(dump, dict(zip(("frames", "pooled", "counts"), out)))
+    del out
     bsec, = ctx.max_over_ranks(float(np.mean(bms)))
     bsec /= 1e3
     out_bytes = n_win * (128 * 128 + I)
@@ -594,20 +650,21 @@ def main():
     if rank == 0:
         sampler.start()                      # samples through warm-up and the timed regions
 
+    dump = args.dump_outputs if rank == 0 else None
     if "places" not in c:                    # --config 4: binning is the main line
-        b = measure_binning(ctx, c, args.steps)
+        b = measure_binning(ctx, c, args.steps, dump=dump)
         line = dict(metric="events_per_sec", value=b["value"], unit="events/s", n_gpus=world, steps=args.steps,
                     warmup=max(args.warmup, 3), ms_per_step=b["ms"], higher_is_better=True, scaling=c["scaling"],
                     vs_baseline=None, dtype="u8+int32", data="synthetic", config=workload_config(c, world),
-                    roofline=b["roofline"], binning=b, gpu_launches=2 * max(3, min(args.steps, 10)))
+                    roofline=b["roofline"], binning=b, gpu_launches=2 * args.steps)
     elif c["name"] == "config1":
-        lat = measure_latency(ctx, c, reps=max(args.steps, 3))
+        lat = measure_latency(ctx, c, reps=args.steps, dump=dump)
         line = dict(metric="query_timesteps_per_sec", value=lat["value"], unit="query_timesteps/s", n_gpus=world,
                     steps=args.steps, warmup=max(args.warmup, 3), ms_per_step=lat["ms_per_pass"],
                     higher_is_better=True, scaling="replicas", vs_baseline=None, dtype="i8->i64+f32",
                     data="synthetic", config=workload_config(c, world), latency=lat)
     else:
-        m = measure_snn(ctx, c, args.steps, args.warmup, W_out_sharded=(c["name"] == "config5"))
+        m = measure_snn(ctx, c, args.steps, args.warmup, W_out_sharded=(c["name"] == "config5"), dump=dump)
         line = dict(metric="query_timesteps_per_sec", value=m.pop("value"), unit="query_timesteps/s", n_gpus=world,
                     steps=args.steps, warmup=max(args.warmup, 3), ms_per_step=m.pop("ms_per_step"),
                     higher_is_better=True, scaling=c["scaling"], vs_baseline=None, dtype="i8->i64+f32",

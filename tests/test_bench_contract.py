@@ -48,3 +48,43 @@ def test_config_table_matches_baseline_json():
     over = argparse.Namespace(config=3, streams=64, queries=None, places=500, seq_len=None, events=None)
     co = bench.resolve(over, world=1)
     assert co["overridden"] and "overridden" in bench.workload_config(co, 1)["workload"]
+
+
+def test_steps_must_be_positive():
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"],
+                         capture_output=True, text=True, timeout=120)
+    assert res.returncode == 2 and "--steps must be at least 1" in res.stderr
+
+
+def test_dump_outputs_writes_a_seeded_row_sample_within_budget(tmp_path):
+    """--dump-outputs: float32 / float64 files, the same rows of every per-stream array, the byte budget kept,
+    the whole array when it fits, and the same sample from call to call."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    g = torch.Generator().manual_seed(0)
+    B, Q, P, N = 300, 3, 40, 5
+    arrays = dict(S=torch.randint(0, 60, (B, Q, P), generator=g).float(),
+                  top_val=torch.rand((B, Q - 1, N), generator=g),
+                  top_idx=torch.randint(-1, P, (B, Q - 1, N), generator=g, dtype=torch.int32),
+                  hits=torch.tensor([5, 9, 11], dtype=torch.int64), n_valid=torch.tensor([17], dtype=torch.int64))
+    budget = 100_000
+    per_row = Q * P * 4 + (Q - 1) * N * (4 + 8) + 8
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, budget=budget)
+    got = {n: np.load(tmp_path / "a" / (n + ".npy")) for n in list(arrays) + ["sample_rows"]}
+    for n, a in got.items():
+        assert np.array_equal(a, np.load(tmp_path / "b" / (n + ".npy"))), n
+    assert got["S"].dtype == got["top_val"].dtype == np.float32
+    assert got["top_idx"].dtype == got["hits"].dtype == got["sample_rows"].dtype == np.float64
+    rows = got["sample_rows"].astype(np.int64)
+    assert len(rows) == (budget - 4 * 8) // per_row < B
+    assert np.all(np.diff(rows) > 0) and rows[0] >= 0 and rows[-1] < B
+    for n in ("S", "top_val", "top_idx"):
+        assert np.array_equal(got[n], arrays[n].numpy()[rows]), n
+    assert np.array_equal(got["hits"], [5, 9, 11]) and np.array_equal(got["n_valid"], [17])
+    assert sum(a.nbytes for a in got.values()) <= budget
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    assert np.array_equal(np.load(tmp_path / "whole" / "sample_rows.npy"), np.arange(B))
+    assert np.array_equal(np.load(tmp_path / "whole" / "S.npy"), arrays["S"].numpy())

@@ -1,5 +1,6 @@
 """GPU tests of the reference-facing Python API (LENS, run_inference, recallAtK) on the bundled
 example data (committed as fixtures by tests/golden/make_golden.py)."""
+import hashlib
 import os
 
 import numpy as np
@@ -237,7 +238,11 @@ def test_sad_baseline_matches_reference(golden):
         r = torch.from_numpy(g["ref_frames"].reshape(g["ref_frames"].shape[0], -1))
         D = sad_distance_matrix(q, r, L)
         sim = ops.reciprocal(D.contiguous()).cpu().numpy()
-        assert np.array_equal(sim, g["sad_sim"])
+        if "sad_sim" in g.files:
+            assert np.array_equal(sim, g["sad_sim"])
+        else:                   # a large matrix is stored as the SHA-256 of its float32 bytes (make_golden.py)
+            assert sim.dtype == np.float32 and sim.shape == g["D"].shape
+            assert hashlib.sha256(sim.tobytes()).hexdigest() == str(g["sad_sim_sha256"])
         P, R = createPR(sim, g["GTtol"], None, datatype="SAD", matching="single", n_thresh=100)
         assert np.array_equal(np.array(P, dtype=np.float64), g["sad_P"], equal_nan=True)
         assert np.array_equal(np.array(R, dtype=np.float64), g["sad_R"], equal_nan=True)

@@ -36,3 +36,26 @@ def test_bench_line_has_the_contract_keys():
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["value"] > 0
     assert d["extras"]["config1_latency"]["us_per_step"] > 0
     assert set(("sm_mhz", "sm_max_mhz", "reasons")) <= set(d["clocks"])
+
+
+def test_dump_outputs_repeat_and_match_the_oracle(tmp_path):
+    """--dump-outputs: two runs with the same arguments write the same arrays, and every stream's top-N lists are
+    the oracle's sequence matching + top-N of that stream's dumped spike counts."""
+    import numpy as np
+    from oracle import oracle as O
+    B, Q, P, L = 70, 3, 600, 2
+    argv = [sys.executable, os.path.join(ROOT, "bench.py"), "--config", "2", "--streams", str(B), "--queries", str(Q),
+            "--places", str(P), "--seq-len", str(L), "--steps", "2", "--warmup", "3", "--no-extras", "--no-cpu-baseline"]
+    for run in ("a", "b"):
+        res = subprocess.run(argv + ["--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-3000:]
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == ["S.npy", "hits.npy", "n_valid.npy", "overflow.npy", "sample_rows.npy", "top_idx.npy", "top_val.npy"]
+    a = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    for n, x in a.items():
+        assert x.dtype in (np.float32, np.float64) and np.array_equal(x, np.load(tmp_path / "b" / (n + ".npy"))), n
+    assert np.array_equal(a["sample_rows"], np.arange(B)) and a["S"].shape == (B, Q, P)
+    assert a["overflow"][0] == 0 and 0 < a["n_valid"][0] and np.all(a["hits"] <= a["n_valid"][0])
+    for b in range(B):
+        idx, val = O.topk(O.seqmatch(a["S"][b], L), 25)
+        assert np.array_equal(a["top_idx"][b], idx) and np.array_equal(a["top_val"][b], val), b
