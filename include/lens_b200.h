@@ -17,8 +17,10 @@
  *   - there is no CPU fallback: without a CUDA device every compute call fails.
  *
  * Hard limits (a violation is reported as a negative return code, never silently):
- *   lens_snn_create        I <= 1024, F <= 992; the tensor-core path needs 6 * 128 * Fp + 3 * 64 * Fp bytes of
- *                          shared memory (Fp = F rounded up to 32: F <= 224 today), larger F runs on the CUDA-core path
+ *   lens_snn_create        I <= 1024, F <= 992, every such shape runs on the CUDA-core path (LENS_SNN_SIMT);
+ *                          the tensor-core output layer needs 6 * 128 * Fp + 3 * 64 * Fp bytes of shared memory
+ *                          (Fp = F rounded up to 32: F <= 224), so LENS_SNN_TC rejects larger F and
+ *                          LENS_SNN_AUTO runs it on the CUDA-core path
  *   hidden spikes          <= LENS_MAX_SPIKE (127) per neuron and timestep (int8 transport); larger counts are
  *                          clipped and counted (lens_snn_get_overflow)
  *   lens_seqmatch_topk     N <= 64, 1 <= L <= min(Q, P)
@@ -28,7 +30,8 @@
  *   lens_topn_merge        W * N <= 512
  *   lens_bin_events        t_us ascending (lens_check_sorted_u32), x / y 16-byte aligned
  *   lens_snn_forward_float leaves IAF#0 possibly away from rest: the raster fast paths (and the tensor-core hidden
- *                          layer) stay disabled for the handle until lens_snn_reset
+ *                          layer) stay disabled for the handle until lens_snn_reset; the raster feature path also needs
+ *                          v_min <= 0 (v_min > 0 moves IAF#0 off rest by itself)
  *
  * Reference sites (relative to the reference repo root) each entry replaces are
  * cited per function.

@@ -452,9 +452,11 @@ static size_t raster_smem_bytes(const SnnHandle *h)
            (size_t)kRasterSlots * kChunk * h->Fp;
 }
 
+// IAF#0 stays at rest only for v_min <= 0: with v_min > 0 a step without input lifts it to v_min (and
+// v_min >= 1 makes it fire on its own), which feature_kernel computes and this path does not.
 static bool raster_path_ok(const SnnHandle *h)
 {
-    return h->Uq && h->thr == 1.0f && !h->v0_dirty && (size_t)h->I * h->F <= 65535 &&
+    return h->Uq && h->thr == 1.0f && h->vmin <= 0.0f && !h->v0_dirty && (size_t)h->I * h->F <= 65535 &&
            h->Fp * kRasterSlots <= 1024 && raster_smem_bytes(h) <= 227 * 1024;
 }
 
@@ -566,6 +568,22 @@ __global__ void __launch_bounds__(kOutThreads) output_simt_kernel(OutputParams p
     if (live) p.v2[(size_t)b * P + place] = v2;
 }
 
+static constexpr size_t feature_smem_bytes(int I, int Fp)
+{
+    return (size_t)kChunk * ((I + 31) & ~31) * 4 + kChunk * sizeof(int) + (size_t)kChunk * Fp;
+}
+
+static constexpr size_t output_simt_smem_bytes(int Fp) { return (size_t)kChunk * Fp * 4 + kChunk * sizeof(int); }
+
+// Dynamic shared memory above the default 48 KB needs a per-kernel opt-in.  A handle opts the CUDA-core
+// kernels in once, to what the largest shape lens_snn_create accepts needs (I = 1024, F = 992), so handles
+// of different sizes never lower each other's limit; shapes that fit 48 KB (the bundled models) never make
+// the call.
+constexpr size_t kDefaultSmem = 48 * 1024;
+constexpr size_t kFeatureSmemMax = feature_smem_bytes(1024, 992), kOutputSmemMax = output_simt_smem_bytes(992);
+static_assert(kFeatureSmemMax <= 227 * 1024 && kOutputSmemMax <= 227 * 1024,
+              "the CUDA-core kernels must run every shape lens_snn_create accepts");
+
 static int launch_feature(SnnHandle *h, const uint8_t *pooled, const float *xin, int b0, int nb,
                           int steps, uint8_t *hidden_steps, cudaStream_t st)
 {
@@ -576,8 +594,11 @@ static int launch_feature(SnnHandle *h, const uint8_t *pooled, const float *xin,
     p.v0 = h->v0 + (size_t)b0 * h->I; p.v1 = h->v1 + (size_t)b0 * h->F;
     p.S1 = h->S1; p.hidden_steps = hidden_steps; p.overflow = h->counters;
     int threads = (std::max(std::max(h->I, h->Fp), 32) + 31) & ~31;
-    int Ipad = (h->I + 31) & ~31;
-    size_t smem = (size_t)kChunk * Ipad * 4 + kChunk * sizeof(int) + (size_t)kChunk * h->Fp;
+    const size_t smem = feature_smem_bytes(h->I, h->Fp);
+    if (smem > kDefaultSmem && !h->feature_smem_optin) {
+        LENS_CUDA(cudaFuncSetAttribute(feature_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFeatureSmemMax));
+        h->feature_smem_optin = true;
+    }
     LaunchTimer timer(h, st, 0);
     feature_kernel<<<nb, threads, smem, st>>>(p);
     LENS_LAUNCH_CHECK();
@@ -592,7 +613,11 @@ static int launch_output_simt(SnnHandle *h, int b0, int nb, int steps, float *co
     p.Wo_fx = h->Wo_fx; p.Wo_scale = h->Wo_scale; p.S1 = h->S1; p.steps = steps;
     p.v2 = h->v2 + (size_t)b0 * h->P;
     p.counts = counts; p.spikes_out = spikes_out; p.out_steps = out_steps;
-    size_t smem = (size_t)kChunk * h->Fp * 4 + kChunk * sizeof(int);
+    const size_t smem = output_simt_smem_bytes(h->Fp);
+    if (smem > kDefaultSmem && !h->output_smem_optin) {
+        LENS_CUDA(cudaFuncSetAttribute(output_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kOutputSmemMax));
+        h->output_smem_optin = true;
+    }
     dim3 grid(nb, ceil_div(h->P, kOutThreads));
     LaunchTimer timer(h, st, 1);
     output_simt_kernel<<<grid, kOutThreads, smem, st>>>(p);

@@ -66,6 +66,7 @@ struct SnnHandle {
     bool v0_dirty = false;      // IAF#0 state may be non-zero (float path used): raster fast path is off
     float *v0 = nullptr, *v1 = nullptr, *v2 = nullptr;  // membrane potentials [maxB][I|F|P]
     int64_t *counters = nullptr;  // [0] spike overflow, [1] inexact weights
+    bool feature_smem_optin = false, output_smem_optin = false;  // CUDA-core kernels opted in to > 48 KB
     int8_t *S1 = nullptr;         // scratch hidden spikes [streams][steps][Fp]
     size_t S1_cap = 0;
     // tensor-core operands (built lazily by snn_tc.cu)

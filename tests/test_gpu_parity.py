@@ -81,7 +81,9 @@ def test_pool_frames():
 
 
 # -------------------------------------------------------------------------- K2 + K3
-def run_both(Wf, Wo, U, T, pooled, roi, k, mode, calls=1):
+def run_both(Wf, Wo, U, T, pooled, roi, k, mode, calls=1, want_steps=True):
+    """want_steps=False runs the production kernels (the debug buffers select other instantiations):
+    spike counts, membrane potentials and the overflow counter are compared; True adds every step."""
     from lens_b200.network import B200Network
     B, Q, I = pooled.shape
     onet = O.OracleSNN(Wf, Wo, U, T, n_streams=B)
@@ -90,47 +92,59 @@ def run_both(Wf, Wo, U, T, pooled, roi, k, mode, calls=1):
     assert gnet.n_inexact == 0
     res = []
     for part in np.array_split(np.arange(Q), calls):
-        oc, oh, oo = onet.run_streams(pooled[:, part], want_steps=True)
-        gc, gh, go = gnet.run_streams(pooled=cuda(pooled[:, part]), mode=mode, want_steps=True)
-        res.append((oc, oh, oo, gc.cpu().numpy(), gh.cpu().numpy(), go.cpu().numpy()))
+        if want_steps:
+            oc, oh, oo = onet.run_streams(pooled[:, part], want_steps=True)
+            gc, gh, go = gnet.run_streams(pooled=cuda(pooled[:, part]), mode=mode, want_steps=True)
+            res.append((oc, oh, oo, gc.cpu().numpy(), gh.cpu().numpy(), go.cpu().numpy()))
+        else:
+            oc = onet.run_streams(pooled[:, part])
+            gc = gnet.run_streams(pooled=cuda(pooled[:, part]), mode=mode)
+            res.append((oc, None, None, gc.cpu().numpy(), None, None))
     ov = onet.state()
     gv = [v.cpu().numpy() for v in gnet.state()]
     assert gnet.overflow() == onet.overflow()
     return res, ov, gv
 
 
+# (mode, want_steps): the per-step debug buffers select other instantiations of the kernels than a production
+# run does (with want_steps=False the tensor-core kernels take their fast scans), so both are compared
+SNN_MODES = [pytest.param(1, True, id="1"), pytest.param(2, True, id="2"),
+             pytest.param(1, False, id="1-production"), pytest.param(2, False, id="2-production")]
+
+
 def assert_same(res, ov, gv):
     for oc, oh, oo, gc, gh, go in res:
-        assert np.array_equal(gh, oh), "hidden spikes differ"
-        assert np.array_equal(go, oo), "output spikes differ"
+        if oh is not None:
+            assert np.array_equal(gh, oh), "hidden spikes differ"
+            assert np.array_equal(go, oo), "output spikes differ"
         assert np.array_equal(gc, oc), "spike counts differ"
     for a, b in zip(ov, gv):
         assert np.array_equal(a, b), "membrane potentials differ"
 
 
-@pytest.mark.parametrize("mode", [1, 2])
-def test_snn_config1_golden(golden, mode):
+@pytest.mark.parametrize("mode,want_steps", SNN_MODES)
+def test_snn_config1_golden(golden, mode, want_steps):
     """Bundled model + data: GPU == oracle bit for bit, and == the reference's own output."""
     g = golden("config1")
     roi, dims, T = int(g["roi_dim"]), int(g["dims"]), int(g["timebin"])
     k = roi // dims
     U = O.raster_uniforms(T, roi, k)
     pooled = O.pool(g["frames"], k)[None]
-    res, ov, gv = run_both(g["W_feat"], g["W_out"], U, T, pooled, roi, k, mode)
+    res, ov, gv = run_both(g["W_feat"], g["W_out"], U, T, pooled, roi, k, mode, want_steps=want_steps)
     assert_same(res, ov, gv)
     assert np.array_equal(res[0][3][0], g["S"].astype(np.float32))   # reference similarity matrix
     assert np.abs(gv[2][0] - g["v2"]).max() < 1e-5 and np.abs(gv[1][0] - g["v1"]).max() < 1e-5
 
 
-@pytest.mark.parametrize("mode", [1, 2])
-def test_snn_brisevent_golden_prefix(golden, mode):
+@pytest.mark.parametrize("mode,want_steps", SNN_MODES)
+def test_snn_brisevent_golden_prefix(golden, mode, want_steps):
     """Second bundled model (k = 1, P = 641, multi-spike outputs): first 60 queries."""
     g = golden("brisevent")
     roi, dims, T = int(g["roi_dim"]), int(g["dims"]), int(g["timebin"])
     k = roi // dims
     U = O.raster_uniforms(T, roi, k)
     pooled = O.pool(g["frames"][:60], k)[None]
-    res, ov, gv = run_both(g["W_feat"], g["W_out"], U, T, pooled, roi, k, mode)
+    res, ov, gv = run_both(g["W_feat"], g["W_out"], U, T, pooled, roi, k, mode, want_steps=want_steps)
     assert_same(res, ov, gv)
     S = g["S"][:60].astype(np.float32)
     assert (res[0][3][0] != S).sum() <= 2
@@ -143,8 +157,8 @@ def test_snn_brisevent_golden_prefix(golden, mode):
     (4, 40, 130, 33, 5, 2, 1),        # ragged: P not a multiple of the place tile, T odd
     (3, 9, 5, 7, 1, 1, 1),            # tiny
 ])
-@pytest.mark.parametrize("mode", [1, 2])
-def test_snn_synthetic(I_dims, F, P, T, B, Q, calls, mode):
+@pytest.mark.parametrize("mode,want_steps", SNN_MODES)
+def test_snn_synthetic(I_dims, F, P, T, B, Q, calls, mode, want_steps):
     I = I_dims * I_dims
     Wf, Wo = synth_weights(I, F, P, seed=F + P)
     k = 2
@@ -154,7 +168,7 @@ def test_snn_synthetic(I_dims, F, P, T, B, Q, calls, mode):
     pooled[0, 0, :] = 255          # saturated frame: every input fires every step
     if B > 1:
         pooled[1, :, :] = 0        # empty frames
-    res, ov, gv = run_both(Wf, Wo, U, T, pooled, roi, k, mode, calls=calls)
+    res, ov, gv = run_both(Wf, Wo, U, T, pooled, roi, k, mode, calls=calls, want_steps=want_steps)
     assert_same(res, ov, gv)
 
 
