@@ -29,6 +29,8 @@
  *   lens_sad_matrix        npix <= 65 793 (sums stay exact in fp32)
  *   lens_topn_merge        W * N <= 512
  *   lens_bin_events        t_us ascending (lens_check_sorted_u32), x / y 16-byte aligned
+ *   lens_bin_event_streams B >= 0, Q >= 0, B * Q <= 2^31 - 1 windows; t_us ascending within every stream
+ *                          (lens_check_sorted_segments_u32), x / y 16-byte aligned
  *   lens_snn_forward_float leaves IAF#0 possibly away from rest: the raster fast paths (and the tensor-core hidden
  *                          layer) stay disabled for the handle until lens_snn_reset; the raster feature path also needs
  *                          v_min <= 0 (v_min > 0 moves IAF#0 off rest by itself)
@@ -90,6 +92,33 @@ int lens_bin_events(const uint32_t *t_us, const uint16_t *x, const uint16_t *y, 
  * (4 B/event), therefore separate from the binning call; lens_b200.ops.bin_events(check_sorted=True)
  * runs it and raises.                                                                                  */
 int lens_check_sorted_u32(const uint32_t *t_us, int64_t n, int *unsorted, void *stream);
+
+/* K1 for B independent event streams in one call (launch count independent of B).
+ * Stream b owns events [offsets[b], offsets[b+1]) of the SoA arrays; t_us is ascending WITHIN a stream
+ * (streams may overlap in time and be stored in any order relative to each other).
+ * Window q < Q of stream b covers [t0_us[b] + q*window_us, t0_us[b] + (q+1)*window_us); events of the
+ * stream outside all Q windows are ignored.  Crop, index_shift, wrap_u8, pooling and win_events mean
+ * exactly what they mean for lens_bin_events; for every b the outputs equal lens_bin_events run on a
+ * copy of stream b's events with t0_us[b], byte for byte.  Every window range is clamped to
+ * [offsets[b], offsets[b+1]] inside [0, n_events], so malformed offsets never cause a read outside the
+ * event arrays (the outputs are then meaningless: check them with lens_check_sorted_segments_u32).
+ * B = 0 or Q = 0 returns 0 without launching.
+ *   offsets     [B + 1] i64 device, 0 <= offsets[0] <= ... <= offsets[B] <= n_events
+ *   t0_us       [B] u32 device
+ *   frames      [B][Q][roi][roi] u8 (nullable), pooled [B][Q][dims*dims] u8 (nullable)
+ *   win_events  [B][Q] i32 (nullable)
+ *   win_offsets [B][Q + 1] i64 scratch/out: absolute first event index of each window + end of the last */
+int lens_bin_event_streams(const uint32_t *t_us, const uint16_t *x, const uint16_t *y, int64_t n_events,
+                           const int64_t *offsets, const uint32_t *t0_us, int B, int Q, uint32_t window_us,
+                           int roi_x0, int roi_y0, int roi, int k, int index_shift, int wrap_u8,
+                           uint8_t *frames, uint8_t *pooled, int32_t *win_events, int64_t *win_offsets,
+                           void *stream);
+/* Precondition of lens_bin_event_streams.  *bad (device int) = 1 if some offsets[b] > offsets[b+1],
+ * offsets[0] < 0, offsets[B] > n, or t_us descends inside a stream (a descent where a new stream starts is
+ * allowed); else 0.  One streaming pass over t_us; memory-safe for any offsets content.  t_us 16-byte
+ * aligned.  lens_b200.ops.bin_event_streams(check_sorted=True) runs it and raises.                      */
+int lens_check_sorted_segments_u32(const uint32_t *t_us, int64_t n, const int64_t *offsets, int B, int *bad,
+                                   void *stream);
 
 /* Pooling alone (frames already exist, e.g. decoded PNGs):
  * frames [n][roi][roi] u8 -> pooled [n][dims*dims] u8.  lens/run_model.py:130-137. */

@@ -30,6 +30,9 @@ def _declare(L):
                                   vp, vp, vp, vp, i64, vp]),
         "lens_pool_frames": (i32, [vp, i64, i32, i32, vp, vp]),
         "lens_check_sorted_u32": (i32, [vp, i64, vp, vp]),
+        "lens_bin_event_streams": (i32, [vp, vp, vp, i64, vp, vp, i32, i32, u32, i32, i32, i32, i32, i32, i32,
+                                         vp, vp, vp, vp, vp]),
+        "lens_check_sorted_segments_u32": (i32, [vp, i64, vp, i32, vp, vp]),
         "lens_snn_create": (i32, [i32, i32, i32, i32, f32, f32, vp, vp, vp, i32,
                                   C.POINTER(vp), pi64, vp]),
         "lens_snn_destroy": (i32, [vp]),

@@ -64,6 +64,42 @@ def bin_events(t_us, x, y, t0_us, window_us, n_win, roi, k, roi_x0=0, roi_y0=0, 
     return frames, pooled, cnt
 
 
+def bin_event_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi, k, roi_x0=0, roi_y0=0, index_shift=1,
+                      wrap_u8=True, want_frames=False, want_pooled=True, check_sorted=False):
+    """B independent event streams in one call -> (frames u8 [B, Q, roi, roi], pooled u8 [B, Q, I],
+    events-per-window i32 [B, Q]); frames / pooled are None unless wanted.
+
+    Stream b is events [offsets[b], offsets[b+1]) of t_us / x / y (offsets i64 [B + 1] on the device) and
+    its window q covers [t0_us[b] + q * window_us, t0_us[b] + (q + 1) * window_us) (t0_us i32 / u32 [B]).
+    Per stream the results equal `bin_events` on that stream's events with t0_us[b].  t_us must be ascending
+    within every stream; check_sorted=True verifies that and the offsets (one extra pass over t_us,
+    lens_check_sorted_segments_u32, synchronises) and raises ValueError before binning.
+    """
+    require_cuda(t_us, x, y, offsets, t0_us)
+    assert t_us.dtype in (torch.int32, torch.uint32) and t0_us.dtype in (torch.int32, torch.uint32)
+    assert x.dtype in (torch.int16, torch.uint16) and y.dtype in (torch.int16, torch.uint16)
+    assert offsets.dtype == torch.int64 and offsets.dim() == 1 and offsets.numel() >= 1
+    B, Q, n = offsets.numel() - 1, int(Q), t_us.numel()
+    assert t0_us.shape == (B,) and x.numel() == n and y.numel() == n
+    dev = t_us.device
+    if check_sorted:
+        flag = torch.zeros(1, dtype=torch.int32, device=dev)
+        check(_lib.lib().lens_check_sorted_segments_u32(ptr(t_us), n, ptr(offsets), B, ptr(flag), stream_ptr()),
+              "lens_check_sorted_segments_u32")
+        if int(flag.item()):
+            raise ValueError("event timestamps must be ascending within every stream, and offsets non-decreasing "
+                             "inside [0, n_events]")
+    dims, _ = pool_geometry(roi, k)
+    frames = torch.empty((B, Q, roi, roi), dtype=torch.uint8, device=dev) if want_frames else None
+    pooled = torch.empty((B, Q, dims * dims), dtype=torch.uint8, device=dev) if want_pooled else None
+    cnt = torch.empty((B, Q), dtype=torch.int32, device=dev)
+    offs = torch.empty((max(B, 1), Q + 1), dtype=torch.int64, device=dev)   # never NULL, even for B = 0
+    check(_lib.lib().lens_bin_event_streams(ptr(t_us), ptr(x), ptr(y), n, ptr(offsets), ptr(t0_us), B, Q, window_us,
+                                            roi_x0, roi_y0, roi, k, index_shift, int(wrap_u8), ptr(frames),
+                                            ptr(pooled), ptr(cnt), ptr(offs), stream_ptr()), "lens_bin_event_streams")
+    return frames, pooled, cnt
+
+
 def seqmatch_topk(S, L, N=25, want_D=False):
     """S f32 [B, Q, P] -> (top_val [B, Qo, N], top_idx [B, Qo, N], D [B, Po, Qo] or None).
 

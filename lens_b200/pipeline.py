@@ -1,4 +1,4 @@
-"""The hot path as one object: frames -> pooled pixels -> spike counts -> sequence matching ->
+"""The hot path as one object: events or frames -> pooled pixels -> spike counts -> sequence matching ->
 top-N -> Recall@N counters, for a shard of independent query streams on one GPU.
 
 This is what `LENS.evaluate` does for one stream and what bench.py / the multi-GPU driver do for
@@ -10,6 +10,7 @@ GPU, no data-path collective) and the Recall@N counters are summed with one all-
 import torch
 
 from . import ops
+from ._lib import LensError
 from .network import B200Network, MODE_AUTO
 
 
@@ -69,11 +70,76 @@ class InferencePipeline:
             self._stage_events.append(ev)
         out["S"] = S
         out["overflow"] = self.net.overflow_tensor()   # device counter, no synchronisation: check with .item()
-        if reduce and out["hits"] is not None and torch.distributed.is_available() \
+        if reduce:
+            self._all_reduce_hits(out)
+        return out
+
+    @staticmethod
+    def _all_reduce_hits(out):
+        if out["hits"] is not None and torch.distributed.is_available() \
                 and torch.distributed.is_initialized() and torch.distributed.get_world_size() > 1:
             packed = torch.cat([out["hits"], out["n_valid"]])
             torch.distributed.all_reduce(packed)          # sum of 6 hit counters + valid count
             out["hits"], out["n_valid"] = packed[:-1], packed[-1:]
+
+    def _bin_streams(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0):
+        net = self.net
+        _, pooled, n_ev = ops.bin_event_streams(t_us, x, y, offsets, t0_us, window_us, Q, net.roi, net.k,
+                                                roi_x0=roi_x0, roi_y0=roi_y0, want_frames=False, want_pooled=True)
+        return pooled, n_ev
+
+    def step_events(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0=0, roi_y0=0, gt_dense=None,
+                    gt_center=None, gt_tol=0, reduce=True):
+        """The step fed from raw event streams: stream b is events [offsets[b], offsets[b+1]) of the device
+        arrays t_us / x / y, and query q of stream b is its window [t0_us[b] + q * window_us, + window_us)
+        (see ops.bin_event_streams).  The events are binned straight to pooled pixels (no frames are
+        written) and run through the same work as `step(pooled=...)`.  Returns `step`'s dict plus
+        "events_per_window" i32 [B, Q].
+
+        Every stream yields exactly Q queries: a window without events becomes an all-zero pooled row and
+        stays a query, unlike collect_data.create_images in the reference, which drops empty windows
+        (collect_data.frames_from_events is the single-stream path that reproduces that)."""
+        with torch.cuda.device(self.device):
+            pooled, n_ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
+            out = self.step(pooled=pooled, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce)
+        out["events_per_window"] = n_ev
+        return out
+
+    def step_event_groups(self, groups, B, Q, window_us, roi_x0=0, roi_y0=0, gt_dense=None, gt_center=None,
+                          gt_tol=0, reduce=True):
+        """`step_events` for fleets whose events do not fit in device memory together.
+
+        `groups` yields (b0, t_us, x, y, offsets, t0_us) for consecutive ranges of streams that cover
+        [0, B): the group's streams are b0 .. b0 + len(t0_us) - 1, with offsets relative to its own arrays.
+        b0 must be even (the network tiles streams in pairs).  Each group is binned and run through the
+        network as soon as it arrives, into one spike-count tensor S [B, Q, P]; matching, top-N and recall
+        run once at the end.  The results equal `step_events` on the same events bit for bit; the per-group
+        event arrays may be released or refilled once the group's kernels have run (stream order)."""
+        net = self.net
+        with torch.cuda.device(self.device):
+            net.ensure_streams(B)
+            S = torch.empty((B, Q, net.P), dtype=torch.float32, device=self.device)
+            n_ev = torch.empty((B, Q), dtype=torch.int32, device=self.device)
+            b_next = 0
+            for b0, t_us, x, y, offsets, t0_us in groups:
+                nb = offsets.numel() - 1
+                if b0 % 2:
+                    raise LensError(f"event group starts at odd stream {b0}: b0 must be even")
+                if b0 != b_next or b0 + nb > B:
+                    raise LensError(f"event groups must cover streams [0, {B}) in order: got [{b0}, {b0 + nb}) "
+                                    f"after [0, {b_next})")
+                pooled, ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
+                n_ev[b0:b0 + nb] = ev
+                net.run_streams_range(pooled, b0, S[b0:b0 + nb], mode=self.mode)
+                b_next = b0 + nb
+            if b_next != B:
+                raise LensError(f"event groups cover streams [0, {b_next}) of {B}")
+            out = self.match(S, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol)
+            out["S"] = S
+            out["overflow"] = net.overflow_tensor()
+        out["events_per_window"] = n_ev
+        if reduce:
+            self._all_reduce_hits(out)
         return out
 
     def step_host(self, frames_host, gt_dense=None, gt_center=None, gt_tol=0, next_frames=None, reduce=True):

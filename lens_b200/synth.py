@@ -2,8 +2,9 @@
 
 No datasets or checkpoints are reachable from the GPU box, so benchmarks and scale tests use
 random weights with the statistics of the trained LENS models and random count frames / event
-streams with the statistics of the bundled Speck recordings.  Everything is generated on the
-host with numpy (deterministic per seed) and moved to the device by the caller.
+streams with the statistics of the bundled Speck recordings.  The small generators run on the
+host with numpy (deterministic per seed) and the caller moves their output to the device; the
+*_device ones draw full-size workloads on the GPU.
 """
 import numpy as np
 
@@ -104,6 +105,13 @@ def events_device(n_events, sensor=128, window_us=250_000, events_per_window=131
         tt = torch.randint(0, wins * window_us, (n,), dtype=torch.int32, device=device, generator=g)
         t[c0:c0 + n] = torch.sort(tt).values + base
     assert n_win * window_us < 2 ** 31
+    x, y = _pixels_device(n_events, sensor, hot_pixels, hot_rate, g, device)
+    return t, x, y, int(n_win)
+
+
+def _pixels_device(n_events, sensor, hot_pixels, hot_rate, g, device):
+    """x, y i16 [n_events] uniform over the sensor, `hot_pixels` pixels firing `hot_rate` times more often."""
+    import torch
     x = torch.randint(0, sensor, (n_events,), dtype=torch.int16, device=device, generator=g)
     y = torch.randint(0, sensor, (n_events,), dtype=torch.int16, device=device, generator=g)
     if hot_pixels:
@@ -117,4 +125,51 @@ def events_device(n_events, sensor=128, window_us=250_000, events_per_window=131
             pick = torch.randint(0, hot_pixels, (n,), device=device, generator=g)
             x[c0:c0 + n] = torch.where(m, hx[pick], x[c0:c0 + n])
             y[c0:c0 + n] = torch.where(m, hy[pick], y[c0:c0 + n])
-    return t, x, y, int(n_win)
+    return x, y
+
+
+def event_streams_device(B, Q, window_us=250_000, events_per_window=131_072, sensor=128, seed=11, hot_pixels=16,
+                         hot_rate=100.0, device="cuda", chunk_events=1 << 26):
+    """B independent DVS streams of Q windows each (the query streams of BASELINE configs 2 and 3), drawn
+    on the device: (t_us i32, x i16, y i16, offsets i64 [B + 1], t0_us i32 [B]); stream b is events
+    [offsets[b], offsets[b+1]), its window q is [t0_us[b] + q * window_us, + window_us).
+
+    Timestamps are relative to each stream (all below 2^31) and ascending within it.  t0_us[b] is uniform in
+    [window_us / 4, window_us); fewer than 64 events per stream fall before it.  Window q holds
+    events_per_window +- 1/16 events at uniform times, so stream and window starts fall anywhere relative to
+    16-byte boundaries.  x, y as in `events_device`: at the default density 8 events per sensor pixel and
+    window, the mean count of `frames`.  Deterministic per seed and device type."""
+    import torch
+    assert (Q + 1) * window_us < 2 ** 31
+    g = torch.Generator(device=device).manual_seed(int(seed))
+    i64 = dict(dtype=torch.int64, device=device)
+    t0 = torch.randint(window_us // 4, window_us, (B,), generator=g, **i64)
+    jit = events_per_window // 16
+    counts = torch.randint(events_per_window - jit, events_per_window + jit + 1, (B, Q), generator=g, **i64)
+    pre = torch.randint(0, 64, (B, 1), generator=g, **i64)
+    seg_len = torch.cat([pre, counts], 1)                         # [B, Q + 1]: before t0, then the Q windows
+    seg_t0 = torch.cat([torch.zeros((B, 1), **i64), t0[:, None] + window_us * torch.arange(Q, **i64)], 1)
+    seg_span = torch.cat([t0[:, None], torch.full((B, Q), window_us, **i64)], 1)
+    offsets = torch.zeros(B + 1, **i64)
+    offsets[1:] = torch.cumsum(seg_len.sum(1), 0)
+    n = int(offsets[-1])
+    t = torch.empty(n, dtype=torch.int32, device=device)
+    bits = int(window_us).bit_length()
+    off_host = offsets.cpu()
+    b0 = 0
+    while b0 < B:                                                 # whole streams, about chunk_events at a time
+        b1 = int(torch.searchsorted(off_host, off_host[b0] + chunk_events, right=True)) - 1
+        b1 = min(max(b1, b0 + 1), B)
+        lens = seg_len[b0:b1].reshape(-1)
+        seg = torch.repeat_interleave(torch.arange(lens.numel(), **i64), lens)
+        span = seg_span[b0:b1].reshape(-1)[seg]
+        local = torch.minimum((torch.rand(seg.numel(), device=device, generator=g, dtype=torch.float64)
+                               * span).to(torch.int64), span - 1)
+        del span
+        key = torch.sort((seg << bits) | local).values            # sorted inside each segment
+        seg = key >> bits
+        t[int(off_host[b0]):int(off_host[b1])] = (seg_t0[b0:b1].reshape(-1)[seg] + (key & ((1 << bits) - 1))).to(torch.int32)
+        del seg, local, key
+        b0 = b1
+    x, y = _pixels_device(n, sensor, hot_pixels, hot_rate, g, device)
+    return t, x, y, offsets, t0.to(torch.int32)
