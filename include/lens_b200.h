@@ -24,6 +24,8 @@
  *   hidden spikes          <= LENS_MAX_SPIKE (127) per neuron and timestep (int8 transport); larger counts are
  *                          clipped and counted (lens_snn_get_overflow)
  *   lens_seqmatch_topk     N <= 64, 1 <= L <= min(Q, P)
+ *   lens_seqmatch_topk_stream
+ *                          N <= 64, 1 <= L <= P, Q >= 1, B * Q <= 2^31 - 1; ring non-NULL unless L == 1, seen non-NULL
  *   lens_recall / _bounds  at most 8 values of N per call
  *   lens_pr_counts         Qo <= 8192 (one CTA, shared-memory resident)
  *   lens_sad_matrix        npix <= 65 793 (sums stay exact in fp32)
@@ -144,6 +146,11 @@ int lens_snn_create(int I, int F, int P, int T, float thr, float v_min, const fl
 int lens_snn_destroy(void *handle);
 /* sinabs Network.reset_states(): zero all membrane potentials. */
 int lens_snn_reset(void *handle, void *stream);
+/* Per-stream sinabs reset_states(): zero v0/v1/v2 of every stream b < max_streams with mask[b] != 0.
+ *   mask [max_streams] u8 device.
+ * Other streams' state, the overflow counter and the forward_float flag (IAF#0 off rest) are untouched.
+ * One launch whatever the number of streams.                                                            */
+int lens_snn_reset_streams(void *handle, const uint8_t *mask, void *stream);
 /* copy membrane potentials out (any pointer nullable): v0 [B][I], v1 [B][F], v2 [B][P] */
 int lens_snn_get_state(void *handle, float *v0, float *v1, float *v2, void *stream);
 /* overflow[0] (device, i64) counts per-step spike counts that exceeded LENS_MAX_SPIKE */
@@ -196,6 +203,24 @@ int lens_snn_forward_float(void *handle, const float *x, int B, int steps, float
  * L >= 1 (the reference's L == 0 branch returns S itself and is handled by the caller). */
 int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, int N, float *D_out,
                        float *top_val, int32_t *top_idx, void *stream);
+
+/* K4 across calls, for live streams that deliver a few rows at a time.  All B streams advance in lockstep; number
+ * a stream's rows g = 0, 1, 2, ... since its last reset.  New row g closes the sequence column
+ *   D_g[r] = (1/L) * sum_{j<L} S[g - L + 1 + j][r + j],   r in [0, P - L + 1)
+ * (same arithmetic and order as lens_seqmatch_topk).  It is valid once the stream has seen L rows (g >= L - 1);
+ * a warm-up row gets -inf / -1 in every slot.  Fed any chunking of the same rows, the valid rows equal the columns
+ * of one lens_seqmatch_topk over all of them, bit for bit.
+ *   S       [B][Q][P] f32: the Q new rows of every stream
+ *   ring    [B][L-1][P] f32, caller-owned: the last L-1 rows of every stream, row g at slot g mod (L-1), where g
+ *           counts rows pushed (t), not rows since the reset; NULL allowed iff L == 1.  Need not be initialised.
+ *   seen    [B] i32: rows seen since the stream's reset, saturating at L-1 (0 = fresh / just reset)
+ *   t       rows pushed so far (the same for every stream; the caller adds Q after each call)
+ *   top_val [B][Q][N] f32, top_idx [B][Q][N] i32: row q = the sequence ending at new row q
+ * Matches first, then stores the last min(Q, L-1) rows of S into the ring and advances seen (stream order).
+ * Two launches per call (one when L == 1), three when the places of a row are split into segments (the
+ * segmented kernel and lens_topn_merge's kernel); never more with B.  B = 0 returns 0 without launching.  */
+int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, int L, int N, float *ring, int32_t *seen,
+                              int64_t t, float *top_val, int32_t *top_idx, void *stream);
 
 /* Recall@N counters (lens/src/metrics.py:213-224 + lens/run_model.py:301-302).
  * Ground truth is either dense, gt_dense [B or 1][Po][Qo] u8 (gt_stream_stride = Po*Qo

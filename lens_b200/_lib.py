@@ -37,12 +37,14 @@ def _declare(L):
                                   C.POINTER(vp), pi64, vp]),
         "lens_snn_destroy": (i32, [vp]),
         "lens_snn_reset": (i32, [vp, vp]),
+        "lens_snn_reset_streams": (i32, [vp, vp, vp]),
         "lens_snn_get_state": (i32, [vp, vp, vp, vp, vp]),
         "lens_snn_get_overflow": (i32, [vp, vp, vp]),
         "lens_snn_forward": (i32, [vp, vp, i32, i32, vp, vp, vp, i32, vp]),
         "lens_snn_forward_range": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, i32, vp]),
         "lens_snn_forward_float": (i32, [vp, vp, i32, i32, vp, vp]),
         "lens_seqmatch_topk": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp]),
+        "lens_seqmatch_topk_stream": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, i64, vp, vp, vp]),
         "lens_sad_matrix": (i32, [vp, vp, i32, i32, i32, vp, vp]),
         "lens_reciprocal": (i32, [vp, i64, vp, vp]),
         "lens_online_accumulate": (i32, [vp, vp, i32, i32, vp, vp]),

@@ -33,6 +33,59 @@ __device__ __forceinline__ float f32_from_orderable(uint32_t u)
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
+// One top-N slot from its key (0 = empty slot: -inf / -1).
+__device__ __forceinline__ void store_key(unsigned long long k, size_t o, float *__restrict__ top_val,
+                                          int32_t *__restrict__ top_idx)
+{
+    if (k == 0ull) {
+        top_val[o] = -INFINITY;
+        top_idx[o] = -1;
+    } else {
+        top_val[o] = f32_from_orderable((uint32_t)(k >> 32));
+        top_idx[o] = (int32_t)(uint32_t)(k & 0xffffffffull);
+    }
+}
+
+// Merges the nr keys of cand (a chunk of places) into the running top-N `best` (descending, 0 = empty slot); all
+// arrays in shared memory, called by every thread of the CTA between barriers.
+__device__ __forceinline__ void cta_merge_chunk(unsigned long long *cand, unsigned long long *best,
+                                                unsigned long long *next_best, unsigned long long *warp_best,
+                                                unsigned long long &s_winner, int nr, int N, int tid, int lane,
+                                                int warp)
+{
+    // N rounds of block-wide max over (running best U chunk); keys are unique
+    // (distinct place index) so exactly one slot holds the winner.
+    for (int n = 0; n < N; ++n) {
+        unsigned long long mine = 0ull;
+        int mine_pos = -1;
+        for (int i = tid; i < N + nr; i += kMatchThreads) {
+            const unsigned long long k = (i < N) ? best[i] : cand[i - N];
+            if (k > mine) { mine = k; mine_pos = i; }
+        }
+        unsigned long long wb = mine;
+        for (int o = 16; o > 0; o >>= 1) {
+            const unsigned long long other = __shfl_xor_sync(0xffffffffu, wb, o);
+            wb = other > wb ? other : wb;
+        }
+        if (lane == 0) warp_best[warp] = wb;
+        __syncthreads();
+        if (tid == 0) {
+            unsigned long long w = 0ull;
+            for (int i = 0; i < kMatchThreads / 32; ++i) w = warp_best[i] > w ? warp_best[i] : w;
+            s_winner = w;
+            next_best[n] = w;
+        }
+        __syncthreads();
+        if (mine != 0ull && mine == s_winner) {
+            if (mine_pos < N) best[mine_pos] = 0ull;
+            else cand[mine_pos - N] = 0ull;
+        }
+        __syncthreads();
+    }
+    for (int i = tid; i < N; i += kMatchThreads) best[i] = next_best[i];
+    __syncthreads();
+}
+
 // grid = B * Qo.  One CTA scores every database place for one (stream, query).
 __global__ void __launch_bounds__(kMatchThreads)
 seqmatch_topk_kernel(const float *__restrict__ S, int Q, int P, int L, int N,
@@ -62,49 +115,9 @@ seqmatch_topk_kernel(const float *__restrict__ S, int Q, int P, int L, int N,
             cand[i] = ((unsigned long long)f32_orderable(d) << 32) | (uint32_t)r;
         }
         __syncthreads();
-        // N rounds of block-wide max over (running best U chunk); keys are unique
-        // (distinct place index) so exactly one slot holds the winner.
-        for (int n = 0; n < N; ++n) {
-            unsigned long long mine = 0ull;
-            int mine_pos = -1;
-            for (int i = tid; i < N + nr; i += kMatchThreads) {
-                const unsigned long long k = (i < N) ? best[i] : cand[i - N];
-                if (k > mine) { mine = k; mine_pos = i; }
-            }
-            unsigned long long wb = mine;
-            for (int o = 16; o > 0; o >>= 1) {
-                const unsigned long long other = __shfl_xor_sync(0xffffffffu, wb, o);
-                wb = other > wb ? other : wb;
-            }
-            if (lane == 0) warp_best[warp] = wb;
-            __syncthreads();
-            if (tid == 0) {
-                unsigned long long w = 0ull;
-                for (int i = 0; i < kMatchThreads / 32; ++i) w = warp_best[i] > w ? warp_best[i] : w;
-                s_winner = w;
-                next_best[n] = w;
-            }
-            __syncthreads();
-            if (mine != 0ull && mine == s_winner) {
-                if (mine_pos < N) best[mine_pos] = 0ull;
-                else cand[mine_pos - N] = 0ull;
-            }
-            __syncthreads();
-        }
-        for (int i = tid; i < N; i += kMatchThreads) best[i] = next_best[i];
-        __syncthreads();
+        cta_merge_chunk(cand, best, next_best, warp_best, s_winner, nr, N, tid, lane, warp);
     }
-    for (int n = tid; n < N; n += kMatchThreads) {
-        const unsigned long long k = best[n];
-        const size_t o = ((size_t)b * Qo + q) * N + n;
-        if (k == 0ull) {
-            top_val[o] = -INFINITY;
-            top_idx[o] = -1;
-        } else {
-            top_val[o] = f32_from_orderable((uint32_t)(k >> 32));
-            top_idx[o] = (int32_t)(uint32_t)(k & 0xffffffffull);
-        }
-    }
+    for (int n = tid; n < N; n += kMatchThreads) store_key(best[n], ((size_t)b * Qo + q) * N + n, top_val, top_idx);
 }
 
 // ---- warp-per-query variant (N <= 32) ------------------------------------------------------------
@@ -123,6 +136,31 @@ __device__ __forceinline__ unsigned long long shfl_u64(unsigned long long v, int
     const unsigned lo = __shfl_sync(0xffffffffu, (unsigned)v, src);
     const unsigned hi = __shfl_sync(0xffffffffu, (unsigned)(v >> 32), src);
     return ((unsigned long long)hi << 32) | lo;
+}
+
+// Lane i of `best` holds the i-th largest key of a warp's running list; `key` is one candidate per lane.  Returns the
+// top 32 of (list U batch): a bitonic sort of the batch, then a bitonic merge with the list.
+__device__ __forceinline__ unsigned long long warp_top32_merge(unsigned long long best, unsigned long long key, int lane)
+{
+    // bitonic sort of the batch, descending
+#pragma unroll
+    for (int k = 2; k <= 32; k <<= 1) {
+#pragma unroll
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            const unsigned long long other = shfl_xor_u64(key, j);
+            const bool take_max = (((lane & j) == 0) == ((lane & k) == 0));
+            key = take_max ? (key > other ? key : other) : (key < other ? key : other);
+        }
+    }
+    // top 32 of (running list U batch): elementwise max against the reversed batch is bitonic
+    const unsigned long long rev = shfl_u64(key, 31 - lane);
+    unsigned long long c = best > rev ? best : rev;
+#pragma unroll
+    for (int j = 16; j > 0; j >>= 1) {
+        const unsigned long long other = shfl_xor_u64(c, j);
+        c = ((lane & j) == 0) ? (c > other ? c : other) : (c < other ? c : other);
+    }
+    return c;
 }
 
 // kSeg = false is the plain one-warp-per-query kernel (40 registers: six CTAs per SM; the segmented instantiation
@@ -178,37 +216,159 @@ seqmatch_topk_warp_kernel(const float *__restrict__ S, long long n_queries, int 
                 }
                 const unsigned long long kth = shfl_u64(best, 31);          // current 32nd largest
                 if (!__any_sync(0xffffffffu, key > kth)) continue;          // nothing in this batch can enter
-                // bitonic sort of the batch, descending
+                best = warp_top32_merge(best, key, lane);
+            }
+        }
+        if (lane < N) store_key(best, (size_t)w * N + lane, top_val, top_idx);     // w = seg * n_queries + g
+    }
+}
+
+// ---- streaming K4 (lens_seqmatch_topk_stream) -------------------------------------------------------------------
+// New row q of stream b (global row t + q) closes the sequence of rows t + q - L + 1 .. t + q.  Term j of its diagonal
+// is new row q - L + 1 + j of S when that is >= 0, else an older row, kept in the stream's ring at slot
+// (t + q - L + 1 + j) mod (L - 1).  The choice depends on (q, j) only, so the pointer is warp-uniform per term and
+// the loads along the places stay coalesced as in the batch kernels.
+struct StreamRows {
+    const float *Sq;       // new row q of stream b
+    const float *ring_b;   // [L-1][P] ring of stream b
+    int n_old;             // terms j < n_old come from the ring
+    int slot0;             // ring slot of term 0 (valid rows only: t + q - L + 1 >= 0 there)
+    int Lm1, L;
+    size_t P;
+    __device__ __forceinline__ StreamRows(const float *S, const float *ring, int b, int Q, int q, int P_, int L_,
+                                          long long t)
+        : Sq(S + ((size_t)b * Q + q) * P_), ring_b(ring + (size_t)b * (L_ - 1) * P_), n_old(max(L_ - 1 - q, 0)),
+          slot0(L_ > 1 ? (int)((t + q - L_ + 1) % (L_ - 1)) : 0), Lm1(L_ - 1), L(L_), P((size_t)P_) {}
+    __device__ __forceinline__ const float *row(int j) const
+    {
+        if (j < n_old) {
+            int s = slot0 + j;
+            if (s >= Lm1) s -= Lm1;
+            return ring_b + (size_t)s * P;
+        }
+        return Sq - (size_t)(L - 1 - j) * P;
+    }
+};
+
+// A row is a sequence end once its stream has seen L rows since its reset (seen saturates at L - 1).
+__device__ __forceinline__ bool stream_row_valid(const int32_t *__restrict__ seen, int b, int q, int L)
+{
+    return __ldg(seen + b) + q + 1 >= L;
+}
+
+// The warp-per-query kernel (N <= 32) over the B * Q new rows, kSeg as in seqmatch_topk_warp_kernel.  A warm-up row
+// (not valid) skips the scan and stores an empty list.
+template <bool kSeg>
+__global__ void __launch_bounds__(256, kSeg ? 1 : 6)
+seqmatch_topk_stream_warp_kernel(const float *__restrict__ S, const float *__restrict__ ring,
+                                 const int32_t *__restrict__ seen, long long t, long long n_queries, int Q, int P, int L,
+                                 int N, int n_seg, int seg_len, float *__restrict__ top_val, int32_t *__restrict__ top_idx)
+{
+    const int lane = threadIdx.x & 31;
+    const int Po_all = P - L + 1;
+    const float fl = (float)L;
+    const long long warp0 = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long w = warp0; w < (kSeg ? n_queries * n_seg : n_queries); w += n_warps) {
+        const int seg = kSeg ? (int)(w / n_queries) : 0;
+        const long long g = kSeg ? w - (long long)seg * n_queries : w;
+        const int b = (int)(g / Q), q = (int)(g - (long long)b * Q);
+        const int Po = kSeg ? min(Po_all, (seg + 1) * seg_len) : Po_all;
+        unsigned long long best = 0ull;                    // lane i: i-th largest key, 0 = empty
+        if (stream_row_valid(seen, b, q, L)) {
+            const StreamRows rows(S, ring, b, Q, q, P, L, t);
+            for (int r0 = kSeg ? seg * seg_len : 0; r0 < Po; r0 += 32 * kUnrollR) {
+                float acc[kUnrollR];
 #pragma unroll
-                for (int k = 2; k <= 32; k <<= 1) {
+                for (int u = 0; u < kUnrollR; ++u) acc[u] = 0.0f;
+                if (r0 + 32 * kUnrollR <= Po) {
+                    // two diagonal terms per iteration: with one new row per push nearly every load misses L2
+                    // (the batch kernel re-reads each row L times from L2), so more bytes must be in flight
+#pragma unroll 2
+                    for (int j = 0; j < L; ++j) {
+                        const float *row = rows.row(j) + (r0 + lane + j);
 #pragma unroll
-                    for (int j = k >> 1; j > 0; j >>= 1) {
-                        const unsigned long long other = shfl_xor_u64(key, j);
-                        const bool take_max = (((lane & j) == 0) == ((lane & k) == 0));
-                        key = take_max ? (key > other ? key : other) : (key < other ? key : other);
+                        for (int u = 0; u < kUnrollR; ++u) acc[u] += __ldg(row + 32 * u);
+                    }
+                } else {
+                    for (int j = 0; j < L; ++j) {
+                        const float *row = rows.row(j) + (r0 + lane + j);
+#pragma unroll
+                        for (int u = 0; u < kUnrollR; ++u)
+                            if (r0 + 32 * u + lane < Po) acc[u] += __ldg(row + 32 * u);
                     }
                 }
-                // top 32 of (running list U batch): elementwise max against the reversed batch is bitonic
-                const unsigned long long rev = shfl_u64(key, 31 - lane);
-                unsigned long long c = best > rev ? best : rev;
 #pragma unroll
-                for (int j = 16; j > 0; j >>= 1) {
-                    const unsigned long long other = shfl_xor_u64(c, j);
-                    c = ((lane & j) == 0) ? (c > other ? c : other) : (c < other ? c : other);
+                for (int u = 0; u < kUnrollR; ++u) {
+                    const int r = r0 + 32 * u + lane;
+                    unsigned long long key = 0ull;
+                    if (r < Po) key = ((unsigned long long)f32_orderable(__fdiv_rn(acc[u], fl)) << 32) | (uint32_t)r;
+                    const unsigned long long kth = shfl_u64(best, 31);
+                    if (!__any_sync(0xffffffffu, key > kth)) continue;
+                    best = warp_top32_merge(best, key, lane);
                 }
-                best = c;
             }
         }
-        if (lane < N) {
-            const size_t o = (size_t)w * N + lane;             // w = seg * n_queries + g
-            if (best == 0ull) {
-                top_val[o] = -INFINITY;
-                top_idx[o] = -1;
-            } else {
-                top_val[o] = f32_from_orderable((uint32_t)(best >> 32));
-                top_idx[o] = (int32_t)(uint32_t)(best & 0xffffffffull);
+        if (lane < N) store_key(best, (size_t)w * N + lane, top_val, top_idx);     // w = seg * n_queries + g
+    }
+}
+
+// The CTA-per-query kernel (32 < N <= 64) over the B * Q new rows; grid = B * Q.
+__global__ void __launch_bounds__(kMatchThreads)
+seqmatch_topk_stream_kernel(const float *__restrict__ S, const float *__restrict__ ring,
+                            const int32_t *__restrict__ seen, long long t, int Q, int P, int L, int N,
+                            float *__restrict__ top_val, int32_t *__restrict__ top_idx)
+{
+    __shared__ unsigned long long cand[kCandChunk];
+    __shared__ unsigned long long best[kMaxTopN];
+    __shared__ unsigned long long next_best[kMaxTopN];
+    __shared__ unsigned long long warp_best[kMatchThreads / 32];
+    __shared__ unsigned long long s_winner;
+    const int Po = P - L + 1;
+    const int b = blockIdx.x / Q, q = blockIdx.x - b * Q;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const float fl = (float)L;
+    for (int i = tid; i < kMaxTopN; i += kMatchThreads) best[i] = 0ull;
+    if (stream_row_valid(seen, b, q, L)) {                 // block-uniform
+        const StreamRows rows(S, ring, b, Q, q, P, L, t);
+        for (int r0 = 0; r0 < Po; r0 += kCandChunk) {
+            const int nr = min(kCandChunk, Po - r0);
+            for (int i = tid; i < nr; i += kMatchThreads) {
+                const int r = r0 + i;
+                float acc = 0.0f;
+                for (int j = 0; j < L; ++j) acc += __ldg(rows.row(j) + (r + j));
+                cand[i] = ((unsigned long long)f32_orderable(__fdiv_rn(acc, fl)) << 32) | (uint32_t)r;
             }
+            __syncthreads();
+            cta_merge_chunk(cand, best, next_best, warp_best, s_winner, nr, N, tid, lane, warp);
         }
+    }
+    for (int n = tid; n < N; n += kMatchThreads) store_key(best[n], ((size_t)b * Q + q) * N + n, top_val, top_idx);
+}
+
+// After the match (stream order: it reads the slots this overwrites): the last n_app = min(Q, L - 1) new rows of
+// every stream go to their ring slots (t + q) mod (L - 1), and seen advances by Q, saturating at L - 1.
+// One CTA per (stream, appended row) at a time, 16-byte copies when rows allow them.
+__global__ void __launch_bounds__(256)
+ring_append_kernel(const float *__restrict__ S, int B, int Q, int P, int L, long long t, float *__restrict__ ring,
+                   int32_t *__restrict__ seen)
+{
+    const int Lm1 = L - 1, n_app = min(Q, Lm1);
+    const long long n_rows = (long long)B * n_app;
+    const bool vec = (P & 3) == 0 && ((reinterpret_cast<uintptr_t>(S) | reinterpret_cast<uintptr_t>(ring)) & 15) == 0;
+    for (long long i = blockIdx.x; i < n_rows; i += gridDim.x) {
+        const int b = (int)(i / n_app), k = (int)(i - (long long)b * n_app);
+        const int q = Q - n_app + k;
+        const float *src = S + ((size_t)b * Q + q) * P;
+        float *dst = ring + ((size_t)b * Lm1 + (int)((t + q) % Lm1)) * P;
+        if (vec) {
+            const float4 *s4 = reinterpret_cast<const float4 *>(src);
+            float4 *d4 = reinterpret_cast<float4 *>(dst);
+            for (int p = threadIdx.x; p < P / 4; p += blockDim.x) d4[p] = __ldg(s4 + p);
+        } else {
+            for (int p = threadIdx.x; p < P; p += blockDim.x) dst[p] = __ldg(src + p);
+        }
+        if (k == 0 && threadIdx.x == 0) seen[b] = (int32_t)min((long long)seen[b] + Q, (long long)Lm1);
     }
 }
 
@@ -624,6 +784,23 @@ extern "C" int lens_pr_counts(const float *S, const uint8_t *GT, int Po, int Qo,
     return 0;
 }
 
+// Grid of the warp-per-query kernels.  Few queries against many places (config 5: 1 024 streams x 100 000 places)
+// would leave most SMs without a warp: the places of a query are then split into n_seg segments ranked by different
+// warps, and the per-segment lists are merged by the kernel that merges per-GPU lists (same order: value desc, place
+// index desc).
+static void plan_segments(long long n_queries, int Po, int N, int &n_seg, int &seg_len, long long &blocks)
+{
+    const long long sms = std::max(sm_count(), 1), want_warps = sms * 32;
+    n_seg = 1;
+    if (n_queries < want_warps && Po >= 8192)
+        n_seg = (int)std::min<long long>(std::min<long long>(ceil_div64(want_warps, n_queries), (32 * kMergeSlots) / N),
+                                         Po / 4096);
+    n_seg = std::max(n_seg, 1);
+    seg_len = ceil_div(ceil_div(Po, n_seg), 32 * kUnrollR) * (32 * kUnrollR);
+    n_seg = ceil_div(Po, seg_len);
+    blocks = std::min<long long>((n_queries * n_seg + 7) / 8, sms * 16);
+}
+
 extern "C" int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, int N, float *D_out,
                                   float *top_val, int32_t *top_idx, void *stream)
 {
@@ -635,20 +812,10 @@ extern "C" int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, in
     if (B == 0) return 0;
     const long long n_queries = (long long)B * (Q - L + 1);
     if (N <= 32) {
-        // Few queries against many places (config 5: 1 024 streams x 100 000 places) would leave most SMs without
-        // a warp: the places of a query are then split into segments ranked by different warps, and the per-segment
-        // lists are merged by the kernel that merges per-GPU lists (same order: value desc, place index desc).
-        const int Po = P - L + 1;
-        const long long sms = std::max(sm_count(), 1), want_warps = sms * 32;
-        int n_seg = 1;
-        if (n_queries < want_warps && Po >= 8192)
-            n_seg = (int)std::min<long long>(std::min<long long>(ceil_div64(want_warps, n_queries), (32 * kMergeSlots) / N),
-                                             Po / 4096);
-        n_seg = std::max(n_seg, 1);
-        const int seg_len = ceil_div(ceil_div(Po, n_seg), 32 * kUnrollR) * (32 * kUnrollR);
-        n_seg = ceil_div(Po, seg_len);
+        int n_seg, seg_len;
+        long long blocks;
+        plan_segments(n_queries, P - L + 1, N, n_seg, seg_len, blocks);
         const long long n_work = n_queries * n_seg;
-        const long long blocks = std::min<long long>((n_work + 7) / 8, sms * 16);
         cudaStream_t st = as_stream(stream);
         if (n_seg == 1) {
             seqmatch_topk_warp_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(S, n_queries, Q, P, L, N, 1, seg_len, D_out,
@@ -672,6 +839,55 @@ extern "C" int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, in
         seqmatch_topk_kernel<<<grid, kMatchThreads, 0, as_stream(stream)>>>(S, Q, P, L, N, D_out, top_val, top_idx);
     }
     LENS_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, int L, int N, float *ring, int32_t *seen,
+                                         int64_t t, float *top_val, int32_t *top_idx, void *stream)
+{
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "lens_seqmatch_topk_stream: bad sizes");
+    LENS_CHECK_ARG(L >= 1 && L <= P, "lens_seqmatch_topk_stream: need 1 <= L <= P, got L=%d", L);
+    LENS_CHECK_ARG(N >= 1 && N <= kMaxTopN, "lens_seqmatch_topk_stream: N=%d outside [1, %d]", N, kMaxTopN);
+    LENS_CHECK_ARG(t >= 0, "lens_seqmatch_topk_stream: t must be >= 0");
+    LENS_CHECK_ARG(seen != nullptr, "lens_seqmatch_topk_stream: NULL seen");
+    LENS_CHECK_ARG(L == 1 || ring != nullptr, "lens_seqmatch_topk_stream: NULL ring needs L == 1, got L=%d", L);
+    LENS_CHECK_ARG(B == 0 || (S && top_val && top_idx), "lens_seqmatch_topk_stream: NULL buffer");
+    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "lens_seqmatch_topk_stream: too many (stream, row) pairs");
+    if (B == 0) return 0;
+    cudaStream_t st = as_stream(stream);
+    const long long n_queries = (long long)B * Q;
+    if (N <= 32) {
+        int n_seg, seg_len;
+        long long blocks;
+        plan_segments(n_queries, P - L + 1, N, n_seg, seg_len, blocks);
+        if (n_seg == 1) {
+            seqmatch_topk_stream_warp_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(
+                S, ring, seen, t, n_queries, Q, P, L, N, 1, seg_len, top_val, top_idx);
+            LENS_LAUNCH_CHECK();
+        } else {
+            float *seg_val = nullptr;                      // stream-ordered scratch, as in lens_seqmatch_topk
+            const size_t n_list = (size_t)n_queries * n_seg * N;
+            LENS_CUDA(cudaMallocAsync(&seg_val, n_list * (sizeof(float) + sizeof(int32_t)), st));
+            int32_t *seg_idx = reinterpret_cast<int32_t *>(seg_val + n_list);
+            seqmatch_topk_stream_warp_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(
+                S, ring, seen, t, n_queries, Q, P, L, N, n_seg, seg_len, seg_val, seg_idx);
+            LENS_LAUNCH_CHECK();
+            topn_merge_kernel<<<(unsigned)ceil_div64(n_queries, 8), 256, 0, st>>>(seg_val, seg_idx, n_seg, n_queries, N,
+                                                                                   top_val, top_idx);
+            LENS_LAUNCH_CHECK();
+            LENS_CUDA(cudaFreeAsync(seg_val, st));
+        }
+    } else {
+        seqmatch_topk_stream_kernel<<<(unsigned)n_queries, kMatchThreads, 0, st>>>(S, ring, seen, t, Q, P, L, N,
+                                                                                    top_val, top_idx);
+        LENS_LAUNCH_CHECK();
+    }
+    if (L > 1) {
+        const long long rows = (long long)B * std::min(Q, L - 1);
+        const long long blocks = std::min<long long>(rows, (long long)std::max(sm_count(), 1) * 16);
+        ring_append_kernel<<<(unsigned)blocks, 256, 0, st>>>(S, B, Q, P, L, t, ring, seen);
+        LENS_LAUNCH_CHECK();
+    }
     return 0;
 }
 

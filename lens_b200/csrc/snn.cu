@@ -681,6 +681,19 @@ static int forward_common(SnnHandle *h, const uint8_t *pooled, const float *xin,
     return 0;
 }
 
+// lens_snn_reset_streams: zero the membrane potentials of the masked streams, one CTA per stream at a time.
+__global__ void __launch_bounds__(256) reset_streams_kernel(const uint8_t *__restrict__ mask, int maxB, int I, int F,
+                                                            int P, float *__restrict__ v0, float *__restrict__ v1,
+                                                            float *__restrict__ v2)
+{
+    for (int b = blockIdx.x; b < maxB; b += gridDim.x) {
+        if (!mask[b]) continue;                             // block-uniform
+        for (int i = threadIdx.x; i < I; i += blockDim.x) v0[(size_t)b * I + i] = 0.0f;
+        for (int i = threadIdx.x; i < F; i += blockDim.x) v1[(size_t)b * F + i] = 0.0f;
+        for (int i = threadIdx.x; i < P; i += blockDim.x) v2[(size_t)b * P + i] = 0.0f;
+    }
+}
+
 }  // namespace lens
 
 using namespace lens;
@@ -766,6 +779,17 @@ extern "C" int lens_snn_reset(void *handle, void *stream)
     LENS_CUDA(cudaMemsetAsync(h->v2, 0, (size_t)h->maxB * h->P * sizeof(float), st));
     LENS_CUDA(cudaMemsetAsync(h->counters, 0, sizeof(int64_t), st));
     h->v0_dirty = false;
+    return 0;
+}
+
+extern "C" int lens_snn_reset_streams(void *handle, const uint8_t *mask, void *stream)
+{
+    LENS_CHECK_ARG(handle, "lens_snn_reset_streams: NULL handle");
+    LENS_CHECK_ARG(mask, "lens_snn_reset_streams: NULL mask");
+    SnnHandle *h = static_cast<SnnHandle *>(handle);
+    const int blocks = std::min(h->maxB, std::max(sm_count(), 1) * 16);
+    reset_streams_kernel<<<blocks, 256, 0, as_stream(stream)>>>(mask, h->maxB, h->I, h->F, h->P, h->v0, h->v1, h->v2);
+    LENS_LAUNCH_CHECK();
     return 0;
 }
 

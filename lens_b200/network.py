@@ -109,6 +109,15 @@ class B200Network:
     def reset_states(self):
         check(_lib.lib().lens_snn_reset(self._h, stream_ptr()), "lens_snn_reset")
 
+    @_on_device
+    def reset_streams(self, mask):
+        """reset_states() for the streams with mask[b] != 0 only (mask u8 / bool [max_streams] on the device);
+        the other streams' state and the overflow counter are untouched."""
+        require_cuda(mask)
+        if mask.dtype not in (torch.uint8, torch.bool) or mask.shape != (self.max_streams,):
+            raise LensError(f"mask must be u8 / bool [{self.max_streams}], got {mask.dtype} {tuple(mask.shape)}")
+        check(_lib.lib().lens_snn_reset_streams(self._h, ptr(mask), stream_ptr()), "lens_snn_reset_streams")
+
     def eval(self):
         return self
 

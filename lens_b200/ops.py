@@ -117,6 +117,25 @@ def seqmatch_topk(S, L, N=25, want_D=False):
     return tv, ti, D
 
 
+def seqmatch_topk_stream(S, L, N, ring, seen, t):
+    """Sequence matching across calls: S f32 [B, Q, P] = the Q new rows of B streams in lockstep ->
+    (top_val [B, Q, N], top_idx [B, Q, N]); row q is the top-N of the sequence that ends at new row q, -inf / -1
+    while its stream has seen fewer than L rows since its reset.
+
+    ring f32 [B, L - 1, P] (None iff L == 1) and seen i32 [B] are the caller's device state, updated in place (the
+    last L - 1 rows and the rows seen since each stream's reset, saturating at L - 1); t = rows pushed before this
+    call.  See lens_seqmatch_topk_stream in include/lens_b200.h."""
+    require_cuda(S, ring, seen)
+    assert S.dtype == torch.float32 and S.dim() == 3 and seen.dtype == torch.int32
+    B, Q, P = S.shape
+    assert seen.shape == (B,) and (ring is None or (ring.dtype == torch.float32 and ring.shape == (B, L - 1, P)))
+    tv = torch.empty((B, Q, N), dtype=torch.float32, device=S.device)
+    ti = torch.empty((B, Q, N), dtype=torch.int32, device=S.device)
+    check(_lib.lib().lens_seqmatch_topk_stream(ptr(S), B, Q, P, L, N, ptr(ring), ptr(seen), int(t), ptr(tv), ptr(ti),
+                                               stream_ptr()), "lens_seqmatch_topk_stream")
+    return tv, ti
+
+
 def recall_counts(top_idx, Po, gt_dense=None, gt_center=None, gt_tol=0, ns=RECALL_NS,
                   hits=None, n_valid=None):
     """Accumulate Recall@N hit counters (device int64) for top_idx [B, Qo, N].

@@ -199,6 +199,118 @@ class InferencePipeline:
         return [float(h) / nv if nv else float("nan") for h in hits.tolist()]
 
 
+class StreamingPipeline(InferencePipeline):
+    """The hot path for live cameras: a fixed fleet of `n_streams` streams that deliver a few query windows at a
+    time (one 250 ms timebin per push, typically), with sequence matching that spans the pushes.
+
+    Every push carries Q >= 1 new windows for each stream (all streams advance in lockstep).  Number a stream's
+    rows g = 0, 1, 2, ... since its last reset: new row g yields the top-N of the sequence that ends at it, once
+    the stream has seen L rows (g >= L - 1); earlier (warm-up) rows are -inf / -1.  However the windows are split
+    into pushes, the valid rows equal, bit for bit, the columns of one `step` over all of them (column g - L + 1).
+
+    The object owns the device state that makes this work: the SNN membrane potentials (as any pipeline), `ring`
+    f32 [n_streams, L - 1, P] (the last L - 1 spike-count rows of every stream, row g at slot g mod (L - 1)),
+    `seen` i32 [n_streams] (rows since each stream's reset, saturating at L - 1) and `t` (rows pushed).  Under
+    torch.distributed every rank builds one for its own shard of streams; the Recall@N counters are all-reduced
+    like `step`'s."""
+
+    def __init__(self, W_feat, W_out, roi, k, T, L, n_streams, n_top=25, ns=ops.RECALL_NS, device=None,
+                 mode=MODE_AUTO):
+        super().__init__(W_feat, W_out, roi, k, T, L, n_top=n_top, ns=ns, max_streams=n_streams, device=device,
+                         mode=mode)
+        self.n_streams = int(n_streams)
+        if self.L < 1 or self.L > self.net.P:
+            raise LensError(f"need 1 <= L <= P={self.net.P}, got L={self.L}")
+        # never read before it is written (a row is used only once its stream has seen it): left uninitialised
+        self.ring = (torch.empty((self.n_streams, self.L - 1, self.net.P), dtype=torch.float32, device=self.device)
+                     if self.L > 1 else None)
+        self.seen = torch.zeros((self.n_streams,), dtype=torch.int32, device=self.device)
+        self.t = 0
+
+    def _check_streams(self, B):
+        if B != self.n_streams:
+            raise LensError(f"this pipeline serves {self.n_streams} streams; the push has {B}")
+
+    def _check_gt(self, gt_center, Q):
+        if gt_center is not None and (not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32
+                                      or tuple(gt_center.shape) != (self.n_streams, Q)):
+            raise LensError(f"gt_center must be i32 [{self.n_streams}, {Q}]")
+
+    def _offline(self, *args, **kwargs):
+        # the batch entry points advance the SNN state without the sequence history (and a different stream count
+        # would recreate the handle): on a live session they would silently mix two timelines
+        raise LensError("StreamingPipeline is a live session: feed it with push / push_events "
+                        "(use an InferencePipeline for batch steps)")
+
+    step = step_events = step_event_groups = step_host = _offline
+
+    def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True):
+        """Q new windows of every stream: frames u8 [B, Q, roi, roi] or pooled u8 [B, Q, I], B = n_streams.
+        -> `step`'s dict with top_val / top_idx [B, Q, N] (row q = the sequence ending at new row q), S [B, Q, P],
+        and hits / n_valid for this push.  gt_center i32 [B, Q] (optional) is the expected place of the sequence
+        ending at each new row (band ground truth, |idx - center| <= gt_tol); warm-up rows never count."""
+        x = frames if frames is not None else pooled
+        if x is None or (frames is not None and pooled is not None):
+            raise LensError("give exactly one of frames / pooled")
+        self._check_streams(x.shape[0])
+        self._check_gt(gt_center, x.shape[1])
+        with torch.cuda.device(self.device):
+            S = self.similarity(frames=frames, pooled=pooled)
+            tv, ti = ops.seqmatch_topk_stream(S, self.L, self.n_top, self.ring, self.seen, self.t)
+            self.t += S.shape[1]
+            out = dict(top_val=tv, top_idx=ti, D=None, hits=None, n_valid=None, S=S,
+                       overflow=self.net.overflow_tensor())
+            if gt_center is not None:
+                gt = torch.where(ti[..., 0] >= 0, gt_center, -1)      # warm-up rows: no ground truth
+                out["hits"], out["n_valid"] = ops.recall_counts(ti, S.shape[2] - self.L + 1, gt_center=gt,
+                                                                gt_tol=gt_tol, ns=self.ns)
+        if reduce:
+            self._all_reduce_hits(out)
+        return out
+
+    def push_events(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0=0, roi_y0=0, gt_center=None, gt_tol=0,
+                    reduce=True):
+        """`push` fed from raw events: the next Q windows of every stream, window q of stream b covering
+        [t0_us[b] + q * window_us, + window_us) of its events [offsets[b], offsets[b+1]) (as in `step_events`).
+        Returns `push`'s dict plus "events_per_window" i32 [B, Q]."""
+        self._check_streams(offsets.numel() - 1)
+        self._check_gt(gt_center, int(Q))
+        with torch.cuda.device(self.device):
+            pooled, n_ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
+            out = self.push(pooled=pooled, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce)
+        out["events_per_window"] = n_ev
+        return out
+
+    def reset_streams(self, streams):
+        """Restart some streams (a camera that rebooted or dropped out): their SNN state and their sequence
+        history.  `streams` is a bool mask [n_streams] (tensor or sequence of bools) or integer stream indices
+        (tensor or sequence).  Their next L - 1 rows are warm-up rows again; the other streams are untouched."""
+        is_tensor = torch.is_tensor(streams)
+        items = streams.reshape(-1).tolist() if is_tensor else list(streams)
+        if (streams.dtype == torch.bool) if is_tensor else (items and all(isinstance(v, bool) for v in items)):
+            if len(items) != self.n_streams:
+                raise LensError(f"a mask must have {self.n_streams} entries, got {len(items)}")
+            mask = torch.tensor(items, dtype=torch.bool)
+        else:
+            if (is_tensor and (streams.dtype == torch.uint8 or streams.dtype.is_floating_point)) or \
+                    any(isinstance(v, bool) or not isinstance(v, int) for v in items):
+                raise LensError("give a bool mask or integer stream indices (a u8 tensor is ambiguous)")
+            if any(v < 0 or v >= self.n_streams for v in items):
+                raise LensError(f"stream indices must lie in [0, {self.n_streams})")
+            mask = torch.zeros((self.n_streams,), dtype=torch.bool)
+            mask[torch.tensor(items, dtype=torch.int64)] = True
+        with torch.cuda.device(self.device):
+            mask = mask.to(self.device)
+            self.net.reset_streams(mask)
+            self.seen.masked_fill_(mask, 0)
+
+    def reset(self):
+        """Every stream from scratch: SNN state (and the overflow counter), sequence history, and t."""
+        self.net.reset_states()
+        self.seen.zero_()
+        self.t = 0
+
+
 class PlaceShardedPipeline:
     """The same hot path with the DATABASE sharded across ranks instead of the streams (SURVEY.md 8e, the
     alternative for few streams / very large databases): every rank runs ALL streams against its own range
