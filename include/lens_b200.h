@@ -255,15 +255,18 @@ int lens_recall_bounds(const float *D, const uint8_t *GT, int Po, int Qo, const 
  * lens/run_model.py:319-327 with n_thresh = 100.  S and GT are [Po][Qo] (rows = database), exactly the
  * matrices the reference passes (after its transposes).  Per query column the best match is the FIRST
  * row attaining the maximum (np.argmax); thresholds are np.linspace(max, min, n_thresh) over the best
- * similarities, evaluated in float64 like numpy.
+ * similarities, evaluated like numpy (>= 2.0) in the dtype of the caller's matrix: thresh_f64 = 0 for a
+ * float32 matrix (float32 arithmetic and comparison), 1 for float64, integer or bool matrices (float64;
+ * exact when every value is representable in float32, the type S is read in).
  *   tp, fp [n_thresh] i64 device: true / false positives with best >= threshold
  *   gtp    [1] i64 device: number of queries that have a positive at all (GT.any(0))             */
 int lens_pr_counts(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
-                   int64_t *fp, int64_t *gtp, void *stream);
+                   int64_t *fp, int64_t *gtp, void *stream, int thresh_f64);
 /* The same for matching='multi' (lens/src/metrics.py:63-91): every entry of S counts, thresholds are
- * np.linspace(S.max(), S.min(), n_thresh), gtp = count_nonzero(GT).  tp, fp, gtp are overwritten.          */
+ * np.linspace(S.max(), S.min(), n_thresh) (thresh_f64 as above), gtp = count_nonzero(GT).  tp, fp, gtp are
+ * overwritten.                                                                                              */
 int lens_pr_counts_multi(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
-                         int64_t *fp, int64_t *gtp, void *stream);
+                         int64_t *fp, int64_t *gtp, void *stream, int thresh_f64);
 
 /* Sum-of-absolute-differences baseline, lens/src/sad.py:25-42: dist[q][r] = sum_p |a[q][p] - b[r][p]|
  * (torch.cdist(a, b, p=1) on float32 copies of uint8 frames; the sums are integers < 2^24, hence exact

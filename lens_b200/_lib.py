@@ -51,8 +51,8 @@ def _declare(L):
         "lens_online_match": (i32, [vp, i32, i32, i32, vp, vp, vp]),
         "lens_event_windows": (i32, [vp, vp, vp, i64, vp, i32, i32, i32, f64, f64, i64, vp, vp, vp, vp, vp, vp]),
         "lens_bin_events_lut": (i32, [vp, vp, vp, i32, i32, vp, vp, i64, i32, i32, i64, vp, vp, vp]),
-        "lens_pr_counts": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, vp]),
-        "lens_pr_counts_multi": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, vp]),
+        "lens_pr_counts": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, vp, i32]),
+        "lens_pr_counts_multi": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, vp, i32]),
         "lens_recall": (i32, [vp, i32, i32, i32, i32, vp, i64, vp, i32, pi32, i32, vp, vp, vp]),
         "lens_recall_bounds": (i32, [vp, vp, i32, i32, pi32, i32, vp, vp, vp, vp]),
         "lens_topn_merge": (i32, [vp, vp, i32, i64, i32, vp, vp, vp]),

@@ -545,10 +545,31 @@ __global__ void __launch_bounds__(256) recall_bounds_kernel(BoundsParams p)
     }
 }
 
+// Threshold i of np.linspace(start, stop, n) with start = max, stop = min of createPR's values.  numpy (>= 2.0)
+// evaluates it in the dtype of those values: float64 for float64, integer and bool matrices (f64 != 0), float32 for
+// float32 ones.  Each operation is rounded on its own, like numpy's sequence of array operations, hence the
+// explicit intrinsics (no FMA contraction):
+//   step = (stop - start) / (n - 1);  y_i = i * step + start,  or, when step underflows to 0 (denormal ranges),
+//   y_i = (i / (n - 1)) * (stop - start) + start;  the last element is stop.
+// The float32 threshold is returned widened to float64, which is exact, so `(double)v >= t` is the float32
+// comparison numpy makes.  The float64 branch never sees step == 0 unless start == stop, where both forms give start.
+__device__ __forceinline__ double pr_threshold(int i, int n, float start, float stop, bool f64)
+{
+    if (f64) {
+        const double step = __ddiv_rn(__dsub_rn((double)stop, (double)start), (double)(n - 1));
+        return (i == n - 1) ? (double)stop : __dadd_rn(__dmul_rn((double)i, step), (double)start);
+    }
+    const float div = (float)(n - 1), delta = __fsub_rn(stop, start);
+    const float step = __fdiv_rn(delta, div);
+    if (i == n - 1) return (double)stop;
+    if (step == 0.0f) return (double)__fadd_rn(__fmul_rn(__fdiv_rn((float)i, div), delta), start);
+    return (double)__fadd_rn(__fmul_rn((float)i, step), start);
+}
+
 // createPR, matching = 'single' (lens/src/metrics.py:21-139): one CTA, columns strided over threads.
 // best[q] / hit[q] live in shared memory (Qo <= 8192).
 __global__ void __launch_bounds__(256) pr_counts_kernel(const float *__restrict__ S, const uint8_t *__restrict__ GT,
-                                                        int Po, int Qo, int n_thresh,
+                                                        int Po, int Qo, int n_thresh, int thresh_f64,
                                                         unsigned long long *__restrict__ tp,
                                                         unsigned long long *__restrict__ fp,
                                                         unsigned long long *__restrict__ gtp)
@@ -583,12 +604,8 @@ __global__ void __launch_bounds__(256) pr_counts_kernel(const float *__restrict_
     if ((threadIdx.x & 31) == 0) { s_max[threadIdx.x >> 5] = vmax; s_min[threadIdx.x >> 5] = vmin; atomicAdd(&s_gtp, my_gtp); }
     __syncthreads();
     for (int i = 0; i < 8; ++i) { vmax = fmaxf(vmax, s_max[i]); vmin = fminf(vmin, s_min[i]); }
-    // np.linspace(start, stop, n): y_i = i * step + start in float64, last element = stop
-    const double start = (double)vmax, stop = (double)vmin;
-    const double step = __ddiv_rn(__dsub_rn(stop, start), (double)(n_thresh - 1));
     for (int i = threadIdx.x; i < n_thresh; i += blockDim.x) {
-        // numpy: y = arange(n) * step; y += start  (two separately rounded float64 operations, no FMA)
-        const double t = (i == n_thresh - 1) ? stop : __dadd_rn(__dmul_rn((double)i, step), start);
+        const double t = pr_threshold(i, n_thresh, vmax, vmin, thresh_f64 != 0);
         unsigned long long a = 0, b = 0;
         for (int q = 0; q < Qo; ++q) {
             if ((double)s_best[q] >= t) { if (s_hit[q]) ++a; else ++b; }
@@ -601,7 +618,7 @@ __global__ void __launch_bounds__(256) pr_counts_kernel(const float *__restrict_
 // createPR, matching = 'multi' (lens/src/metrics.py:63-91): every entry of the matrix counts.  Pass 1: extreme
 // values (as order-preserving integers) and the number of ground-truth positives; pass 2: one CTA per (threshold,
 // slice of the matrix) counts the entries >= threshold that are / are not positives.  Thresholds as in the
-// 'single' kernel: np.linspace(max, min, n) evaluated in float64 without FMA contraction.
+// 'single' kernel (pr_threshold).
 __global__ void __launch_bounds__(256) pr_multi_minmax_kernel(const float *__restrict__ S, const uint8_t *__restrict__ GT,
                                                               long long n, unsigned int *__restrict__ mm,
                                                               unsigned long long *__restrict__ gtp)
@@ -624,14 +641,13 @@ __global__ void __launch_bounds__(256) pr_multi_minmax_kernel(const float *__res
 }
 
 __global__ void __launch_bounds__(256) pr_multi_counts_kernel(const float *__restrict__ S, const uint8_t *__restrict__ GT,
-                                                              long long n, int n_thresh, const unsigned int *__restrict__ mm,
+                                                              long long n, int n_thresh, int thresh_f64,
+                                                              const unsigned int *__restrict__ mm,
                                                               unsigned long long *__restrict__ tp,
                                                               unsigned long long *__restrict__ fp)
 {
     const int i = blockIdx.x;
-    const double start = (double)f32_from_orderable(mm[0]), stop = (double)f32_from_orderable(mm[1]);
-    const double step = __ddiv_rn(__dsub_rn(stop, start), (double)(n_thresh - 1));
-    const double t = (i == n_thresh - 1) ? stop : __dadd_rn(__dmul_rn((double)i, step), start);
+    const double t = pr_threshold(i, n_thresh, f32_from_orderable(mm[0]), f32_from_orderable(mm[1]), thresh_f64 != 0);
     const long long per = ceil_div64(n, gridDim.y), e0 = per * blockIdx.y, e1 = min(n, e0 + per);
     unsigned long long a = 0, b = 0;
     for (long long e = e0 + threadIdx.x; e < e1; e += blockDim.x)
@@ -772,13 +788,13 @@ extern "C" int lens_reciprocal(const float *in, int64_t n, float *out, void *str
 }
 
 extern "C" int lens_pr_counts(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
-                              int64_t *fp, int64_t *gtp, void *stream)
+                              int64_t *fp, int64_t *gtp, void *stream, int thresh_f64)
 {
     LENS_CHECK_ARG(S && GT && tp && fp && gtp, "lens_pr_counts: NULL buffer");
     LENS_CHECK_ARG(Po > 0 && Qo > 0 && Qo <= 8192, "lens_pr_counts: need 0 < Qo <= 8192, Po > 0");
     LENS_CHECK_ARG(n_thresh > 1, "lens_pr_counts: n_thresh must be > 1");
     pr_counts_kernel<<<1, 256, (size_t)Qo * 5, as_stream(stream)>>>(
-        S, GT, Po, Qo, n_thresh, reinterpret_cast<unsigned long long *>(tp),
+        S, GT, Po, Qo, n_thresh, thresh_f64, reinterpret_cast<unsigned long long *>(tp),
         reinterpret_cast<unsigned long long *>(fp), reinterpret_cast<unsigned long long *>(gtp));
     LENS_LAUNCH_CHECK();
     return 0;
@@ -954,7 +970,7 @@ extern "C" int lens_topn_merge(const float *val, const int32_t *idx, int W, int6
 }
 
 extern "C" int lens_pr_counts_multi(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
-                                    int64_t *fp, int64_t *gtp, void *stream)
+                                    int64_t *fp, int64_t *gtp, void *stream, int thresh_f64)
 {
     LENS_CHECK_ARG(Po > 0 && Qo > 0, "lens_pr_counts_multi: bad sizes");
     LENS_CHECK_ARG(n_thresh > 1 && n_thresh <= 65535, "lens_pr_counts_multi: n_thresh must be in (1, 65535]");
@@ -973,7 +989,8 @@ extern "C" int lens_pr_counts_multi(const float *S, const uint8_t *GT, int Po, i
     LENS_LAUNCH_CHECK();
     const int slices = (int)std::max<long long>(1, std::min<long long>(ceil_div64(n, 65536), 64));
     pr_multi_counts_kernel<<<dim3((unsigned)n_thresh, (unsigned)slices), 256, 0, st>>>(
-        S, GT, n, n_thresh, mm, reinterpret_cast<unsigned long long *>(tp), reinterpret_cast<unsigned long long *>(fp));
+        S, GT, n, n_thresh, thresh_f64, mm, reinterpret_cast<unsigned long long *>(tp),
+        reinterpret_cast<unsigned long long *>(fp));
     LENS_LAUNCH_CHECK();
     LENS_CUDA(cudaFreeAsync(mm, st));
     return 0;

@@ -92,13 +92,25 @@ def createPR(S_in, GThard, outputdir=None, datatype="LENS", GTsoft=None, matchin
     """Precision / recall lists of lens/src/metrics.py:21-139: matching='single' (best match per query, the mode
     the reference's inference path uses, lens/run_model.py:321) or 'multi' (every entry of the matrix, the
     reference's default).  S_in, GThard: numpy [database, query].  Returns (P, R): python lists of length
-    n_thresh + 1 starting with P = 1, R = 0.  The figure the reference saves on the last threshold is not produced."""
+    n_thresh + 1 starting with P = 1, R = 0.  The figure the reference saves on the last threshold is not produced.
+
+    The thresholds are np.linspace(max, min, n_thresh), which numpy (>= 2.0) evaluates in the matrix's own type:
+    float32 arithmetic for a float32 S_in, float64 for float64, integer and bool ones.  The kernels read S_in as
+    float32, so a float64 S_in gives the reference's lists only when every value is representable in float32 (the
+    spike-count averages and SAD similarities of this package are).  Other dtypes (float16, longdouble, ...) raise
+    ValueError."""
     from .._lib import lib, check, ptr, stream_ptr
     S_in, GThard = np.asarray(S_in), np.asarray(GThard)
     assert S_in.shape == GThard.shape, "S_in, GThard and GTsoft must have the same shape"
     assert S_in.ndim == 2, "S_in, GThard and GTsoft must be two-dimensional"
     assert matching in ("single", "multi"), "matching should contain one of the following strings: [single, multi]"
     assert n_thresh > 1, "n_thresh must be >1"
+    if S_in.dtype == np.float32:
+        thresh_f64 = 0
+    elif S_in.dtype == np.float64 or S_in.dtype.kind in "biu":
+        thresh_f64 = 1
+    else:
+        raise ValueError(f"createPR: S_in of dtype {S_in.dtype} is not supported (float32, float64, integer or bool)")
     GT = GThard.astype(bool)
     S = S_in.astype(np.float32, copy=True)
     if GTsoft is not None:
@@ -111,11 +123,11 @@ def createPR(S_in, GThard, outputdir=None, datatype="LENS", GTsoft=None, matchin
     fp = torch.zeros(n_thresh, dtype=torch.int64, device="cuda")
     gtp = torch.zeros(1, dtype=torch.int64, device="cuda")
     if matching == "single":
-        check(lib().lens_pr_counts(ptr(dS), ptr(dG), Po, Qo, n_thresh, ptr(tp), ptr(fp), ptr(gtp), stream_ptr()),
-              "lens_pr_counts")
+        check(lib().lens_pr_counts(ptr(dS), ptr(dG), Po, Qo, n_thresh, ptr(tp), ptr(fp), ptr(gtp), stream_ptr(),
+                                   thresh_f64), "lens_pr_counts")
     else:
-        check(lib().lens_pr_counts_multi(ptr(dS), ptr(dG), Po, Qo, n_thresh, ptr(tp), ptr(fp), ptr(gtp), stream_ptr()),
-              "lens_pr_counts_multi")
+        check(lib().lens_pr_counts_multi(ptr(dS), ptr(dG), Po, Qo, n_thresh, ptr(tp), ptr(fp), ptr(gtp), stream_ptr(),
+                                         thresh_f64), "lens_pr_counts_multi")
     tp, fp, gtp = tp.cpu().numpy(), fp.cpu().numpy(), int(gtp.item())
     P, R = [1], [0]
     with np.errstate(divide="ignore", invalid="ignore"):
