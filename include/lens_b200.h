@@ -28,6 +28,8 @@
  *                          N <= 64, 1 <= L <= P, Q >= 1, B * Q <= 2^31 - 1; ring non-NULL unless L == 1, seen non-NULL
  *   lens_recall / _bounds  at most 8 values of N per call
  *   lens_pr_counts         Qo <= 8192 (one CTA, shared-memory resident)
+ *   lens_seqpr_scan / _counts
+ *                          1 <= L <= min(Q, P), 2 <= n_thresh <= 4096 (table and histograms in 48 KB of shared memory)
  *   lens_sad_matrix        npix <= 65 793 (sums stay exact in fp32)
  *   lens_topn_merge        W * N <= 512
  *   lens_bin_events        t_us ascending (lens_check_sorted_u32), x / y 16-byte aligned
@@ -267,6 +269,39 @@ int lens_pr_counts(const float *S, const uint8_t *GT, int Po, int Qo, int n_thre
  * overwritten.                                                                                              */
 int lens_pr_counts_multi(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
                          int64_t *fp, int64_t *gtp, void *stream, int thresh_f64);
+
+/* Fleet precision-recall: createPR's counts for B streams, straight from the spike counts S [B][Q][P] f32.
+ * D_b[p][q] = (sum_{j<L} S[b][q+j][p+j]) / L is recomputed exactly as lens_seqmatch_topk computes it and never
+ * written.  The fleet's matrix is the streams' matrices concatenated along createPR's column axis:
+ *   LENS_SEQPR_PLACE  createPR(D_b.T, GT_b.T, 'single') at B = 1 (lens/run_model.py:321): a column per (stream,
+ *                     place), its best query is the FIRST maximum (lowest query index); gtp = places with a positive
+ *   LENS_SEQPR_QUERY  createPR(D_b, GT_b, 'single') at B = 1 (the SAD path, lens/src/sad.py): a column per (stream,
+ *                     query), its best place is the first maximum (lowest place index); gtp = queries with a positive
+ *   LENS_SEQPR_MULTI  createPR(D_b, GT_b, 'multi'): every entry; gtp = positive entries
+ * Thresholds: np.linspace(max, min, n_thresh) of the float32 values (numpy's float32 recipe, as lens_pr_counts
+ * with thresh_f64 = 0) over the whole fleet.  Ground truth as lens_recall: gt_dense [B or 1][Po][Qo] u8
+ * (gt_stream_stride = Po*Qo, or 0 to share one matrix) or gt_center [B][Qo] i32 (< 0: no positive; else the
+ * places |p - center| <= gt_tol), exactly one non-NULL.  Finite S only.
+ *   lens_seqpr_records_bytes  *bytes (host) = the records a call needs: 5*B*Po (place), 9*B*Qo (query), 0 (multi)
+ *   lens_seqpr_scan    one read of S (and GT).  records [bytes] 8-byte aligned, written (NULL allowed in multi
+ *                      mode); extremes [2] u64 = {max key, ~min key} of the order-preserving float keys, MERGED by
+ *                      max (zero them before the first call); gtp [1] i64 ACCUMULATED.  Groups of streams (or ranks,
+ *                      by an all-reduce MAX of extremes) scanned into one extremes / gtp form one fleet.
+ *   lens_seqpr_counts  thresholds from the merged extremes; every record (multi: every entry, a second read of
+ *                      S) binned once.  tp, fp [n_thresh] i64 ACCUMULATED: true / false positives with value >=
+ *                      threshold i.  The same S, sizes, mode, GT and records as the scan.
+ * One launch per scan (two in query mode) and two per count, whatever B; stream-ordered scratch of 16 B per
+ * threshold in lens_seqpr_counts.  B = 0 returns 0 without launching.                                        */
+#define LENS_SEQPR_PLACE 0
+#define LENS_SEQPR_QUERY 1
+#define LENS_SEQPR_MULTI 2
+int lens_seqpr_records_bytes(int B, int Q, int P, int L, int mode, int64_t *bytes);
+int lens_seqpr_scan(const float *S, int B, int Q, int P, int L, int mode, const uint8_t *gt_dense,
+                    int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, void *records,
+                    uint64_t *extremes, int64_t *gtp, void *stream);
+int lens_seqpr_counts(const float *S, int B, int Q, int P, int L, int mode, const uint8_t *gt_dense,
+                      int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, const void *records,
+                      const uint64_t *extremes, int n_thresh, int64_t *tp, int64_t *fp, void *stream);
 
 /* Sum-of-absolute-differences baseline, lens/src/sad.py:25-42: dist[q][r] = sum_p |a[q][p] - b[r][p]|
  * (torch.cdist(a, b, p=1) on float32 copies of uint8 frames; the sums are integers < 2^24, hence exact

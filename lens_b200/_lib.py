@@ -56,6 +56,9 @@ def _declare(L):
         "lens_recall": (i32, [vp, i32, i32, i32, i32, vp, i64, vp, i32, pi32, i32, vp, vp, vp]),
         "lens_recall_bounds": (i32, [vp, vp, i32, i32, pi32, i32, vp, vp, vp, vp]),
         "lens_topn_merge": (i32, [vp, vp, i32, i64, i32, vp, vp, vp]),
+        "lens_seqpr_records_bytes": (i32, [i32, i32, i32, i32, i32, pi64]),
+        "lens_seqpr_scan": (i32, [vp, i32, i32, i32, i32, i32, vp, i64, vp, i32, vp, vp, vp, vp]),
+        "lens_seqpr_counts": (i32, [vp, i32, i32, i32, i32, i32, vp, i64, vp, i32, vp, vp, i32, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)          # AttributeError if the .so lacks a declared symbol

@@ -662,6 +662,287 @@ __global__ void __launch_bounds__(256) pr_multi_counts_kernel(const float *__res
     }
 }
 
+// ---- fleet precision-recall (lens_seqpr_scan / lens_seqpr_counts) --------------------------------------------
+// createPR's counts over the sequence-matched matrices of B streams, recomputed from S as K4 does (D is never
+// written).  The columns of the fleet are those of np.concatenate([D_b.T] or [D_b], axis=1): per place (b, p),
+// per query (b, q), or every entry (multi).  Scan: one read of S; per-column records, the extremes as
+// order-preserving keys {max, ~min} (merged with atomicMax, so groups and ranks combine by max) and gtp.
+// Count: the thresholds of the merged extremes in shared memory, every record (or entry, re-read) binned once,
+// then prefix sums into tp / fp.
+constexpr int kPrPlace = LENS_SEQPR_PLACE, kPrQuery = LENS_SEQPR_QUERY, kPrMulti = LENS_SEQPR_MULTI;
+constexpr int kPrTile = 32 * kUnrollR;    // places per warp item
+constexpr int kPrMaxThresh = 4096;        // 12 B per threshold of shared memory: table + two histograms
+
+struct SeqPrArgs {
+    const float *S;
+    int B, Q, P, L, Qo, Po;
+    const uint8_t *gt_dense;
+    int64_t gt_stride;
+    const int32_t *gt_center;
+    int gt_tol;
+    float *rec_val;                  // per place: [B * Po] best value over the queries
+    unsigned long long *rec_key;     // per query: [B * Qo] orderable(best) << 32 | ~place
+    uint8_t *rec_flag;               // [B * Po] GT at the first maximum (per place) / [B * Qo] any positive (per query)
+    unsigned long long *ext;         // {max key, ~min key}
+    unsigned long long *gtp;
+    int n_thresh;
+    unsigned long long *hist;        // count pass: [2][n_thresh] positives | negatives per bin
+};
+
+__device__ __forceinline__ bool seqpr_positive(const SeqPrArgs &a, int b, int p, int q, int center)
+{
+    if (a.gt_dense) return __ldg(a.gt_dense + (size_t)b * a.gt_stride + (size_t)p * a.Qo + q) != 0;
+    return center >= 0 && abs(p - center) <= a.gt_tol;
+}
+
+__device__ __forceinline__ int seqpr_center(const SeqPrArgs &a, int b, int q)
+{
+    return a.gt_dense ? 0 : __ldg(a.gt_center + (size_t)b * a.Qo + q);
+}
+
+// D_b[p][q] for the places p0 + 32 u + lane of one tile, as K4 computes it (exact integer partial sums, one IEEE
+// division); loads coalesced along the places, four batches of L terms in flight.
+__device__ __forceinline__ void seqpr_tile_values(const SeqPrArgs &a, const float *Sb, int q, int p0, int lane,
+                                                  float (&d)[kUnrollR])
+{
+    float acc[kUnrollR];
+#pragma unroll
+    for (int u = 0; u < kUnrollR; ++u) acc[u] = 0.0f;
+    const float *base = Sb + (size_t)q * a.P + p0 + lane;
+    if (p0 + kPrTile <= a.Po) {
+        for (int j = 0; j < a.L; ++j) {
+            const float *row = base + (size_t)j * a.P + j;
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) acc[u] += __ldg(row + 32 * u);
+        }
+    } else {
+        for (int j = 0; j < a.L; ++j) {
+            const float *row = base + (size_t)j * a.P + j;
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u)
+                if (p0 + 32 * u + lane < a.Po) acc[u] += __ldg(row + 32 * u);
+        }
+    }
+    const float fl = (float)a.L;
+#pragma unroll
+    for (int u = 0; u < kUnrollR; ++u) d[u] = __fdiv_rn(acc[u], fl);
+}
+
+// Warp-wide merge of a warp's extremes (orderable keys, 0 / ~0 = none) and positives into the caller's totals.
+__device__ __forceinline__ void seqpr_merge_extremes(const SeqPrArgs &a, unsigned kmax, unsigned kmin,
+                                                     unsigned long long pos, int lane)
+{
+    kmax = __reduce_max_sync(0xffffffffu, kmax);
+    kmin = __reduce_min_sync(0xffffffffu, kmin);
+    for (int o = 16; o > 0; o >>= 1) pos += __shfl_xor_sync(0xffffffffu, pos, o);
+    if (lane == 0) {
+        if (kmax) {
+            atomicMax(a.ext, (unsigned long long)kmax);
+            atomicMax(a.ext + 1, (unsigned long long)(~kmin));
+        }
+        if (pos) atomicAdd(a.gtp, pos);
+    }
+}
+
+// Scan pass.  One warp per (stream, tile of kPrTile places), queries in ascending order.  48 registers (five CTAs
+// per SM): capped at 40 like K4, the per-place and multi forms spill.
+template <int kMode>
+__global__ void __launch_bounds__(256, 5) seqpr_scan_kernel(SeqPrArgs a)
+{
+    const int lane = threadIdx.x & 31;
+    const long long warp0 = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    const long long n_tiles = ceil_div(a.Po, kPrTile), n_items = (long long)a.B * n_tiles;
+    unsigned kmax = 0u, kmin = 0xffffffffu;
+    unsigned long long pos = 0;
+    for (long long w = warp0; w < n_items; w += n_warps) {
+        const int b = (int)(w / n_tiles), p0 = (int)(w - (long long)b * n_tiles) * kPrTile;
+        const float *Sb = a.S + (size_t)b * a.Q * a.P;
+        float best[kUnrollR];
+        bool hit[kUnrollR], any[kUnrollR];
+#pragma unroll
+        for (int u = 0; u < kUnrollR; ++u) { best[u] = 0.0f; hit[u] = any[u] = false; }
+        for (int q = 0; q < a.Qo; ++q) {
+            float d[kUnrollR];
+            seqpr_tile_values(a, Sb, q, p0, lane, d);
+            const int c = seqpr_center(a, b, q);
+            unsigned long long kq = 0ull;
+            bool anyq = false;
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) {
+                const int p = p0 + 32 * u + lane;
+                if (p >= a.Po) continue;
+                const bool g = seqpr_positive(a, b, p, q, c);
+                if (kMode == kPrPlace) {
+                    if (q == 0 || d[u] > best[u]) { best[u] = d[u]; hit[u] = g; }   // strict: first maximum
+                    any[u] |= g;
+                } else if (kMode == kPrQuery) {
+                    // ~p: among equal values the lowest place wins (np.argmax); -0 keyed as +0, which numpy ties
+                    const unsigned long long k =
+                        ((unsigned long long)f32_orderable(__fadd_rn(d[u], 0.0f)) << 32) | (uint32_t)~p;
+                    kq = k > kq ? k : kq;
+                    anyq |= g;
+                } else {
+                    const unsigned o = f32_orderable(d[u]);
+                    kmax = max(kmax, o); kmin = min(kmin, o);
+                    pos += g;
+                }
+            }
+            if (kMode == kPrQuery) {
+                for (int o = 16; o > 0; o >>= 1) {
+                    const unsigned long long other = shfl_xor_u64(kq, o);
+                    kq = other > kq ? other : kq;
+                }
+                anyq = __any_sync(0xffffffffu, anyq);
+                if (lane == 0) {
+                    const size_t r = (size_t)b * a.Qo + q;
+                    atomicMax(a.rec_key + r, kq);
+                    if (anyq) a.rec_flag[r] = 1;
+                }
+            }
+        }
+        if (kMode == kPrPlace) {
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) {
+                const int p = p0 + 32 * u + lane;
+                if (p >= a.Po) continue;
+                const size_t r = (size_t)b * a.Po + p;
+                a.rec_val[r] = best[u];
+                a.rec_flag[r] = hit[u];
+                const unsigned o = f32_orderable(best[u]);
+                kmax = max(kmax, o); kmin = min(kmin, o);
+                pos += any[u];
+            }
+        }
+    }
+    if (kMode != kPrQuery) seqpr_merge_extremes(a, kmax, kmin, pos, lane);
+}
+
+// Per-query records are final only once every tile has merged into them: their extremes and gtp come after.
+__global__ void __launch_bounds__(256) seqpr_query_extremes_kernel(SeqPrArgs a)
+{
+    const long long n = (long long)a.B * a.Qo;
+    unsigned kmax = 0u, kmin = 0xffffffffu;
+    unsigned long long pos = 0;
+    for (long long i0 = blockIdx.x * (long long)blockDim.x; i0 < n; i0 += (long long)gridDim.x * blockDim.x) {
+        const long long i = i0 + threadIdx.x;
+        if (i < n) {
+            const unsigned o = (unsigned)(a.rec_key[i] >> 32);
+            kmax = max(kmax, o); kmin = min(kmin, o);
+            pos += a.rec_flag[i];
+        }
+    }
+    seqpr_merge_extremes(a, kmax, kmin, pos, threadIdx.x & 31);
+}
+
+// Bin of value v: the first k <= n - 2 with y[k] <= v, else n - 1.  The float32 table is non-increasing over
+// 0 .. n - 2 (each step a monotone operation, monotonically rounded); only y[n - 1] = stop can break the order, and
+// every value is >= stop (the minimum of the very values binned), so threshold n - 1 counts everything.
+__device__ __forceinline__ int seqpr_bin(const float *y, int n, float v)
+{
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (y[mid] <= v) hi = mid; else lo = mid + 1;
+    }
+    return lo;
+}
+
+// Every lane of the warp calls this; lanes with the same (bin, hit) add once (spike-count D takes few values).
+__device__ __forceinline__ void seqpr_add(unsigned *h, int n, bool valid, int bin, bool hit, int lane)
+{
+    const unsigned key = valid ? ((unsigned)bin << 1 | (unsigned)hit) : 0xffffffffu;
+    const unsigned peers = __match_any_sync(0xffffffffu, key);
+    if (valid && __ffs(peers) - 1 == lane) atomicAdd(h + (hit ? 0 : n) + bin, (unsigned)__popc(peers));
+}
+
+// Count pass: histograms per CTA in shared memory ([n] thresholds, [2][n] counts), merged into a.hist.
+template <int kMode>
+__global__ void __launch_bounds__(256, 5) seqpr_count_kernel(SeqPrArgs a)
+{
+    extern __shared__ float s_y[];
+    unsigned *s_h = reinterpret_cast<unsigned *>(s_y + a.n_thresh);
+    const int n = a.n_thresh, lane = threadIdx.x & 31;
+    const float start = f32_from_orderable((uint32_t)a.ext[0]), stop = f32_from_orderable(~(uint32_t)a.ext[1]);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        s_y[i] = (float)pr_threshold(i, n, start, stop, false);
+        s_h[i] = s_h[n + i] = 0u;
+    }
+    __syncthreads();
+    if (kMode == kPrMulti) {
+        const long long warp0 = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+        const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
+        const long long n_tiles = ceil_div(a.Po, kPrTile), n_items = (long long)a.B * n_tiles;
+        for (long long w = warp0; w < n_items; w += n_warps) {
+            const int b = (int)(w / n_tiles), p0 = (int)(w - (long long)b * n_tiles) * kPrTile;
+            const float *Sb = a.S + (size_t)b * a.Q * a.P;
+            for (int q = 0; q < a.Qo; ++q) {
+                float d[kUnrollR];
+                seqpr_tile_values(a, Sb, q, p0, lane, d);
+                const int c = seqpr_center(a, b, q);
+#pragma unroll
+                for (int u = 0; u < kUnrollR; ++u) {
+                    const int p = p0 + 32 * u + lane;
+                    const bool valid = p < a.Po;
+                    const bool g = valid && seqpr_positive(a, b, p, q, c);
+                    seqpr_add(s_h, n, valid, valid ? seqpr_bin(s_y, n, d[u]) : 0, g, lane);
+                }
+            }
+        }
+    } else {
+        // records: four per thread and iteration, loads first; every lane runs the same number of iterations
+        constexpr int kPer = 4;
+        const long long n_rec = (long long)a.B * (kMode == kPrPlace ? a.Po : a.Qo);
+        const long long stride = (long long)gridDim.x * blockDim.x;
+        for (long long i0 = blockIdx.x * (long long)blockDim.x; i0 < n_rec; i0 += stride * kPer) {
+            float v[kPer];
+            bool g[kPer], valid[kPer];
+#pragma unroll
+            for (int k = 0; k < kPer; ++k) {
+                const long long i = i0 + k * stride + threadIdx.x;
+                valid[k] = i < n_rec;
+                v[k] = 0.0f; g[k] = false;
+                if (!valid[k]) continue;
+                if (kMode == kPrPlace) {
+                    v[k] = a.rec_val[i];
+                    g[k] = a.rec_flag[i] != 0;
+                } else {
+                    const unsigned long long key = a.rec_key[i];
+                    const int b = (int)(i / a.Qo), q = (int)(i - (long long)b * a.Qo);
+                    v[k] = f32_from_orderable((uint32_t)(key >> 32));
+                    g[k] = seqpr_positive(a, b, (int)~(uint32_t)key, q, seqpr_center(a, b, q));
+                }
+            }
+#pragma unroll
+            for (int k = 0; k < kPer; ++k) seqpr_add(s_h, n, valid[k], valid[k] ? seqpr_bin(s_y, n, v[k]) : 0, g[k], lane);
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < 2 * n; i += blockDim.x)
+        if (s_h[i]) atomicAdd(a.hist + i, (unsigned long long)s_h[i]);
+}
+
+// tp[i] += positives with bin <= i, fp[i] likewise (the values >= threshold i).  Warp 0: tp, warp 1: fp.
+__global__ void __launch_bounds__(64) seqpr_prefix_kernel(const unsigned long long *__restrict__ hist, int n,
+                                                          unsigned long long *__restrict__ tp,
+                                                          unsigned long long *__restrict__ fp)
+{
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const unsigned long long *h = hist + (size_t)w * n;
+    unsigned long long *out = w ? fp : tp, carry = 0;
+    for (int base = 0; base < n; base += 32) {
+        const int i = base + lane;
+        unsigned long long v = i < n ? h[i] : 0ull;
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long up = shfl_u64(v, max(lane - o, 0));
+            if (lane >= o) v += up;
+        }
+        v += carry;
+        if (i < n) out[i] += v;
+        carry = shfl_u64(v, 31);
+    }
+}
+
 // SAD baseline (lens/src/sad.py:38): one warp per (query, reference) pair, 16 pixels per lane-iteration
 // with byte-wise SIMD sum of absolute differences; integer accumulation (exact), stored as fp32.
 __global__ void __launch_bounds__(256) sad_kernel(const uint8_t *__restrict__ a, const uint8_t *__restrict__ b,
@@ -993,5 +1274,117 @@ extern "C" int lens_pr_counts_multi(const float *S, const uint8_t *GT, int Po, i
         reinterpret_cast<unsigned long long *>(fp));
     LENS_LAUNCH_CHECK();
     LENS_CUDA(cudaFreeAsync(mm, st));
+    return 0;
+}
+
+// Validates the arguments shared by lens_seqpr_scan / lens_seqpr_counts and fills the kernel arguments.
+static int seqpr_args(SeqPrArgs &a, const char *fn, const float *S, int B, int Q, int P, int L, int mode,
+                      const uint8_t *gt_dense, int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol,
+                      void *records)
+{
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "%s: bad sizes", fn);
+    LENS_CHECK_ARG(L >= 1 && L <= Q && L <= P, "%s: need 1 <= L <= min(Q, P), got L=%d", fn, L);
+    LENS_CHECK_ARG(mode == LENS_SEQPR_PLACE || mode == LENS_SEQPR_QUERY || mode == LENS_SEQPR_MULTI,
+                   "%s: unknown mode %d", fn, mode);
+    LENS_CHECK_ARG((gt_dense != nullptr) != (gt_center != nullptr),
+                   "%s: exactly one of gt_dense / gt_center must be given", fn);
+    LENS_CHECK_ARG(gt_stream_stride >= 0 && gt_tol >= 0, "%s: gt_stream_stride and gt_tol must be >= 0", fn);
+    LENS_CHECK_ARG(B == 0 || S != nullptr, "%s: NULL S", fn);
+    LENS_CHECK_ARG(mode == LENS_SEQPR_MULTI || B == 0 || (records && (reinterpret_cast<uintptr_t>(records) & 7) == 0),
+                   "%s: the single modes need 8-byte aligned records", fn);
+    a = SeqPrArgs{};
+    a.S = S; a.B = B; a.Q = Q; a.P = P; a.L = L; a.Qo = Q - L + 1; a.Po = P - L + 1;
+    a.gt_dense = gt_dense; a.gt_stride = gt_stream_stride; a.gt_center = gt_center; a.gt_tol = gt_tol;
+    const size_t n_rec = (size_t)B * (mode == LENS_SEQPR_PLACE ? a.Po : a.Qo);
+    if (mode == LENS_SEQPR_PLACE) {
+        a.rec_val = static_cast<float *>(records);
+        a.rec_flag = reinterpret_cast<uint8_t *>(a.rec_val + n_rec);
+    } else if (mode == LENS_SEQPR_QUERY) {
+        a.rec_key = static_cast<unsigned long long *>(records);
+        a.rec_flag = reinterpret_cast<uint8_t *>(a.rec_key + n_rec);
+    }
+    return 0;
+}
+
+extern "C" int lens_seqpr_records_bytes(int B, int Q, int P, int L, int mode, int64_t *bytes)
+{
+    LENS_CHECK_ARG(bytes != nullptr, "lens_seqpr_records_bytes: NULL bytes");
+    LENS_CHECK_ARG(B >= 0 && L >= 1 && L <= Q && L <= P, "lens_seqpr_records_bytes: bad sizes");
+    LENS_CHECK_ARG(mode == LENS_SEQPR_PLACE || mode == LENS_SEQPR_QUERY || mode == LENS_SEQPR_MULTI,
+                   "lens_seqpr_records_bytes: unknown mode %d", mode);
+    if (mode == LENS_SEQPR_PLACE) *bytes = (int64_t)B * (P - L + 1) * (sizeof(float) + 1);
+    else if (mode == LENS_SEQPR_QUERY) *bytes = (int64_t)B * (Q - L + 1) * (sizeof(unsigned long long) + 1);
+    else *bytes = 0;
+    return 0;
+}
+
+extern "C" int lens_seqpr_scan(const float *S, int B, int Q, int P, int L, int mode, const uint8_t *gt_dense,
+                               int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, void *records,
+                               uint64_t *extremes, int64_t *gtp, void *stream)
+{
+    SeqPrArgs a;
+    if (int rc = seqpr_args(a, "lens_seqpr_scan", S, B, Q, P, L, mode, gt_dense, gt_stream_stride, gt_center, gt_tol,
+                            records))
+        return rc;
+    LENS_CHECK_ARG(extremes && gtp, "lens_seqpr_scan: NULL extremes / gtp");
+    if (B == 0) return 0;
+    a.ext = reinterpret_cast<unsigned long long *>(extremes);
+    a.gtp = reinterpret_cast<unsigned long long *>(gtp);
+    cudaStream_t st = as_stream(stream);
+    const long long sms = std::max(sm_count(), 1);
+    const long long items = (long long)B * ceil_div(a.Po, kPrTile);
+    const unsigned blocks = (unsigned)std::min<long long>(ceil_div64(items, 8), sms * 16);
+    if (mode == LENS_SEQPR_PLACE) {
+        seqpr_scan_kernel<kPrPlace><<<blocks, 256, 0, st>>>(a);
+        LENS_LAUNCH_CHECK();
+    } else if (mode == LENS_SEQPR_QUERY) {
+        const size_t n_rec = (size_t)B * a.Qo;
+        LENS_CUDA(cudaMemsetAsync(records, 0, n_rec * (sizeof(unsigned long long) + 1), st));
+        seqpr_scan_kernel<kPrQuery><<<blocks, 256, 0, st>>>(a);
+        LENS_LAUNCH_CHECK();
+        seqpr_query_extremes_kernel<<<(unsigned)std::min<long long>(ceil_div64((long long)n_rec, 256), sms * 8), 256, 0,
+                                      st>>>(a);
+        LENS_LAUNCH_CHECK();
+    } else {
+        seqpr_scan_kernel<kPrMulti><<<blocks, 256, 0, st>>>(a);
+        LENS_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
+extern "C" int lens_seqpr_counts(const float *S, int B, int Q, int P, int L, int mode, const uint8_t *gt_dense,
+                                 int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, const void *records,
+                                 const uint64_t *extremes, int n_thresh, int64_t *tp, int64_t *fp, void *stream)
+{
+    SeqPrArgs a;
+    if (int rc = seqpr_args(a, "lens_seqpr_counts", S, B, Q, P, L, mode, gt_dense, gt_stream_stride, gt_center,
+                            gt_tol, const_cast<void *>(records)))
+        return rc;
+    LENS_CHECK_ARG(n_thresh >= 2 && n_thresh <= kPrMaxThresh, "lens_seqpr_counts: n_thresh must be in [2, %d], got %d",
+                   kPrMaxThresh, n_thresh);
+    LENS_CHECK_ARG(extremes && tp && fp, "lens_seqpr_counts: NULL extremes / tp / fp");
+    if (B == 0) return 0;
+    a.ext = const_cast<unsigned long long *>(reinterpret_cast<const unsigned long long *>(extremes));
+    a.n_thresh = n_thresh;
+    cudaStream_t st = as_stream(stream);
+    const long long sms = std::max(sm_count(), 1);
+    const size_t hist_bytes = (size_t)2 * n_thresh * sizeof(unsigned long long);
+    LENS_CUDA(cudaMallocAsync(&a.hist, hist_bytes, st));          // stream-ordered scratch, as in lens_seqmatch_topk
+    LENS_CUDA(cudaMemsetAsync(a.hist, 0, hist_bytes, st));
+    const size_t smem = (size_t)n_thresh * (sizeof(float) + 2 * sizeof(unsigned));   // <= 48 KB
+    if (mode == LENS_SEQPR_MULTI) {
+        const long long items = (long long)B * ceil_div(a.Po, kPrTile);
+        seqpr_count_kernel<kPrMulti><<<(unsigned)std::min<long long>(ceil_div64(items, 8), sms * 8), 256, smem, st>>>(a);
+    } else {
+        const long long n_rec = (long long)B * (mode == LENS_SEQPR_PLACE ? a.Po : a.Qo);
+        const unsigned blocks = (unsigned)std::min<long long>(ceil_div64(n_rec, 256 * 4), sms * 8);
+        if (mode == LENS_SEQPR_PLACE) seqpr_count_kernel<kPrPlace><<<blocks, 256, smem, st>>>(a);
+        else seqpr_count_kernel<kPrQuery><<<blocks, 256, smem, st>>>(a);
+    }
+    LENS_LAUNCH_CHECK();
+    seqpr_prefix_kernel<<<1, 64, 0, st>>>(a.hist, n_thresh, reinterpret_cast<unsigned long long *>(tp),
+                                          reinterpret_cast<unsigned long long *>(fp));
+    LENS_LAUNCH_CHECK();
+    LENS_CUDA(cudaFreeAsync(a.hist, st));
     return 0;
 }

@@ -167,6 +167,76 @@ def recall_counts(top_idx, Po, gt_dense=None, gt_center=None, gt_tol=0, ns=RECAL
     return hits, n_valid
 
 
+SEQPR_MODES = {("single", "place"): 0, ("single", "query"): 1, ("multi", None): 2}   # LENS_SEQPR_*
+SEQPR_MAX_THRESH = 4096
+
+
+def seqpr_mode(matching, best="place"):
+    """createPR's matching ('single' with best='place' or 'query', or 'multi') -> LENS_SEQPR_* mode."""
+    key = (matching, best if matching == "single" else None)
+    if key not in SEQPR_MODES:
+        raise ValueError(f"matching must be 'single' (best='place' or 'query') or 'multi', got {matching!r}, "
+                         f"best={best!r}")
+    return SEQPR_MODES[key]
+
+
+def _seqpr_check(S, L, mode, gt_dense, gt_center, n_thresh=2):
+    """Shape and value checks of the fleet precision-recall calls (before anything touches the device)."""
+    if not torch.is_tensor(S) or S.dtype != torch.float32 or S.dim() != 3:
+        raise ValueError("S must be f32 [B, Q, P]")
+    B, Q, P = S.shape
+    if not 1 <= L <= min(Q, P):
+        raise ValueError(f"need 1 <= L <= min(Q, P) = {min(Q, P)}, got L={L}")
+    if mode not in SEQPR_MODES.values():
+        raise ValueError(f"unknown mode {mode}")
+    if not 2 <= n_thresh <= SEQPR_MAX_THRESH:
+        raise ValueError(f"n_thresh must be in [2, {SEQPR_MAX_THRESH}], got {n_thresh}")
+    Qo, Po = Q - L + 1, P - L + 1
+    if (gt_dense is None) == (gt_center is None):
+        raise ValueError("give exactly one of gt_dense / gt_center")
+    if gt_dense is not None and (gt_dense.dtype != torch.uint8 or tuple(gt_dense.shape) not in ((Po, Qo), (B, Po, Qo))):
+        raise ValueError(f"gt_dense must be u8 [{Po}, {Qo}] or [{B}, {Po}, {Qo}], got {tuple(gt_dense.shape)}")
+    if gt_center is not None and (gt_center.dtype != torch.int32 or tuple(gt_center.shape) != (B, Qo)):
+        raise ValueError(f"gt_center must be i32 [{B}, {Qo}], got {tuple(gt_center.shape)}")
+    return B, Q, P, (Po * Qo if gt_dense is not None and gt_dense.dim() == 3 else 0)
+
+
+def seqpr_scan(S, L, mode, gt_dense=None, gt_center=None, gt_tol=0, extremes=None, gtp=None):
+    """Scan pass of the fleet precision-recall (lens_seqpr_scan): S f32 [B, Q, P] spike counts, ground truth as in
+    `recall_counts`.  -> (records u8 [bytes] or None, extremes i64 [2], gtp i64 [1]) on the device.  extremes
+    ({max, ~min} as order-preserving keys) are merged by max and gtp accumulated, so passing the tensors of an
+    earlier scan makes one fleet of both groups of streams."""
+    B, Q, P, stride = _seqpr_check(S, L, mode, gt_dense, gt_center)
+    require_cuda(S, gt_dense, gt_center, extremes, gtp)
+    nbytes = C.c_int64(0)
+    check(_lib.lib().lens_seqpr_records_bytes(B, Q, P, L, mode, C.byref(nbytes)), "lens_seqpr_records_bytes")
+    records = torch.empty((nbytes.value,), dtype=torch.uint8, device=S.device) if nbytes.value else None
+    if extremes is None:
+        extremes = torch.zeros((2,), dtype=torch.int64, device=S.device)
+    if gtp is None:
+        gtp = torch.zeros((1,), dtype=torch.int64, device=S.device)
+    check(_lib.lib().lens_seqpr_scan(ptr(S), B, Q, P, L, mode, ptr(gt_dense), stride, ptr(gt_center), int(gt_tol),
+                                     ptr(records), ptr(extremes), ptr(gtp), stream_ptr()), "lens_seqpr_scan")
+    return records, extremes, gtp
+
+
+def seqpr_counts(S, L, mode, records, extremes, n_thresh=100, gt_dense=None, gt_center=None, gt_tol=0, tp=None,
+                 fp=None):
+    """Count pass (lens_seqpr_counts) with the same S / L / mode / ground truth and the scan's records, over the
+    thresholds np.linspace(max, min, n_thresh) of the (merged) extremes.  -> (tp, fp) i64 [n_thresh] on the device,
+    accumulated into tp / fp when given."""
+    B, Q, P, stride = _seqpr_check(S, L, mode, gt_dense, gt_center, n_thresh)
+    require_cuda(S, gt_dense, gt_center, records, extremes, tp, fp)
+    if tp is None:
+        tp = torch.zeros((n_thresh,), dtype=torch.int64, device=S.device)
+    if fp is None:
+        fp = torch.zeros((n_thresh,), dtype=torch.int64, device=S.device)
+    check(_lib.lib().lens_seqpr_counts(ptr(S), B, Q, P, L, mode, ptr(gt_dense), stride, ptr(gt_center), int(gt_tol),
+                                       ptr(records), ptr(extremes), n_thresh, ptr(tp), ptr(fp), stream_ptr()),
+          "lens_seqpr_counts")
+    return tp, fp
+
+
 def topn_merge(vals, idx):
     """Global top-N from W per-shard lists: vals f32 / idx i32 [W, B, Qo, N] (idx = global place index, -1 =
     empty) -> (val [B, Qo, N], idx [B, Qo, N]) under the order (value desc, place index desc)."""

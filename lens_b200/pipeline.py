@@ -193,6 +193,39 @@ class InferencePipeline:
         self._stage_events = []
         return dict(similarity_ms=sim, match_ms=mat, n=n)
 
+    def precision_recall(self, S, gt_dense=None, gt_center=None, gt_tol=0, matching="single", best="place",
+                         n_thresh=100, reduce=True):
+        """createPR's precision-recall lists for the whole fleet, from the spike counts S f32 [B, Q, P] that the
+        steps return; the sequence-matched matrices are recomputed on the GPU, never stored.
+        -> dict(P, R, tp, fp, gtp): P / R python lists of length n_thresh + 1 (as createPR), tp / fp numpy i64.
+
+        The fleet's curve is createPR over the streams' matrices concatenated along its column axis, so the
+        thresholds span the whole fleet (and every rank, under torch.distributed with reduce=True):
+          matching='single', best='place': createPR(D_b.T, GT_b.T, 'single') at B = 1, the reference's --PR_curve
+          matching='single', best='query': createPR(D_b, GT_b, 'single') at B = 1, the SAD path's call
+          matching='multi':                createPR(D_b, GT_b, 'multi') at B = 1
+        Ground truth as `match`: gt_dense u8 [Po, Qo] or [B, Po, Qo], or gt_center i32 [B, Qo] with gt_tol.
+        Under torch.distributed with reduce=True: one all-reduce MAX of the extremes between the two passes and one
+        all-reduce SUM of [tp, fp, gtp]; reduce=False gives this rank's own curve."""
+        from .src.metrics import pr_lists
+        mode = ops.seqpr_mode(matching, best)
+        ops._seqpr_check(S, self.L, mode, gt_dense, gt_center, n_thresh)
+        gt = dict(gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol)
+        dist = torch.distributed
+        shared = reduce and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+        with torch.cuda.device(S.device):
+            records, extremes, gtp = ops.seqpr_scan(S, self.L, mode, **gt)
+            if shared:
+                dist.all_reduce(extremes, op=dist.ReduceOp.MAX)     # {max, ~min} keys: max merges both
+            tp, fp = ops.seqpr_counts(S, self.L, mode, records, extremes, n_thresh, **gt)
+            packed = torch.cat([tp, fp, gtp])
+            if shared:
+                dist.all_reduce(packed)
+        packed = packed.cpu().numpy()
+        tp, fp, gtp = packed[:n_thresh], packed[n_thresh:2 * n_thresh], int(packed[-1])
+        P, R = pr_lists(tp, fp, gtp)
+        return dict(P=P, R=R, tp=tp, fp=fp, gtp=gtp)
+
     @staticmethod
     def recall(hits, n_valid):
         nv = int(n_valid.item())
@@ -242,7 +275,8 @@ class StreamingPipeline(InferencePipeline):
         raise LensError("StreamingPipeline is a live session: feed it with push / push_events "
                         "(use an InferencePipeline for batch steps)")
 
-    step = step_events = step_event_groups = step_host = _offline
+    # precision_recall needs whole sequences, and a push's S holds only the new rows
+    step = step_events = step_event_groups = step_host = precision_recall = _offline
 
     def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True):
         """Q new windows of every stream: frames u8 [B, Q, roi, roi] or pooled u8 [B, Q, I], B = n_streams.

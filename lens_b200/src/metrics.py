@@ -128,7 +128,12 @@ def createPR(S_in, GThard, outputdir=None, datatype="LENS", GTsoft=None, matchin
     else:
         check(lib().lens_pr_counts_multi(ptr(dS), ptr(dG), Po, Qo, n_thresh, ptr(tp), ptr(fp), ptr(gtp), stream_ptr(),
                                          thresh_f64), "lens_pr_counts_multi")
-    tp, fp, gtp = tp.cpu().numpy(), fp.cpu().numpy(), int(gtp.item())
+    return pr_lists(tp.cpu().numpy(), fp.cpu().numpy(), int(gtp.item()))
+
+
+def pr_lists(tp, fp, gtp):
+    """createPR's (P, R) from the counts at its thresholds (lens/src/metrics.py:21-139): lists of length
+    len(tp) + 1 starting with P = 1, R = 0, each entry a float64 division as the reference makes it."""
     P, R = [1], [0]
     with np.errstate(divide="ignore", invalid="ignore"):
         for a, b in zip(tp, fp):
