@@ -30,6 +30,8 @@
  *   lens_pr_counts         Qo <= 8192 (one CTA, shared-memory resident)
  *   lens_seqpr_scan / _counts
  *                          1 <= L <= min(Q, P), 2 <= n_thresh <= 4096 (table and histograms in 48 KB of shared memory)
+ *   lens_seqpr_stream_*    1 <= L <= P, B * Q <= 2^31 - 1, every sequence sum k an integer in [0, 65 535]
+ *                          (LENS_SEQPR_STREAM_BINS - 1; otherwise n_bad), 2 <= n_thresh <= 4096
  *   lens_sad_matrix        npix <= 65 793 (sums stay exact in fp32)
  *   lens_topn_merge        W * N <= 512
  *   lens_bin_events        t_us ascending (lens_check_sorted_u32), x / y 16-byte aligned
@@ -302,6 +304,34 @@ int lens_seqpr_scan(const float *S, int B, int Q, int P, int L, int mode, const 
 int lens_seqpr_counts(const float *S, int B, int Q, int P, int L, int mode, const uint8_t *gt_dense,
                       int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, const void *records,
                       const uint64_t *extremes, int n_thresh, int64_t *tp, int64_t *fp, void *stream);
+
+/* Session precision-recall of a live fleet (lens_seqmatch_topk_stream), accumulated push by push in bounded memory.
+ * A stream's session matrix has its valid rows as query columns, in push order (warm-up rows are never columns);
+ * fleets and ranks concatenate along createPR's column axis, in the same three modes as the fleet calls above.
+ * Every D entry is acc / L with acc an integer-valued spike sum; for 0 <= acc < LENS_SEQPR_STREAM_BINS the value is a
+ * strictly increasing function of k = acc, so the curve depends on k only.  An entry outside that range, or not
+ * integer-valued, is counted in n_bad and makes the session's numbers invalid.
+ *   lens_seqpr_stream_bytes      *bytes (host) = the size of one mode's accumulator: 16 + 4*B*(P-L+1) (place) or
+ *                                16 + 16*LENS_SEQPR_STREAM_BINS (query, multi).  Zeroed memory is an empty session.
+ *   lens_seqpr_stream_accumulate folds the valid new rows of one push into the accumulators of the tracked modes
+ *                                (NULL = not tracked; 8-byte aligned).  S, sizes, ring, seen and t as for the
+ *                                lens_seqmatch_topk_stream call of the same push, which must come AFTER this one (it
+ *                                advances seen and overwrites ring slots).  gt_center [B][Q] i32: the expected place
+ *                                of each new row (< 0: no positive), positives |p - center| <= gt_tol.  One launch,
+ *                                two when the query mode is tracked; never more with B.
+ *   lens_seqpr_stream_histogram  one accumulator -> hist [2][LENS_SEQPR_STREAM_BINS] u64 (positives | negatives per
+ *                                k), gtp [1], n_bad [1], all ACCUMULATED.  Sums of these over ranks form one fleet.
+ *   lens_seqpr_hist_counts       tp, fp [n_thresh] i64 ACCUMULATED: thresholds np.linspace(max, min, n_thresh) of the
+ *                                float32 values fl(k / L) of the lowest and highest non-empty k (numpy's float32
+ *                                recipe); nothing is added for an empty histogram.  2 <= n_thresh <= 4096.      */
+#define LENS_SEQPR_STREAM_BINS 65536
+int lens_seqpr_stream_bytes(int B, int P, int L, int mode, int64_t *bytes);
+int lens_seqpr_stream_accumulate(const float *S, int B, int Q, int P, int L, const float *ring, const int32_t *seen,
+                                 int64_t t, const int32_t *gt_center, int gt_tol, void *acc_place, void *acc_query,
+                                 void *acc_multi, void *stream);
+int lens_seqpr_stream_histogram(const void *acc, int B, int P, int L, int mode, uint64_t *hist, int64_t *gtp,
+                                int64_t *n_bad, void *stream);
+int lens_seqpr_hist_counts(const uint64_t *hist, int L, int n_thresh, int64_t *tp, int64_t *fp, void *stream);
 
 /* Sum-of-absolute-differences baseline, lens/src/sad.py:25-42: dist[q][r] = sum_p |a[q][p] - b[r][p]|
  * (torch.cdist(a, b, p=1) on float32 copies of uint8 frames; the sums are integers < 2^24, hence exact

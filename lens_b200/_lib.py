@@ -59,6 +59,10 @@ def _declare(L):
         "lens_seqpr_records_bytes": (i32, [i32, i32, i32, i32, i32, pi64]),
         "lens_seqpr_scan": (i32, [vp, i32, i32, i32, i32, i32, vp, i64, vp, i32, vp, vp, vp, vp]),
         "lens_seqpr_counts": (i32, [vp, i32, i32, i32, i32, i32, vp, i64, vp, i32, vp, vp, i32, vp, vp, vp]),
+        "lens_seqpr_stream_bytes": (i32, [i32, i32, i32, i32, pi64]),
+        "lens_seqpr_stream_accumulate": (i32, [vp, i32, i32, i32, i32, vp, vp, i64, vp, i32, vp, vp, vp, vp]),
+        "lens_seqpr_stream_histogram": (i32, [vp, i32, i32, i32, i32, vp, vp, vp, vp]),
+        "lens_seqpr_hist_counts": (i32, [vp, i32, i32, vp, vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)          # AttributeError if the .so lacks a declared symbol

@@ -943,6 +943,229 @@ __global__ void __launch_bounds__(64) seqpr_prefix_kernel(const unsigned long lo
     }
 }
 
+// ---- session precision-recall of a live fleet (lens_seqpr_stream_*) -------------------------------------------
+// Every D entry is __fdiv_rn(acc, L) with acc an integer-valued sum of spike counts; for an integer 0 <= k < 2^16,
+// fl(k / L) is strictly increasing in k, so a session's createPR curve depends only on the k of its entries:
+// place mode keeps one record per (stream, place) (the first maximum over the session's rows), query and multi mode
+// a histogram over k.  Accumulators start with a header {n_bad, gtp} (u64); zeroed memory is an empty session.
+constexpr int kStreamBins = LENS_SEQPR_STREAM_BINS;
+constexpr int kStreamShBins = 2048;       // k below this is counted in shared memory first (spike sums are small)
+
+struct SeqPrStreamArgs {
+    const float *S, *ring;
+    const int32_t *seen;
+    long long t;
+    int B, Q, P, L, Po;
+    const int32_t *gt_center;            // [B][Q]
+    int gt_tol;
+    unsigned *rec;                       // place: [B][Po] records (k + 1) << 2 | hit at first max << 1 | any positive
+    unsigned long long *key;             // query: [B][Q] per-push scratch, k << 32 | ~p of the row's first maximum
+    unsigned long long *hist;            // multi: [2][kStreamBins], positives first
+    unsigned long long *multi_gtp;
+    unsigned long long *bad[3];          // n_bad of each tracked accumulator, NULL when the mode is not tracked
+};
+
+// One count of (k, hit) per valid lane; lanes with the same (k, hit) add once.  Small k goes to the block's shared
+// histogram s_h [2][kStreamShBins], the rare large k straight to the global one g_h [2][kStreamBins].
+__device__ __forceinline__ void stream_hist_add(unsigned *s_h, unsigned long long *g_h, bool valid, int k, bool hit,
+                                                int lane)
+{
+    const unsigned key = valid ? ((unsigned)k << 1 | (unsigned)hit) : 0xffffffffu;
+    const unsigned peers = __match_any_sync(0xffffffffu, key);
+    if (valid && __ffs(peers) - 1 == lane) {
+        if (k < kStreamShBins) atomicAdd(s_h + (hit ? 0 : kStreamShBins) + k, (unsigned)__popc(peers));
+        else atomicAdd(g_h + (hit ? 0 : kStreamBins) + k, (unsigned long long)__popc(peers));
+    }
+}
+
+__device__ __forceinline__ void stream_hist_flush(const unsigned *s_h, unsigned long long *g_h)
+{
+    __syncthreads();
+    for (int i = threadIdx.x; i < 2 * kStreamShBins; i += blockDim.x)
+        if (s_h[i]) atomicAdd(g_h + (i < kStreamShBins ? i : kStreamBins + i - kStreamShBins), (unsigned long long)s_h[i]);
+}
+
+// One warp per (stream, kPrTile places), the push's new rows in order; warm-up rows are skipped.  The diagonal terms
+// come through StreamRows as in seqmatch_topk_stream_warp_kernel, so this runs before that call (same t, same seen).
+__global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_kernel(SeqPrStreamArgs a)
+{
+    extern __shared__ unsigned s_h[];    // multi mode: [2][kStreamShBins]
+    const int lane = threadIdx.x & 31;
+    if (a.hist) {
+        for (int i = threadIdx.x; i < 2 * kStreamShBins; i += blockDim.x) s_h[i] = 0u;
+        __syncthreads();
+    }
+    const long long warp0 = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    const long long n_tiles = ceil_div(a.Po, kPrTile), n_items = (long long)a.B * n_tiles;
+    unsigned bad = 0, pos = 0;                       // per lane: at most kUnrollR * Q entries per item
+    for (long long w = warp0; w < n_items; w += n_warps) {
+        const int b = (int)(w / n_tiles), p0 = (int)(w - (long long)b * n_tiles) * kPrTile;
+        unsigned rec[kUnrollR];
+#pragma unroll
+        for (int u = 0; u < kUnrollR; ++u) {
+            const int p = p0 + 32 * u + lane;
+            rec[u] = (a.rec && p < a.Po) ? a.rec[(size_t)b * a.Po + p] : 0u;
+        }
+        for (int q = 0; q < a.Q; ++q) {
+            if (!stream_row_valid(a.seen, b, q, a.L)) continue;           // warp-uniform
+            const StreamRows rows(a.S, a.ring, b, a.Q, q, a.P, a.L, a.t);
+            float acc[kUnrollR];
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) acc[u] = 0.0f;
+            if (p0 + kPrTile <= a.Po) {
+                for (int j = 0; j < a.L; ++j) {
+                    const float *row = rows.row(j) + (p0 + lane + j);
+#pragma unroll
+                    for (int u = 0; u < kUnrollR; ++u) acc[u] += __ldg(row + 32 * u);
+                }
+            } else {
+                for (int j = 0; j < a.L; ++j) {
+                    const float *row = rows.row(j) + (p0 + lane + j);
+#pragma unroll
+                    for (int u = 0; u < kUnrollR; ++u)
+                        if (p0 + 32 * u + lane < a.Po) acc[u] += __ldg(row + 32 * u);
+                }
+            }
+            const int c = __ldg(a.gt_center + (size_t)b * a.Q + q);
+            unsigned long long kq = 0ull;
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) {
+                const int p = p0 + 32 * u + lane;
+                const bool in = p < a.Po;
+                // k is exact only for an integer-valued sum in [0, 2^16); anything else makes the session invalid
+                const bool ok = in && acc[u] >= 0.0f && acc[u] < (float)kStreamBins && acc[u] == truncf(acc[u]);
+                bad += in && !ok;
+                const int k = ok ? (int)acc[u] : 0;
+                const bool g = ok && c >= 0 && abs(p - c) <= a.gt_tol;
+                if (a.rec && ok) {
+                    const unsigned any = (rec[u] & 1u) | (unsigned)g;
+                    if ((unsigned)(k + 1) > rec[u] >> 2) rec[u] = (unsigned)(k + 1) << 2 | (unsigned)g << 1 | any;  // strict: first maximum
+                    else rec[u] |= any;
+                }
+                if (a.key && ok) {
+                    const unsigned long long kk = (unsigned long long)k << 32 | (uint32_t)~p;   // lowest place among ties
+                    kq = kk > kq ? kk : kq;
+                }
+                if (a.hist) {
+                    stream_hist_add(s_h, a.hist, ok, k, g, lane);
+                    pos += g;
+                }
+            }
+            if (a.key) {
+                for (int o = 16; o > 0; o >>= 1) {
+                    const unsigned long long other = shfl_xor_u64(kq, o);
+                    kq = other > kq ? other : kq;
+                }
+                if (lane == 0 && kq) atomicMax(a.key + (size_t)b * a.Q + q, kq);
+            }
+        }
+        if (a.rec) {
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) {
+                const int p = p0 + 32 * u + lane;
+                if (p < a.Po) a.rec[(size_t)b * a.Po + p] = rec[u];
+            }
+        }
+    }
+    const unsigned long long bad_w = __reduce_add_sync(0xffffffffu, bad), pos_w = __reduce_add_sync(0xffffffffu, pos);
+    if (lane == 0) {
+        if (bad_w)
+            for (int m = 0; m < 3; ++m)
+                if (a.bad[m]) atomicAdd(a.bad[m], bad_w);
+        if (pos_w) atomicAdd(a.multi_gtp, pos_w);
+    }
+    if (a.hist) stream_hist_flush(s_h, a.hist);
+}
+
+// Query mode, after the accumulate kernel: one thread per new row folds its first maximum into the histogram and
+// clears the scratch; gtp counts the valid rows with a positive among the places [0, Po).
+__global__ void __launch_bounds__(256) seqpr_stream_query_fold_kernel(SeqPrStreamArgs a, unsigned long long *acc_hist,
+                                                                      unsigned long long *gtp)
+{
+    const long long n = (long long)a.B * a.Q;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const int b = (int)(i / a.Q), q = (int)(i - (long long)b * a.Q);
+        if (!stream_row_valid(a.seen, b, q, a.L)) continue;
+        const unsigned long long key = a.key[i];
+        a.key[i] = 0ull;
+        const int c = __ldg(a.gt_center + i);
+        if (c >= 0 && c - a.gt_tol < a.Po) atomicAdd(gtp, 1ull);
+        if (!key) continue;                                              // every entry of the row was bad
+        const int k = (int)(key >> 32), p = (int)~(uint32_t)key;
+        const bool g = c >= 0 && abs(p - c) <= a.gt_tol;
+        atomicAdd(acc_hist + (g ? 0 : kStreamBins) + k, 1ull);
+    }
+}
+
+// Place mode, finish: every record that saw a valid row is one column (k, hit at its first maximum); gtp counts the
+// records with a positive, n_bad takes the accumulator's.
+__global__ void __launch_bounds__(256) seqpr_stream_place_hist_kernel(const unsigned long long *__restrict__ acc,
+                                                                      long long n,
+                                                                      unsigned long long *__restrict__ hist,
+                                                                      unsigned long long *__restrict__ gtp,
+                                                                      unsigned long long *__restrict__ n_bad)
+{
+    __shared__ unsigned s_h[2 * kStreamShBins];
+    const int lane = threadIdx.x & 31;
+    const unsigned *rec = reinterpret_cast<const unsigned *>(acc + 2);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && acc[0]) atomicAdd(n_bad, acc[0]);
+    for (int i = threadIdx.x; i < 2 * kStreamShBins; i += blockDim.x) s_h[i] = 0u;
+    __syncthreads();
+    unsigned long long pos = 0;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long i0 = blockIdx.x * (long long)blockDim.x; i0 < n; i0 += stride) {   // the same trip count per warp
+        const long long i = i0 + threadIdx.x;
+        const unsigned r = i < n ? __ldg(rec + i) : 0u;
+        stream_hist_add(s_h, hist, r != 0u, r ? (int)(r >> 2) - 1 : 0, (r >> 1) & 1u, lane);
+        pos += r & 1u;
+    }
+    for (int o = 16; o > 0; o >>= 1) pos += __shfl_xor_sync(0xffffffffu, pos, o);
+    if (lane == 0 && pos) atomicAdd(gtp, pos);
+    stream_hist_flush(s_h, hist);
+}
+
+// Query / multi mode, finish: hist += the accumulator's histogram, {n_bad, gtp} += its header.
+__global__ void __launch_bounds__(256) seqpr_stream_add_kernel(const unsigned long long *__restrict__ acc,
+                                                               unsigned long long *__restrict__ hist,
+                                                               unsigned long long *__restrict__ gtp,
+                                                               unsigned long long *__restrict__ n_bad)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 2 * kStreamBins) hist[i] += acc[2 + i];
+    if (i == 0) { *n_bad += acc[0]; *gtp += acc[1]; }
+}
+
+// createPR's thresholds from the lowest and highest non-empty k (values fl(k / L)), then every non-empty k binned
+// once into binned [2][n]; seqpr_prefix_kernel turns that into tp / fp.  One CTA.
+__global__ void __launch_bounds__(1024) seqpr_stream_bin_kernel(const unsigned long long *__restrict__ hist, int L,
+                                                                int n, unsigned long long *__restrict__ binned)
+{
+    __shared__ float s_y[kPrMaxThresh];
+    __shared__ int s_lo, s_hi;
+    if (threadIdx.x == 0) { s_lo = kStreamBins; s_hi = -1; }
+    __syncthreads();
+    int lo = kStreamBins, hi = -1;
+    for (int k = threadIdx.x; k < kStreamBins; k += blockDim.x)
+        if (hist[k] | hist[kStreamBins + k]) { lo = min(lo, k); hi = max(hi, k); }
+    lo = __reduce_min_sync(0xffffffffu, lo);
+    hi = __reduce_max_sync(0xffffffffu, hi);
+    if ((threadIdx.x & 31) == 0) { atomicMin(&s_lo, lo); atomicMax(&s_hi, hi); }
+    __syncthreads();
+    if (s_hi < 0) return;                                                // empty session: nothing to count
+    const float fl = (float)L;
+    const float start = __fdiv_rn((float)s_hi, fl), stop = __fdiv_rn((float)s_lo, fl);
+    for (int i = threadIdx.x; i < n; i += blockDim.x) s_y[i] = (float)pr_threshold(i, n, start, stop, false);
+    __syncthreads();
+    for (int k = s_lo + threadIdx.x; k <= s_hi; k += blockDim.x) {
+        const unsigned long long tp = hist[k], fp = hist[kStreamBins + k];
+        if (!(tp | fp)) continue;
+        const int bin = seqpr_bin(s_y, n, __fdiv_rn((float)k, fl));
+        if (tp) atomicAdd(binned + bin, tp);
+        if (fp) atomicAdd(binned + n + bin, fp);
+    }
+}
+
 // SAD baseline (lens/src/sad.py:38): one warp per (query, reference) pair, 16 pixels per lane-iteration
 // with byte-wise SIMD sum of absolute differences; integer accumulation (exact), stored as fp32.
 __global__ void __launch_bounds__(256) sad_kernel(const uint8_t *__restrict__ a, const uint8_t *__restrict__ b,
@@ -1386,5 +1609,112 @@ extern "C" int lens_seqpr_counts(const float *S, int B, int Q, int P, int L, int
                                           reinterpret_cast<unsigned long long *>(fp));
     LENS_LAUNCH_CHECK();
     LENS_CUDA(cudaFreeAsync(a.hist, st));
+    return 0;
+}
+
+extern "C" int lens_seqpr_stream_bytes(int B, int P, int L, int mode, int64_t *bytes)
+{
+    LENS_CHECK_ARG(bytes != nullptr, "lens_seqpr_stream_bytes: NULL bytes");
+    LENS_CHECK_ARG(B >= 0 && P > 0 && L >= 1 && L <= P, "lens_seqpr_stream_bytes: bad sizes");
+    LENS_CHECK_ARG(mode == LENS_SEQPR_PLACE || mode == LENS_SEQPR_QUERY || mode == LENS_SEQPR_MULTI,
+                   "lens_seqpr_stream_bytes: unknown mode %d", mode);
+    const int64_t header = 2 * sizeof(unsigned long long);
+    if (mode == LENS_SEQPR_PLACE) *bytes = header + (int64_t)B * (P - L + 1) * sizeof(unsigned);
+    else *bytes = header + (int64_t)2 * kStreamBins * sizeof(unsigned long long);
+    return 0;
+}
+
+extern "C" int lens_seqpr_stream_accumulate(const float *S, int B, int Q, int P, int L, const float *ring,
+                                            const int32_t *seen, int64_t t, const int32_t *gt_center, int gt_tol,
+                                            void *acc_place, void *acc_query, void *acc_multi, void *stream)
+{
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "lens_seqpr_stream_accumulate: bad sizes");
+    LENS_CHECK_ARG(L >= 1 && L <= P, "lens_seqpr_stream_accumulate: need 1 <= L <= P, got L=%d", L);
+    LENS_CHECK_ARG(t >= 0 && gt_tol >= 0, "lens_seqpr_stream_accumulate: t and gt_tol must be >= 0");
+    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "lens_seqpr_stream_accumulate: too many (stream, row) pairs");
+    LENS_CHECK_ARG(B == 0 || (S && seen && gt_center), "lens_seqpr_stream_accumulate: NULL S / seen / gt_center");
+    LENS_CHECK_ARG(B == 0 || L == 1 || ring, "lens_seqpr_stream_accumulate: NULL ring needs L == 1, got L=%d", L);
+    void *accs[3] = {acc_place, acc_query, acc_multi};
+    for (int m = 0; m < 3; ++m)
+        LENS_CHECK_ARG((reinterpret_cast<uintptr_t>(accs[m]) & 7) == 0,
+                       "lens_seqpr_stream_accumulate: accumulators must be 8-byte aligned");
+    if (B == 0 || !(acc_place || acc_query || acc_multi)) return 0;
+    SeqPrStreamArgs a{};
+    a.S = S; a.ring = ring; a.seen = seen; a.t = t;
+    a.B = B; a.Q = Q; a.P = P; a.L = L; a.Po = P - L + 1;
+    a.gt_center = gt_center; a.gt_tol = gt_tol;
+    for (int m = 0; m < 3; ++m) a.bad[m] = static_cast<unsigned long long *>(accs[m]);     // header word 0
+    if (acc_place) a.rec = reinterpret_cast<unsigned *>(static_cast<unsigned long long *>(acc_place) + 2);
+    if (acc_multi) {
+        a.multi_gtp = static_cast<unsigned long long *>(acc_multi) + 1;
+        a.hist = static_cast<unsigned long long *>(acc_multi) + 2;
+    }
+    cudaStream_t st = as_stream(stream);
+    if (acc_query) {
+        LENS_CUDA(cudaMallocAsync(&a.key, (size_t)B * Q * sizeof(unsigned long long), st));   // stream-ordered scratch
+        LENS_CUDA(cudaMemsetAsync(a.key, 0, (size_t)B * Q * sizeof(unsigned long long), st));
+    }
+    const long long sms = std::max(sm_count(), 1);
+    const long long items = (long long)B * ceil_div(a.Po, kPrTile);
+    const unsigned blocks = (unsigned)std::min<long long>(ceil_div64(items, 8), sms * 16);
+    const size_t smem = acc_multi ? 2 * kStreamShBins * sizeof(unsigned) : 0;
+    seqpr_stream_accumulate_kernel<<<blocks, 256, smem, st>>>(a);
+    LENS_LAUNCH_CHECK();
+    if (acc_query) {
+        unsigned long long *q = static_cast<unsigned long long *>(acc_query);
+        seqpr_stream_query_fold_kernel<<<(unsigned)std::min<long long>(ceil_div64((long long)B * Q, 256), sms * 8), 256,
+                                         0, st>>>(a, q + 2, q + 1);
+        LENS_LAUNCH_CHECK();
+        LENS_CUDA(cudaFreeAsync(a.key, st));
+    }
+    return 0;
+}
+
+extern "C" int lens_seqpr_stream_histogram(const void *acc, int B, int P, int L, int mode, uint64_t *hist,
+                                           int64_t *gtp, int64_t *n_bad, void *stream)
+{
+    LENS_CHECK_ARG(B >= 0 && P > 0 && L >= 1 && L <= P, "lens_seqpr_stream_histogram: bad sizes");
+    LENS_CHECK_ARG(mode == LENS_SEQPR_PLACE || mode == LENS_SEQPR_QUERY || mode == LENS_SEQPR_MULTI,
+                   "lens_seqpr_stream_histogram: unknown mode %d", mode);
+    LENS_CHECK_ARG(acc && hist && gtp && n_bad, "lens_seqpr_stream_histogram: NULL buffer");
+    LENS_CHECK_ARG((reinterpret_cast<uintptr_t>(acc) & 7) == 0, "lens_seqpr_stream_histogram: acc must be 8-byte aligned");
+    const unsigned long long *a = static_cast<const unsigned long long *>(acc);
+    auto *h = reinterpret_cast<unsigned long long *>(hist);
+    auto *g = reinterpret_cast<unsigned long long *>(gtp);
+    auto *nb = reinterpret_cast<unsigned long long *>(n_bad);
+    cudaStream_t st = as_stream(stream);
+    if (mode == LENS_SEQPR_PLACE) {
+        const long long n = (long long)B * (P - L + 1);
+        const long long sms = std::max(sm_count(), 1);
+        if (n > 0) {
+            seqpr_stream_place_hist_kernel<<<(unsigned)std::min<long long>(ceil_div64(n, 256), sms * 8), 256, 0, st>>>(
+                a, n, h, g, nb);
+            LENS_LAUNCH_CHECK();
+        }
+    } else {
+        seqpr_stream_add_kernel<<<(unsigned)ceil_div(2 * kStreamBins, 256), 256, 0, st>>>(a, h, g, nb);
+        LENS_LAUNCH_CHECK();
+    }
+    return 0;
+}
+
+extern "C" int lens_seqpr_hist_counts(const uint64_t *hist, int L, int n_thresh, int64_t *tp, int64_t *fp,
+                                      void *stream)
+{
+    LENS_CHECK_ARG(L >= 1, "lens_seqpr_hist_counts: need L >= 1, got L=%d", L);
+    LENS_CHECK_ARG(n_thresh >= 2 && n_thresh <= kPrMaxThresh,
+                   "lens_seqpr_hist_counts: n_thresh must be in [2, %d], got %d", kPrMaxThresh, n_thresh);
+    LENS_CHECK_ARG(hist && tp && fp, "lens_seqpr_hist_counts: NULL buffer");
+    cudaStream_t st = as_stream(stream);
+    unsigned long long *binned = nullptr;
+    const size_t bytes = (size_t)2 * n_thresh * sizeof(unsigned long long);
+    LENS_CUDA(cudaMallocAsync(&binned, bytes, st));                     // stream-ordered scratch
+    LENS_CUDA(cudaMemsetAsync(binned, 0, bytes, st));
+    seqpr_stream_bin_kernel<<<1, 1024, 0, st>>>(reinterpret_cast<const unsigned long long *>(hist), L, n_thresh, binned);
+    LENS_LAUNCH_CHECK();
+    seqpr_prefix_kernel<<<1, 64, 0, st>>>(binned, n_thresh, reinterpret_cast<unsigned long long *>(tp),
+                                          reinterpret_cast<unsigned long long *>(fp));
+    LENS_LAUNCH_CHECK();
+    LENS_CUDA(cudaFreeAsync(binned, st));
     return 0;
 }

@@ -237,6 +237,84 @@ def seqpr_counts(S, L, mode, records, extremes, n_thresh=100, gt_dense=None, gt_
     return tp, fp
 
 
+SEQPR_STREAM_BINS = 65536                      # LENS_SEQPR_STREAM_BINS: sequence sums k in [0, 65 535]
+SEQPR_STREAM_MODES = ("place", "query", "multi")   # index = LENS_SEQPR_* mode
+
+
+def _seqpr_stream_check(S, L, ring, seen, gt_center, accs):
+    """Shape checks of seqpr_stream_accumulate (before anything touches the device)."""
+    if not torch.is_tensor(S) or S.dtype != torch.float32 or S.dim() != 3:
+        raise ValueError("S must be f32 [B, Q, P]")
+    B, Q, P = S.shape
+    if not 1 <= L <= P:
+        raise ValueError(f"need 1 <= L <= P = {P}, got L={L}")
+    if not torch.is_tensor(seen) or seen.dtype != torch.int32 or tuple(seen.shape) != (B,):
+        raise ValueError(f"seen must be i32 [{B}]")
+    if L > 1 and (ring is None or ring.dtype != torch.float32 or tuple(ring.shape) != (B, L - 1, P)):
+        raise ValueError(f"ring must be f32 [{B}, {L - 1}, {P}]")
+    if not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32 or tuple(gt_center.shape) != (B, Q):
+        raise ValueError(f"gt_center must be i32 [{B}, {Q}]")
+    for mode, acc in enumerate(accs):
+        if acc is not None and (acc.dtype != torch.uint8 or acc.numel() != seqpr_stream_bytes(B, P, L, mode)):
+            raise ValueError(f"the {SEQPR_STREAM_MODES[mode]} accumulator must be u8 "
+                             f"[{seqpr_stream_bytes(B, P, L, mode)}] (seqpr_stream_bytes)")
+    return B, Q, P
+
+
+def seqpr_stream_bytes(B, P, L, mode):
+    """Size in bytes of one mode's session accumulator (lens_seqpr_stream_bytes); zeroed = an empty session."""
+    n = C.c_int64(0)
+    check(_lib.lib().lens_seqpr_stream_bytes(B, P, L, mode, C.byref(n)), "lens_seqpr_stream_bytes")
+    return int(n.value)
+
+
+def seqpr_stream_accumulate(S, L, ring, seen, t, gt_center, gt_tol=0, acc_place=None, acc_query=None,
+                            acc_multi=None):
+    """Fold the valid new rows of one push (S f32 [B, Q, P], with the ring / seen / t the push's
+    seqmatch_topk_stream call is about to use) into the session accumulators of the tracked modes (u8 tensors of
+    seqpr_stream_bytes, None = not tracked).  gt_center i32 [B, Q]: expected place of each new row, -1 = none."""
+    accs = (acc_place, acc_query, acc_multi)
+    B, Q, P = _seqpr_stream_check(S, L, ring, seen, gt_center, accs)
+    require_cuda(S, ring, seen, gt_center, *accs)
+    check(_lib.lib().lens_seqpr_stream_accumulate(ptr(S), B, Q, P, L, ptr(ring), ptr(seen), int(t), ptr(gt_center),
+                                                  int(gt_tol), *(ptr(a) for a in accs), stream_ptr()),
+          "lens_seqpr_stream_accumulate")
+
+
+def seqpr_stream_histogram(acc, B, P, L, mode, packed=None):
+    """One mode's accumulator -> packed i64 [2 * SEQPR_STREAM_BINS + 2] on the device: the histogram of k
+    (positives | negatives), then gtp and n_bad; accumulated into `packed` when given.  Summing the packed tensors
+    of several ranks makes one fleet."""
+    require_cuda(acc, packed)
+    if packed is None:
+        packed = torch.zeros((2 * SEQPR_STREAM_BINS + 2,), dtype=torch.int64, device=acc.device)
+    n = 2 * SEQPR_STREAM_BINS
+    check(_lib.lib().lens_seqpr_stream_histogram(ptr(acc), B, P, L, mode, ptr(packed), ptr(packed[n:n + 1]),
+                                                 ptr(packed[n + 1:]), stream_ptr()), "lens_seqpr_stream_histogram")
+    return packed
+
+
+def seqpr_stream_counts(packed, L, n_thresh=100):
+    """createPR's counts of a (summed) packed histogram -> (tp, fp) numpy i64 [n_thresh], gtp.  Raises LensError
+    when a sequence sum fell outside [0, 65 535] or was not an integer (the curve would be wrong), or when the
+    session has no column yet."""
+    if not 2 <= n_thresh <= SEQPR_MAX_THRESH:
+        raise ValueError(f"n_thresh must be in [2, {SEQPR_MAX_THRESH}], got {n_thresh}")
+    require_cuda(packed)
+    n = 2 * SEQPR_STREAM_BINS
+    out = torch.zeros((2 * n_thresh,), dtype=torch.int64, device=packed.device)
+    check(_lib.lib().lens_seqpr_hist_counts(ptr(packed), int(L), n_thresh, ptr(out[:n_thresh]), ptr(out[n_thresh:]),
+                                            stream_ptr()), "lens_seqpr_hist_counts")
+    host = torch.cat([out, packed[n:]]).cpu().numpy()
+    tp, fp, gtp, n_bad = host[:n_thresh], host[n_thresh:2 * n_thresh], int(host[-2]), int(host[-1])
+    if n_bad:
+        raise _lib.LensError(f"{n_bad} sequence sums were not integers in [0, {SEQPR_STREAM_BINS - 1}]: the session "
+                             "precision-recall needs integer spike counts")
+    if tp[-1] + fp[-1] == 0:
+        raise _lib.LensError("the precision-recall session has no valid row yet")
+    return tp, fp, gtp
+
+
 def topn_merge(vals, idx):
     """Global top-N from W per-shard lists: vals f32 / idx i32 [W, B, Qo, N] (idx = global place index, -1 =
     empty) -> (val [B, Qo, N], idx [B, Qo, N]) under the order (value desc, place index desc)."""

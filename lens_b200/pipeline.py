@@ -245,26 +245,41 @@ class StreamingPipeline(InferencePipeline):
     f32 [n_streams, L - 1, P] (the last L - 1 spike-count rows of every stream, row g at slot g mod (L - 1)),
     `seen` i32 [n_streams] (rows since each stream's reset, saturating at L - 1) and `t` (rows pushed).  Under
     torch.distributed every rank builds one for its own shard of streams; the Recall@N counters are all-reduced
-    like `step`'s."""
+    like `step`'s.
+
+    `track_pr` (any of "place", "query", "multi") also accumulates createPR's precision-recall curve of the session
+    on the GPU, push by push, in bounded memory: see `session_precision_recall`.  The "place" accumulator holds
+    4 bytes per (stream, place), the other two 1 MB each."""
 
     def __init__(self, W_feat, W_out, roi, k, T, L, n_streams, n_top=25, ns=ops.RECALL_NS, device=None,
-                 mode=MODE_AUTO):
+                 mode=MODE_AUTO, track_pr=()):
         super().__init__(W_feat, W_out, roi, k, T, L, n_top=n_top, ns=ns, max_streams=n_streams, device=device,
                          mode=mode)
         self.n_streams = int(n_streams)
         if self.L < 1 or self.L > self.net.P:
             raise LensError(f"need 1 <= L <= P={self.net.P}, got L={self.L}")
+        track_pr = (track_pr,) if isinstance(track_pr, str) else tuple(track_pr)
+        unknown = set(track_pr) - set(ops.SEQPR_STREAM_MODES)
+        if unknown:
+            raise LensError(f"track_pr takes modes from {ops.SEQPR_STREAM_MODES}, got {sorted(unknown)}")
         # never read before it is written (a row is used only once its stream has seen it): left uninitialised
         self.ring = (torch.empty((self.n_streams, self.L - 1, self.net.P), dtype=torch.float32, device=self.device)
                      if self.L > 1 else None)
         self.seen = torch.zeros((self.n_streams,), dtype=torch.int32, device=self.device)
         self.t = 0
+        # session accumulators of the tracked precision-recall modes (zeroed = empty session)
+        self._pr_acc = {m: torch.zeros((ops.seqpr_stream_bytes(self.n_streams, self.net.P, self.L, i),),
+                                       dtype=torch.uint8, device=self.device)
+                        for i, m in enumerate(ops.SEQPR_STREAM_MODES) if m in track_pr}
 
     def _check_streams(self, B):
         if B != self.n_streams:
             raise LensError(f"this pipeline serves {self.n_streams} streams; the push has {B}")
 
-    def _check_gt(self, gt_center, Q):
+    def _check_gt(self, gt_center, Q, gt_tol):
+        if self._pr_acc and (gt_center is None or gt_tol < 0):
+            raise LensError(f"precision-recall tracking ({', '.join(self._pr_acc)}) needs gt_center and gt_tol >= 0 "
+                            "on every push")
         if gt_center is not None and (not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32
                                       or tuple(gt_center.shape) != (self.n_streams, Q)):
             raise LensError(f"gt_center must be i32 [{self.n_streams}, {Q}]")
@@ -275,21 +290,30 @@ class StreamingPipeline(InferencePipeline):
         raise LensError("StreamingPipeline is a live session: feed it with push / push_events "
                         "(use an InferencePipeline for batch steps)")
 
-    # precision_recall needs whole sequences, and a push's S holds only the new rows
-    step = step_events = step_event_groups = step_host = precision_recall = _offline
+    step = step_events = step_event_groups = step_host = _offline
+
+    def precision_recall(self, *args, **kwargs):
+        # the batch method needs whole sequences, and a push's S holds only the new rows
+        raise LensError("StreamingPipeline is a live session: construct it with track_pr=(...) and call "
+                        "session_precision_recall for the curve of the rows pushed so far")
 
     def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True):
         """Q new windows of every stream: frames u8 [B, Q, roi, roi] or pooled u8 [B, Q, I], B = n_streams.
         -> `step`'s dict with top_val / top_idx [B, Q, N] (row q = the sequence ending at new row q), S [B, Q, P],
-        and hits / n_valid for this push.  gt_center i32 [B, Q] (optional) is the expected place of the sequence
-        ending at each new row (band ground truth, |idx - center| <= gt_tol); warm-up rows never count."""
+        and hits / n_valid for this push.  gt_center i32 [B, Q] (optional; required with track_pr) is the expected
+        place of the sequence ending at each new row (band ground truth, |idx - center| <= gt_tol, -1 = none);
+        warm-up rows never count.  With track_pr the valid new rows also join the precision-recall session; what
+        the push returns is the same as without tracking."""
         x = frames if frames is not None else pooled
         if x is None or (frames is not None and pooled is not None):
             raise LensError("give exactly one of frames / pooled")
         self._check_streams(x.shape[0])
-        self._check_gt(gt_center, x.shape[1])
+        self._check_gt(gt_center, x.shape[1], gt_tol)
         with torch.cuda.device(self.device):
             S = self.similarity(frames=frames, pooled=pooled)
+            if self._pr_acc:      # before the match, which advances seen and overwrites ring slots
+                ops.seqpr_stream_accumulate(S, self.L, self.ring, self.seen, self.t, gt_center, gt_tol,
+                                            **{"acc_" + m: a for m, a in self._pr_acc.items()})
             tv, ti = ops.seqmatch_topk_stream(S, self.L, self.n_top, self.ring, self.seen, self.t)
             self.t += S.shape[1]
             out = dict(top_val=tv, top_idx=ti, D=None, hits=None, n_valid=None, S=S,
@@ -308,7 +332,7 @@ class StreamingPipeline(InferencePipeline):
         [t0_us[b] + q * window_us, + window_us) of its events [offsets[b], offsets[b+1]) (as in `step_events`).
         Returns `push`'s dict plus "events_per_window" i32 [B, Q]."""
         self._check_streams(offsets.numel() - 1)
-        self._check_gt(gt_center, int(Q))
+        self._check_gt(gt_center, int(Q), gt_tol)
         with torch.cuda.device(self.device):
             pooled, n_ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
             out = self.push(pooled=pooled, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce)
@@ -339,10 +363,46 @@ class StreamingPipeline(InferencePipeline):
             self.seen.masked_fill_(mask, 0)
 
     def reset(self):
-        """Every stream from scratch: SNN state (and the overflow counter), sequence history, and t."""
+        """Every stream from scratch: SNN state (and the overflow counter), sequence history, t, and a new
+        precision-recall session."""
         self.net.reset_states()
         self.seen.zero_()
         self.t = 0
+        self.reset_precision_recall()
+
+    def reset_precision_recall(self):
+        """Start a new precision-recall session; streams, ring and t are left alone.  (`reset_streams` does not
+        start one: a restarted stream's later valid rows are more columns of the same session.)"""
+        for acc in self._pr_acc.values():
+            acc.zero_()
+
+    def session_precision_recall(self, matching="single", best="place", n_thresh=100, reduce=True):
+        """createPR's precision-recall lists over every valid row pushed since construction, `reset()` or
+        `reset_precision_recall()`, in the format of InferencePipeline.precision_recall: dict(P, R, tp, fp, gtp).
+
+        A stream's session matrix has its valid rows as query columns, in push order; the fleet (and, under
+        torch.distributed with reduce=True, every rank) concatenates along createPR's column axis.  For a fresh
+        pipeline without stream resets the result equals `precision_recall` of one batch step over all the windows,
+        with gt_center[:, L - 1:].  The mode (matching / best as in `precision_recall`) must be tracked.  Raises
+        LensError for an untracked mode, an empty session, or spike counts whose sequence sums are not integers in
+        [0, 65 535].  Under torch.distributed: one all-reduce SUM of about 1 MB."""
+        from .src.metrics import pr_lists
+        mode = ops.seqpr_mode(matching, best)
+        name = ops.SEQPR_STREAM_MODES[mode]
+        if name not in self._pr_acc:
+            raise LensError(f"precision-recall mode {name!r} is not tracked: construct the pipeline with "
+                            f"track_pr=({name!r}, ...)")
+        if not 2 <= n_thresh <= ops.SEQPR_MAX_THRESH:
+            raise ValueError(f"n_thresh must be in [2, {ops.SEQPR_MAX_THRESH}], got {n_thresh}")
+        dist = torch.distributed
+        shared = reduce and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+        with torch.cuda.device(self.device):
+            packed = ops.seqpr_stream_histogram(self._pr_acc[name], self.n_streams, self.net.P, self.L, mode)
+            if shared:
+                dist.all_reduce(packed)                     # [hist, gtp, n_bad]
+            tp, fp, gtp = ops.seqpr_stream_counts(packed, self.L, n_thresh)
+        P, R = pr_lists(tp, fp, gtp)
+        return dict(P=P, R=R, tp=tp, fp=fp, gtp=gtp)
 
 
 class PlaceShardedPipeline:
