@@ -26,6 +26,12 @@
  *   lens_seqmatch_topk     N <= 64, 1 <= L <= min(Q, P)
  *   lens_seqmatch_topk_stream
  *                          N <= 64, 1 <= L <= P, Q >= 1, B * Q <= 2^31 - 1; ring non-NULL unless L == 1, seen non-NULL
+ *   lens_seqmatch_topk_stream_ids / lens_seqpr_stream_accumulate_ids
+ *                          as their lockstep forms with n * Q <= 2^31 - 1; ids [n] i32 of the fleet of B: an id outside
+ *                          [0, B) is skipped (never an out-of-bounds access), duplicate ids give unspecified values
+ *   lens_snn_forward_streams
+ *                          n * (I + F + P) * 4 bytes of handle-owned workspace (n rounded up to even), kept for the
+ *                          largest n seen; ids outside [0, max_streams) are skipped, duplicates unspecified
  *   lens_recall / _bounds  at most 8 values of N per call
  *   lens_pr_counts         Qo <= 8192 (one CTA, shared-memory resident)
  *   lens_seqpr_scan / _counts
@@ -190,6 +196,16 @@ int lens_snn_forward(void *handle, const uint8_t *pooled, int B, int Q, float *c
 int lens_snn_forward_range(void *handle, const uint8_t *pooled, int b0, int nb, int Q, float *counts,
                            uint8_t *hidden_steps, uint8_t *out_steps, int mode, void *stream);
 
+/* lens_snn_forward for the streams ids[0..n) of the handle, in any order, each advancing from its own state; every
+ * other stream's state is untouched.  pooled [n][Q][I] u8 and counts [n][Q][P] f32 are by position (row i is stream
+ * ids[i]); ids [n] i32 device.  The rows ids[i] of v0 / v1 / v2 are gathered into a handle-owned workspace, run through
+ * the same kernels as lens_snn_forward (mode as there; the counts equal those of lens_snn_forward on the same state),
+ * and scattered back: two launches more than lens_snn_forward, 2 * 2 * n * (I + F + P) * 4 bytes of extra traffic.
+ * The workspace grows on the first call with a larger n (a cudaMalloc) and is freed with the handle.  n = 0 or Q = 0
+ * returns 0 without launching.                                                                                   */
+int lens_snn_forward_streams(void *handle, const uint8_t *pooled, const int32_t *ids, int n, int Q, float *counts,
+                             int mode, void *stream);
+
 /* Operator seam `sinabs_model(x)` (lens/run_model.py:238) for an arbitrary float
  * raster: x [B][steps][I] f32 (already pooled), spikes_out [B][steps][P] f32.     */
 int lens_snn_forward_float(void *handle, const float *x, int B, int steps, float *spikes_out,
@@ -225,6 +241,19 @@ int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, int N, float 
  * segmented kernel and lens_topn_merge's kernel); never more with B.  B = 0 returns 0 without launching.  */
 int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, int L, int N, float *ring, int32_t *seen,
                               int64_t t, float *top_val, int32_t *top_idx, void *stream);
+/* The same for any subset of a fleet of B streams, in any order: the n streams ids[0..n) each push Q new rows, and
+ * every other stream keeps its ring rows, seen and row counter.  Stream ids[i]'s rows are numbered by its own counter:
+ *   S       [n][Q][P] f32, row i = stream ids[i]; top_val / top_idx [n][Q][N] by position, as above
+ *   ids     [n] i32 device, distinct fleet indices in [0, B)
+ *   ring    [B][L-1][P], seen [B] as above (row g of stream b at slot g mod (L-1), g counted by rows[b])
+ *   rows    [B] i64 device: rows pushed to each stream (replaces the scalar t; a lockstep session has rows[b] = t)
+ * Matches, then appends to the ring, then advances seen[ids[i]] (saturating) and rows[ids[i]] += Q (stream order).
+ * For each pushed stream the result is exactly that of lens_seqmatch_topk_stream on that one stream with t = rows[b].
+ * Three launches per call (two when L == 1), four when the places of a row are split into segments; never more with
+ * n.  n = 0 returns 0 without launching.                                                                        */
+int lens_seqmatch_topk_stream_ids(const float *S, int n, int Q, int P, int L, int N, const int32_t *ids, int B,
+                                  float *ring, int32_t *seen, int64_t *rows, float *top_val, int32_t *top_idx,
+                                  void *stream);
 
 /* Recall@N counters (lens/src/metrics.py:213-224 + lens/run_model.py:301-302).
  * Ground truth is either dense, gt_dense [B or 1][Po][Qo] u8 (gt_stream_stride = Po*Qo
@@ -319,6 +348,10 @@ int lens_seqpr_counts(const float *S, int B, int Q, int P, int L, int mode, cons
  *                                advances seen and overwrites ring slots).  gt_center [B][Q] i32: the expected place
  *                                of each new row (< 0: no positive), positives |p - center| <= gt_tol.  One launch,
  *                                two when the query mode is tracked; never more with B.
+ *   lens_seqpr_stream_accumulate_ids
+ *                                the same for the push of lens_seqmatch_topk_stream_ids (S, n, ids, B, ring, seen, rows
+ *                                as for that call, which must come AFTER this one); gt_center [n][Q] by position, the
+ *                                accumulators sized for the fleet of B.  Launches as above; n = 0 launches nothing.
  *   lens_seqpr_stream_histogram  one accumulator -> hist [2][LENS_SEQPR_STREAM_BINS] u64 (positives | negatives per
  *                                k), gtp [1], n_bad [1], all ACCUMULATED.  Sums of these over ranks form one fleet.
  *   lens_seqpr_hist_counts       tp, fp [n_thresh] i64 ACCUMULATED: thresholds np.linspace(max, min, n_thresh) of the
@@ -329,6 +362,10 @@ int lens_seqpr_stream_bytes(int B, int P, int L, int mode, int64_t *bytes);
 int lens_seqpr_stream_accumulate(const float *S, int B, int Q, int P, int L, const float *ring, const int32_t *seen,
                                  int64_t t, const int32_t *gt_center, int gt_tol, void *acc_place, void *acc_query,
                                  void *acc_multi, void *stream);
+int lens_seqpr_stream_accumulate_ids(const float *S, int n, int Q, int P, int L, const int32_t *ids, int B,
+                                     const float *ring, const int32_t *seen, const int64_t *rows,
+                                     const int32_t *gt_center, int gt_tol, void *acc_place, void *acc_query,
+                                     void *acc_multi, void *stream);
 int lens_seqpr_stream_histogram(const void *acc, int B, int P, int L, int mode, uint64_t *hist, int64_t *gtp,
                                 int64_t *n_bad, void *stream);
 int lens_seqpr_hist_counts(const uint64_t *hist, int L, int n_thresh, int64_t *tp, int64_t *fp, void *stream);

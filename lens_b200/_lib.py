@@ -43,8 +43,10 @@ def _declare(L):
         "lens_snn_forward": (i32, [vp, vp, i32, i32, vp, vp, vp, i32, vp]),
         "lens_snn_forward_range": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, i32, vp]),
         "lens_snn_forward_float": (i32, [vp, vp, i32, i32, vp, vp]),
+        "lens_snn_forward_streams": (i32, [vp, vp, vp, i32, i32, vp, i32, vp]),
         "lens_seqmatch_topk": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, vp, vp]),
         "lens_seqmatch_topk_stream": (i32, [vp, i32, i32, i32, i32, i32, vp, vp, i64, vp, vp, vp]),
+        "lens_seqmatch_topk_stream_ids": (i32, [vp, i32, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp, vp, vp]),
         "lens_sad_matrix": (i32, [vp, vp, i32, i32, i32, vp, vp]),
         "lens_reciprocal": (i32, [vp, i64, vp, vp]),
         "lens_online_accumulate": (i32, [vp, vp, i32, i32, vp, vp]),
@@ -61,6 +63,8 @@ def _declare(L):
         "lens_seqpr_counts": (i32, [vp, i32, i32, i32, i32, i32, vp, i64, vp, i32, vp, vp, i32, vp, vp, vp]),
         "lens_seqpr_stream_bytes": (i32, [i32, i32, i32, i32, pi64]),
         "lens_seqpr_stream_accumulate": (i32, [vp, i32, i32, i32, i32, vp, vp, i64, vp, i32, vp, vp, vp, vp]),
+        "lens_seqpr_stream_accumulate_ids": (i32, [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp, i32, vp, vp, vp,
+                                                   vp]),
         "lens_seqpr_stream_histogram": (i32, [vp, i32, i32, i32, i32, vp, vp, vp, vp]),
         "lens_seqpr_hist_counts": (i32, [vp, i32, i32, vp, vp, vp]),
     }

@@ -229,15 +229,15 @@ seqmatch_topk_warp_kernel(const float *__restrict__ S, long long n_queries, int 
 // (t + q - L + 1 + j) mod (L - 1).  The choice depends on (q, j) only, so the pointer is warp-uniform per term and
 // the loads along the places stay coalesced as in the batch kernels.
 struct StreamRows {
-    const float *Sq;       // new row q of stream b
-    const float *ring_b;   // [L-1][P] ring of stream b
+    const float *Sq;       // new row q of the stream at position b of S
+    const float *ring_b;   // [L-1][P] ring of fleet stream fb
     int n_old;             // terms j < n_old come from the ring
     int slot0;             // ring slot of term 0 (valid rows only: t + q - L + 1 >= 0 there)
     int Lm1, L;
     size_t P;
-    __device__ __forceinline__ StreamRows(const float *S, const float *ring, int b, int Q, int q, int P_, int L_,
+    __device__ __forceinline__ StreamRows(const float *S, const float *ring, int b, int fb, int Q, int q, int P_, int L_,
                                           long long t)
-        : Sq(S + ((size_t)b * Q + q) * P_), ring_b(ring + (size_t)b * (L_ - 1) * P_), n_old(max(L_ - 1 - q, 0)),
+        : Sq(S + ((size_t)b * Q + q) * P_), ring_b(ring + (size_t)fb * (L_ - 1) * P_), n_old(max(L_ - 1 - q, 0)),
           slot0(L_ > 1 ? (int)((t + q - L_ + 1) % (L_ - 1)) : 0), Lm1(L_ - 1), L(L_), P((size_t)P_) {}
     __device__ __forceinline__ const float *row(int j) const
     {
@@ -256,13 +256,33 @@ __device__ __forceinline__ bool stream_row_valid(const int32_t *__restrict__ see
     return __ldg(seen + b) + q + 1 >= L;
 }
 
+// Every streaming kernel below serves two kinds of call.  Lockstep (kIdx = false, lens_seqmatch_topk_stream): position
+// b of S is fleet stream b and every stream has had t rows.  Indexed (kIdx = true, the *_ids entry points): position b
+// is fleet stream fb = ids[b] of n_fleet, with its own row counter rows[fb].  The ring, seen and the place records are
+// the fleet's (index fb); S, gt_center, per-push scratch and outputs are by position.  An id outside [0, n_fleet) is
+// skipped (-> false).  The lockstep kernels keep their names and code; the indexed ones are separate entry points of
+// the same bodies.
+template <bool kIdx>
+__device__ __forceinline__ bool fleet_stream(const int32_t *__restrict__ ids, const int64_t *__restrict__ rows,
+                                             int n_fleet, int b, long long t, int &fb, long long &tb)
+{
+    fb = b;
+    tb = t;
+    if (!kIdx) return true;
+    fb = __ldg(ids + b);
+    if ((unsigned)fb >= (unsigned)n_fleet) return false;
+    tb = __ldg(rows + fb);
+    return true;
+}
+
 // The warp-per-query kernel (N <= 32) over the B * Q new rows, kSeg as in seqmatch_topk_warp_kernel.  A warm-up row
 // (not valid) skips the scan and stores an empty list.
-template <bool kSeg>
-__global__ void __launch_bounds__(256, kSeg ? 1 : 6)
-seqmatch_topk_stream_warp_kernel(const float *__restrict__ S, const float *__restrict__ ring,
-                                 const int32_t *__restrict__ seen, long long t, long long n_queries, int Q, int P, int L,
-                                 int N, int n_seg, int seg_len, float *__restrict__ top_val, int32_t *__restrict__ top_idx)
+template <bool kSeg, bool kIdx>
+__device__ __forceinline__ void
+stream_warp_topk(const float *__restrict__ S, const float *__restrict__ ring, const int32_t *__restrict__ seen,
+                 long long t, const int32_t *__restrict__ ids, const int64_t *__restrict__ rows, int n_fleet,
+                 long long n_queries, int Q, int P, int L, int N, int n_seg, int seg_len, float *__restrict__ top_val,
+                 int32_t *__restrict__ top_idx)
 {
     const int lane = threadIdx.x & 31;
     const int Po_all = P - L + 1;
@@ -275,8 +295,10 @@ seqmatch_topk_stream_warp_kernel(const float *__restrict__ S, const float *__res
         const int b = (int)(g / Q), q = (int)(g - (long long)b * Q);
         const int Po = kSeg ? min(Po_all, (seg + 1) * seg_len) : Po_all;
         unsigned long long best = 0ull;                    // lane i: i-th largest key, 0 = empty
-        if (stream_row_valid(seen, b, q, L)) {
-            const StreamRows rows(S, ring, b, Q, q, P, L, t);
+        int fb;
+        long long tb;
+        if (fleet_stream<kIdx>(ids, rows, n_fleet, b, t, fb, tb) && stream_row_valid(seen, fb, q, L)) {
+            const StreamRows rr(S, ring, b, fb, Q, q, P, L, tb);
             for (int r0 = kSeg ? seg * seg_len : 0; r0 < Po; r0 += 32 * kUnrollR) {
                 float acc[kUnrollR];
 #pragma unroll
@@ -286,13 +308,13 @@ seqmatch_topk_stream_warp_kernel(const float *__restrict__ S, const float *__res
                     // (the batch kernel re-reads each row L times from L2), so more bytes must be in flight
 #pragma unroll 2
                     for (int j = 0; j < L; ++j) {
-                        const float *row = rows.row(j) + (r0 + lane + j);
+                        const float *row = rr.row(j) + (r0 + lane + j);
 #pragma unroll
                         for (int u = 0; u < kUnrollR; ++u) acc[u] += __ldg(row + 32 * u);
                     }
                 } else {
                     for (int j = 0; j < L; ++j) {
-                        const float *row = rows.row(j) + (r0 + lane + j);
+                        const float *row = rr.row(j) + (r0 + lane + j);
 #pragma unroll
                         for (int u = 0; u < kUnrollR; ++u)
                             if (r0 + 32 * u + lane < Po) acc[u] += __ldg(row + 32 * u);
@@ -313,11 +335,36 @@ seqmatch_topk_stream_warp_kernel(const float *__restrict__ S, const float *__res
     }
 }
 
-// The CTA-per-query kernel (32 < N <= 64) over the B * Q new rows; grid = B * Q.
+template <bool kSeg>
+__global__ void __launch_bounds__(256, kSeg ? 1 : 6)
+seqmatch_topk_stream_warp_kernel(const float *__restrict__ S, const float *__restrict__ ring,
+                                 const int32_t *__restrict__ seen, long long t, long long n_queries, int Q, int P, int L,
+                                 int N, int n_seg, int seg_len, float *__restrict__ top_val, int32_t *__restrict__ top_idx)
+{
+    stream_warp_topk<kSeg, false>(S, ring, seen, t, nullptr, nullptr, 0, n_queries, Q, P, L, N, n_seg, seg_len, top_val,
+                                  top_idx);
+}
+
+template <bool kSeg>
+__global__ void __launch_bounds__(256, kSeg ? 1 : 6)
+seqmatch_topk_stream_ids_warp_kernel(const float *__restrict__ S, const float *__restrict__ ring,
+                                     const int32_t *__restrict__ seen, const int32_t *__restrict__ ids,
+                                     const int64_t *__restrict__ rows, int n_fleet, long long n_queries, int Q, int P,
+                                     int L, int N, int n_seg, int seg_len, float *__restrict__ top_val,
+                                     int32_t *__restrict__ top_idx)
+{
+    stream_warp_topk<kSeg, true>(S, ring, seen, 0, ids, rows, n_fleet, n_queries, Q, P, L, N, n_seg, seg_len, top_val,
+                                 top_idx);
+}
+
+// The CTA-per-query kernel (32 < N <= 64) over the B * Q new rows; grid = B * Q.  (Its name is not pinned, so the
+// indexed form is a template argument with ids / rows / n_fleet appended, which the lockstep form never reads.)
+template <bool kIdx>
 __global__ void __launch_bounds__(kMatchThreads)
 seqmatch_topk_stream_kernel(const float *__restrict__ S, const float *__restrict__ ring,
                             const int32_t *__restrict__ seen, long long t, int Q, int P, int L, int N,
-                            float *__restrict__ top_val, int32_t *__restrict__ top_idx)
+                            float *__restrict__ top_val, int32_t *__restrict__ top_idx, const int32_t *__restrict__ ids,
+                            const int64_t *__restrict__ rows, int n_fleet)
 {
     __shared__ unsigned long long cand[kCandChunk];
     __shared__ unsigned long long best[kMaxTopN];
@@ -329,14 +376,16 @@ seqmatch_topk_stream_kernel(const float *__restrict__ S, const float *__restrict
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const float fl = (float)L;
     for (int i = tid; i < kMaxTopN; i += kMatchThreads) best[i] = 0ull;
-    if (stream_row_valid(seen, b, q, L)) {                 // block-uniform
-        const StreamRows rows(S, ring, b, Q, q, P, L, t);
+    int fb;
+    long long tb;
+    if (fleet_stream<kIdx>(ids, rows, n_fleet, b, t, fb, tb) && stream_row_valid(seen, fb, q, L)) {   // block-uniform
+        const StreamRows rr(S, ring, b, fb, Q, q, P, L, kIdx ? tb : t);
         for (int r0 = 0; r0 < Po; r0 += kCandChunk) {
             const int nr = min(kCandChunk, Po - r0);
             for (int i = tid; i < nr; i += kMatchThreads) {
                 const int r = r0 + i;
                 float acc = 0.0f;
-                for (int j = 0; j < L; ++j) acc += __ldg(rows.row(j) + (r + j));
+                for (int j = 0; j < L; ++j) acc += __ldg(rr.row(j) + (r + j));
                 cand[i] = ((unsigned long long)f32_orderable(__fdiv_rn(acc, fl)) << 32) | (uint32_t)r;
             }
             __syncthreads();
@@ -347,11 +396,14 @@ seqmatch_topk_stream_kernel(const float *__restrict__ S, const float *__restrict
 }
 
 // After the match (stream order: it reads the slots this overwrites): the last n_app = min(Q, L - 1) new rows of
-// every stream go to their ring slots (t + q) mod (L - 1), and seen advances by Q, saturating at L - 1.
-// One CTA per (stream, appended row) at a time, 16-byte copies when rows allow them.
-__global__ void __launch_bounds__(256)
-ring_append_kernel(const float *__restrict__ S, int B, int Q, int P, int L, long long t, float *__restrict__ ring,
-                   int32_t *__restrict__ seen)
+// every stream go to their ring slots (t + q) mod (L - 1), and seen advances by Q, saturating at L - 1 (indexed calls:
+// in stream_advance_kernel, which runs after every reader of rows).  One CTA per (stream, appended row) at a time,
+// 16-byte copies when rows allow them.
+template <bool kIdx>
+__device__ __forceinline__ void ring_append(const float *__restrict__ S, int B, int Q, int P, int L, long long t,
+                                            float *__restrict__ ring, int32_t *__restrict__ seen,
+                                            const int32_t *__restrict__ ids, const int64_t *__restrict__ rows,
+                                            int n_fleet)
 {
     const int Lm1 = L - 1, n_app = min(Q, Lm1);
     const long long n_rows = (long long)B * n_app;
@@ -359,8 +411,11 @@ ring_append_kernel(const float *__restrict__ S, int B, int Q, int P, int L, long
     for (long long i = blockIdx.x; i < n_rows; i += gridDim.x) {
         const int b = (int)(i / n_app), k = (int)(i - (long long)b * n_app);
         const int q = Q - n_app + k;
+        int fb;
+        long long tb;
+        if (!fleet_stream<kIdx>(ids, rows, n_fleet, b, t, fb, tb)) continue;        // block-uniform
         const float *src = S + ((size_t)b * Q + q) * P;
-        float *dst = ring + ((size_t)b * Lm1 + (int)((t + q) % Lm1)) * P;
+        float *dst = ring + ((size_t)fb * Lm1 + (int)((tb + q) % Lm1)) * P;
         if (vec) {
             const float4 *s4 = reinterpret_cast<const float4 *>(src);
             float4 *d4 = reinterpret_cast<float4 *>(dst);
@@ -368,7 +423,34 @@ ring_append_kernel(const float *__restrict__ S, int B, int Q, int P, int L, long
         } else {
             for (int p = threadIdx.x; p < P; p += blockDim.x) dst[p] = __ldg(src + p);
         }
-        if (k == 0 && threadIdx.x == 0) seen[b] = (int32_t)min((long long)seen[b] + Q, (long long)Lm1);
+        if (!kIdx && k == 0 && threadIdx.x == 0) seen[b] = (int32_t)min((long long)seen[b] + Q, (long long)Lm1);
+    }
+}
+
+__global__ void __launch_bounds__(256)
+ring_append_kernel(const float *__restrict__ S, int B, int Q, int P, int L, long long t, float *__restrict__ ring,
+                   int32_t *__restrict__ seen)
+{
+    ring_append<false>(S, B, Q, P, L, t, ring, seen, nullptr, nullptr, 0);
+}
+
+__global__ void __launch_bounds__(256)
+ring_append_ids_kernel(const float *__restrict__ S, int B, int Q, int P, int L, float *__restrict__ ring,
+                       const int32_t *__restrict__ ids, const int64_t *__restrict__ rows, int n_fleet)
+{
+    ring_append<true>(S, B, Q, P, L, 0, ring, nullptr, ids, rows, n_fleet);
+}
+
+// Indexed calls, last: seen[ids[i]] advances by Q (saturating at L - 1) and rows[ids[i]] by Q.
+__global__ void __launch_bounds__(256)
+stream_advance_kernel(const int32_t *__restrict__ ids, int n, int n_fleet, int Q, int L, int32_t *__restrict__ seen,
+                      int64_t *__restrict__ rows)
+{
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int fb = ids[i];
+        if ((unsigned)fb >= (unsigned)n_fleet) continue;
+        seen[fb] = (int32_t)min((long long)seen[fb] + Q, (long long)(L - 1));
+        rows[fb] += Q;
     }
 }
 
@@ -987,7 +1069,10 @@ __device__ __forceinline__ void stream_hist_flush(const unsigned *s_h, unsigned 
 
 // One warp per (stream, kPrTile places), the push's new rows in order; warm-up rows are skipped.  The diagonal terms
 // come through StreamRows as in seqmatch_topk_stream_warp_kernel, so this runs before that call (same t, same seen).
-__global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_kernel(SeqPrStreamArgs a)
+// kIdx as in the streaming match: place records by fleet stream, gt_center and the query scratch by position.
+template <bool kIdx>
+__device__ __forceinline__ void stream_accumulate(SeqPrStreamArgs a, const int32_t *__restrict__ ids,
+                                                  const int64_t *__restrict__ rows_of, int n_fleet)
 {
     extern __shared__ unsigned s_h[];    // multi mode: [2][kStreamShBins]
     const int lane = threadIdx.x & 31;
@@ -1001,15 +1086,18 @@ __global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_kernel(SeqPrSt
     unsigned bad = 0, pos = 0;                       // per lane: at most kUnrollR * Q entries per item
     for (long long w = warp0; w < n_items; w += n_warps) {
         const int b = (int)(w / n_tiles), p0 = (int)(w - (long long)b * n_tiles) * kPrTile;
+        int fb;
+        long long tb;
+        if (!fleet_stream<kIdx>(ids, rows_of, n_fleet, b, a.t, fb, tb)) continue;     // warp-uniform
         unsigned rec[kUnrollR];
 #pragma unroll
         for (int u = 0; u < kUnrollR; ++u) {
             const int p = p0 + 32 * u + lane;
-            rec[u] = (a.rec && p < a.Po) ? a.rec[(size_t)b * a.Po + p] : 0u;
+            rec[u] = (a.rec && p < a.Po) ? a.rec[(size_t)fb * a.Po + p] : 0u;
         }
         for (int q = 0; q < a.Q; ++q) {
-            if (!stream_row_valid(a.seen, b, q, a.L)) continue;           // warp-uniform
-            const StreamRows rows(a.S, a.ring, b, a.Q, q, a.P, a.L, a.t);
+            if (!stream_row_valid(a.seen, fb, q, a.L)) continue;          // warp-uniform
+            const StreamRows rows(a.S, a.ring, b, fb, a.Q, q, a.P, a.L, kIdx ? tb : a.t);
             float acc[kUnrollR];
 #pragma unroll
             for (int u = 0; u < kUnrollR; ++u) acc[u] = 0.0f;
@@ -1064,7 +1152,7 @@ __global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_kernel(SeqPrSt
 #pragma unroll
             for (int u = 0; u < kUnrollR; ++u) {
                 const int p = p0 + 32 * u + lane;
-                if (p < a.Po) a.rec[(size_t)b * a.Po + p] = rec[u];
+                if (p < a.Po) a.rec[(size_t)fb * a.Po + p] = rec[u];
             }
         }
     }
@@ -1078,15 +1166,33 @@ __global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_kernel(SeqPrSt
     if (a.hist) stream_hist_flush(s_h, a.hist);
 }
 
+__global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_kernel(SeqPrStreamArgs a)
+{
+    stream_accumulate<false>(a, nullptr, nullptr, 0);
+}
+
+__global__ void __launch_bounds__(256, 4) seqpr_stream_accumulate_ids_kernel(SeqPrStreamArgs a,
+                                                                             const int32_t *__restrict__ ids,
+                                                                             const int64_t *__restrict__ rows,
+                                                                             int n_fleet)
+{
+    stream_accumulate<true>(a, ids, rows, n_fleet);
+}
+
 // Query mode, after the accumulate kernel: one thread per new row folds its first maximum into the histogram and
 // clears the scratch; gtp counts the valid rows with a positive among the places [0, Po).
-__global__ void __launch_bounds__(256) seqpr_stream_query_fold_kernel(SeqPrStreamArgs a, unsigned long long *acc_hist,
-                                                                      unsigned long long *gtp)
+template <bool kIdx>
+__device__ __forceinline__ void stream_query_fold(const SeqPrStreamArgs &a, unsigned long long *acc_hist,
+                                                  unsigned long long *gtp, const int32_t *__restrict__ ids,
+                                                  const int64_t *__restrict__ rows, int n_fleet)
 {
     const long long n = (long long)a.B * a.Q;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         const int b = (int)(i / a.Q), q = (int)(i - (long long)b * a.Q);
-        if (!stream_row_valid(a.seen, b, q, a.L)) continue;
+        int fb;
+        long long tb;
+        if (!fleet_stream<kIdx>(ids, rows, n_fleet, b, a.t, fb, tb) || !stream_row_valid(a.seen, fb, q, a.L))
+            continue;
         const unsigned long long key = a.key[i];
         a.key[i] = 0ull;
         const int c = __ldg(a.gt_center + i);
@@ -1096,6 +1202,22 @@ __global__ void __launch_bounds__(256) seqpr_stream_query_fold_kernel(SeqPrStrea
         const bool g = c >= 0 && abs(p - c) <= a.gt_tol;
         atomicAdd(acc_hist + (g ? 0 : kStreamBins) + k, 1ull);
     }
+}
+
+__global__ void __launch_bounds__(256) seqpr_stream_query_fold_kernel(SeqPrStreamArgs a, unsigned long long *acc_hist,
+                                                                      unsigned long long *gtp)
+{
+    stream_query_fold<false>(a, acc_hist, gtp, nullptr, nullptr, 0);
+}
+
+__global__ void __launch_bounds__(256) seqpr_stream_query_fold_ids_kernel(SeqPrStreamArgs a,
+                                                                          unsigned long long *acc_hist,
+                                                                          unsigned long long *gtp,
+                                                                          const int32_t *__restrict__ ids,
+                                                                          const int64_t *__restrict__ rows,
+                                                                          int n_fleet)
+{
+    stream_query_fold<true>(a, acc_hist, gtp, ids, rows, n_fleet);
 }
 
 // Place mode, finish: every record that saw a valid row is one column (k, hit at its first maximum); gtp counts the
@@ -1362,17 +1484,25 @@ extern "C" int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, in
     return 0;
 }
 
-extern "C" int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, int L, int N, float *ring, int32_t *seen,
-                                         int64_t t, float *top_val, int32_t *top_idx, void *stream)
+// Host side of both streaming matches.  kIdx = false: lens_seqmatch_topk_stream (B streams in lockstep, t rows each);
+// kIdx = true: lens_seqmatch_topk_stream_ids (B = the n pushing streams ids[0..n) of a fleet of n_fleet, rows[]).
+template <bool kIdx>
+static int stream_match(const char *fn, const float *S, int B, int Q, int P, int L, int N, const int32_t *ids,
+                        int n_fleet, float *ring, int32_t *seen, int64_t t, int64_t *rows, float *top_val,
+                        int32_t *top_idx, void *stream)
 {
-    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "lens_seqmatch_topk_stream: bad sizes");
-    LENS_CHECK_ARG(L >= 1 && L <= P, "lens_seqmatch_topk_stream: need 1 <= L <= P, got L=%d", L);
-    LENS_CHECK_ARG(N >= 1 && N <= kMaxTopN, "lens_seqmatch_topk_stream: N=%d outside [1, %d]", N, kMaxTopN);
-    LENS_CHECK_ARG(t >= 0, "lens_seqmatch_topk_stream: t must be >= 0");
-    LENS_CHECK_ARG(seen != nullptr, "lens_seqmatch_topk_stream: NULL seen");
-    LENS_CHECK_ARG(L == 1 || ring != nullptr, "lens_seqmatch_topk_stream: NULL ring needs L == 1, got L=%d", L);
-    LENS_CHECK_ARG(B == 0 || (S && top_val && top_idx), "lens_seqmatch_topk_stream: NULL buffer");
-    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "lens_seqmatch_topk_stream: too many (stream, row) pairs");
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "%s: bad sizes", fn);
+    LENS_CHECK_ARG(L >= 1 && L <= P, "%s: need 1 <= L <= P, got L=%d", fn, L);
+    LENS_CHECK_ARG(N >= 1 && N <= kMaxTopN, "%s: N=%d outside [1, %d]", fn, N, kMaxTopN);
+    LENS_CHECK_ARG(t >= 0, "%s: t must be >= 0", fn);
+    LENS_CHECK_ARG(seen != nullptr, "%s: NULL seen", fn);
+    LENS_CHECK_ARG(L == 1 || ring != nullptr, "%s: NULL ring needs L == 1, got L=%d", fn, L);
+    LENS_CHECK_ARG(B == 0 || (S && top_val && top_idx), "%s: NULL buffer", fn);
+    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "%s: too many (stream, row) pairs", fn);
+    if constexpr (kIdx) {
+        LENS_CHECK_ARG(n_fleet >= 0, "%s: bad fleet size %d", fn, n_fleet);
+        LENS_CHECK_ARG(B == 0 || (ids && rows), "%s: NULL ids / rows", fn);
+    }
     if (B == 0) return 0;
     cudaStream_t st = as_stream(stream);
     const long long n_queries = (long long)B * Q;
@@ -1381,16 +1511,24 @@ extern "C" int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, in
         long long blocks;
         plan_segments(n_queries, P - L + 1, N, n_seg, seg_len, blocks);
         if (n_seg == 1) {
-            seqmatch_topk_stream_warp_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(
-                S, ring, seen, t, n_queries, Q, P, L, N, 1, seg_len, top_val, top_idx);
+            if constexpr (kIdx)
+                seqmatch_topk_stream_ids_warp_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(
+                    S, ring, seen, ids, rows, n_fleet, n_queries, Q, P, L, N, 1, seg_len, top_val, top_idx);
+            else
+                seqmatch_topk_stream_warp_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(
+                    S, ring, seen, t, n_queries, Q, P, L, N, 1, seg_len, top_val, top_idx);
             LENS_LAUNCH_CHECK();
         } else {
             float *seg_val = nullptr;                      // stream-ordered scratch, as in lens_seqmatch_topk
             const size_t n_list = (size_t)n_queries * n_seg * N;
             LENS_CUDA(cudaMallocAsync(&seg_val, n_list * (sizeof(float) + sizeof(int32_t)), st));
             int32_t *seg_idx = reinterpret_cast<int32_t *>(seg_val + n_list);
-            seqmatch_topk_stream_warp_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(
-                S, ring, seen, t, n_queries, Q, P, L, N, n_seg, seg_len, seg_val, seg_idx);
+            if constexpr (kIdx)
+                seqmatch_topk_stream_ids_warp_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(
+                    S, ring, seen, ids, rows, n_fleet, n_queries, Q, P, L, N, n_seg, seg_len, seg_val, seg_idx);
+            else
+                seqmatch_topk_stream_warp_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(
+                    S, ring, seen, t, n_queries, Q, P, L, N, n_seg, seg_len, seg_val, seg_idx);
             LENS_LAUNCH_CHECK();
             topn_merge_kernel<<<(unsigned)ceil_div64(n_queries, 8), 256, 0, st>>>(seg_val, seg_idx, n_seg, n_queries, N,
                                                                                    top_val, top_idx);
@@ -1398,17 +1536,45 @@ extern "C" int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, in
             LENS_CUDA(cudaFreeAsync(seg_val, st));
         }
     } else {
-        seqmatch_topk_stream_kernel<<<(unsigned)n_queries, kMatchThreads, 0, st>>>(S, ring, seen, t, Q, P, L, N,
-                                                                                    top_val, top_idx);
+        if constexpr (kIdx)
+            seqmatch_topk_stream_kernel<true><<<(unsigned)n_queries, kMatchThreads, 0, st>>>(
+                S, ring, seen, 0, Q, P, L, N, top_val, top_idx, ids, rows, n_fleet);
+        else
+            seqmatch_topk_stream_kernel<false><<<(unsigned)n_queries, kMatchThreads, 0, st>>>(
+                S, ring, seen, t, Q, P, L, N, top_val, top_idx, nullptr, nullptr, 0);
         LENS_LAUNCH_CHECK();
     }
+    const long long sms = std::max(sm_count(), 1);
     if (L > 1) {
-        const long long rows = (long long)B * std::min(Q, L - 1);
-        const long long blocks = std::min<long long>(rows, (long long)std::max(sm_count(), 1) * 16);
-        ring_append_kernel<<<(unsigned)blocks, 256, 0, st>>>(S, B, Q, P, L, t, ring, seen);
+        const long long n_rows = (long long)B * std::min(Q, L - 1);
+        const long long blocks = std::min<long long>(n_rows, sms * 16);
+        if constexpr (kIdx)
+            ring_append_ids_kernel<<<(unsigned)blocks, 256, 0, st>>>(S, B, Q, P, L, ring, ids, rows, n_fleet);
+        else
+            ring_append_kernel<<<(unsigned)blocks, 256, 0, st>>>(S, B, Q, P, L, t, ring, seen);
+        LENS_LAUNCH_CHECK();
+    }
+    if constexpr (kIdx) {
+        stream_advance_kernel<<<(unsigned)std::min<long long>(ceil_div(B, 256), sms * 8), 256, 0, st>>>(
+            ids, B, n_fleet, Q, L, seen, rows);
         LENS_LAUNCH_CHECK();
     }
     return 0;
+}
+
+extern "C" int lens_seqmatch_topk_stream(const float *S, int B, int Q, int P, int L, int N, float *ring, int32_t *seen,
+                                         int64_t t, float *top_val, int32_t *top_idx, void *stream)
+{
+    return stream_match<false>("lens_seqmatch_topk_stream", S, B, Q, P, L, N, nullptr, B, ring, seen, t, nullptr,
+                               top_val, top_idx, stream);
+}
+
+extern "C" int lens_seqmatch_topk_stream_ids(const float *S, int n, int Q, int P, int L, int N, const int32_t *ids,
+                                             int B, float *ring, int32_t *seen, int64_t *rows, float *top_val,
+                                             int32_t *top_idx, void *stream)
+{
+    return stream_match<true>("lens_seqmatch_topk_stream_ids", S, n, Q, P, L, N, ids, B, ring, seen, 0, rows, top_val,
+                              top_idx, stream);
 }
 
 extern "C" int lens_recall(const int32_t *top_idx, int B, int Qo, int Po, int N,
@@ -1624,20 +1790,26 @@ extern "C" int lens_seqpr_stream_bytes(int B, int P, int L, int mode, int64_t *b
     return 0;
 }
 
-extern "C" int lens_seqpr_stream_accumulate(const float *S, int B, int Q, int P, int L, const float *ring,
-                                            const int32_t *seen, int64_t t, const int32_t *gt_center, int gt_tol,
-                                            void *acc_place, void *acc_query, void *acc_multi, void *stream)
+// Host side of both accumulates, kIdx as in stream_match (B = the pushing streams, n_fleet = the fleet's size).
+template <bool kIdx>
+static int stream_accumulate_launch(const char *fn, const float *S, int B, int Q, int P, int L, const int32_t *ids,
+                                    int n_fleet, const float *ring, const int32_t *seen, int64_t t,
+                                    const int64_t *rows, const int32_t *gt_center, int gt_tol, void *acc_place,
+                                    void *acc_query, void *acc_multi, void *stream)
 {
-    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "lens_seqpr_stream_accumulate: bad sizes");
-    LENS_CHECK_ARG(L >= 1 && L <= P, "lens_seqpr_stream_accumulate: need 1 <= L <= P, got L=%d", L);
-    LENS_CHECK_ARG(t >= 0 && gt_tol >= 0, "lens_seqpr_stream_accumulate: t and gt_tol must be >= 0");
-    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "lens_seqpr_stream_accumulate: too many (stream, row) pairs");
-    LENS_CHECK_ARG(B == 0 || (S && seen && gt_center), "lens_seqpr_stream_accumulate: NULL S / seen / gt_center");
-    LENS_CHECK_ARG(B == 0 || L == 1 || ring, "lens_seqpr_stream_accumulate: NULL ring needs L == 1, got L=%d", L);
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "%s: bad sizes", fn);
+    LENS_CHECK_ARG(L >= 1 && L <= P, "%s: need 1 <= L <= P, got L=%d", fn, L);
+    LENS_CHECK_ARG(t >= 0 && gt_tol >= 0, "%s: t and gt_tol must be >= 0", fn);
+    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "%s: too many (stream, row) pairs", fn);
+    LENS_CHECK_ARG(B == 0 || (S && seen && gt_center), "%s: NULL S / seen / gt_center", fn);
+    LENS_CHECK_ARG(B == 0 || L == 1 || ring, "%s: NULL ring needs L == 1, got L=%d", fn, L);
+    if constexpr (kIdx) {
+        LENS_CHECK_ARG(n_fleet >= 0, "%s: bad fleet size %d", fn, n_fleet);
+        LENS_CHECK_ARG(B == 0 || (ids && rows), "%s: NULL ids / rows", fn);
+    }
     void *accs[3] = {acc_place, acc_query, acc_multi};
     for (int m = 0; m < 3; ++m)
-        LENS_CHECK_ARG((reinterpret_cast<uintptr_t>(accs[m]) & 7) == 0,
-                       "lens_seqpr_stream_accumulate: accumulators must be 8-byte aligned");
+        LENS_CHECK_ARG((reinterpret_cast<uintptr_t>(accs[m]) & 7) == 0, "%s: accumulators must be 8-byte aligned", fn);
     if (B == 0 || !(acc_place || acc_query || acc_multi)) return 0;
     SeqPrStreamArgs a{};
     a.S = S; a.ring = ring; a.seen = seen; a.t = t;
@@ -1658,16 +1830,36 @@ extern "C" int lens_seqpr_stream_accumulate(const float *S, int B, int Q, int P,
     const long long items = (long long)B * ceil_div(a.Po, kPrTile);
     const unsigned blocks = (unsigned)std::min<long long>(ceil_div64(items, 8), sms * 16);
     const size_t smem = acc_multi ? 2 * kStreamShBins * sizeof(unsigned) : 0;
-    seqpr_stream_accumulate_kernel<<<blocks, 256, smem, st>>>(a);
+    if constexpr (kIdx) seqpr_stream_accumulate_ids_kernel<<<blocks, 256, smem, st>>>(a, ids, rows, n_fleet);
+    else seqpr_stream_accumulate_kernel<<<blocks, 256, smem, st>>>(a);
     LENS_LAUNCH_CHECK();
     if (acc_query) {
         unsigned long long *q = static_cast<unsigned long long *>(acc_query);
-        seqpr_stream_query_fold_kernel<<<(unsigned)std::min<long long>(ceil_div64((long long)B * Q, 256), sms * 8), 256,
-                                         0, st>>>(a, q + 2, q + 1);
+        const unsigned fold_blocks = (unsigned)std::min<long long>(ceil_div64((long long)B * Q, 256), sms * 8);
+        if constexpr (kIdx)
+            seqpr_stream_query_fold_ids_kernel<<<fold_blocks, 256, 0, st>>>(a, q + 2, q + 1, ids, rows, n_fleet);
+        else seqpr_stream_query_fold_kernel<<<fold_blocks, 256, 0, st>>>(a, q + 2, q + 1);
         LENS_LAUNCH_CHECK();
         LENS_CUDA(cudaFreeAsync(a.key, st));
     }
     return 0;
+}
+
+extern "C" int lens_seqpr_stream_accumulate(const float *S, int B, int Q, int P, int L, const float *ring,
+                                            const int32_t *seen, int64_t t, const int32_t *gt_center, int gt_tol,
+                                            void *acc_place, void *acc_query, void *acc_multi, void *stream)
+{
+    return stream_accumulate_launch<false>("lens_seqpr_stream_accumulate", S, B, Q, P, L, nullptr, B, ring, seen, t,
+                                           nullptr, gt_center, gt_tol, acc_place, acc_query, acc_multi, stream);
+}
+
+extern "C" int lens_seqpr_stream_accumulate_ids(const float *S, int n, int Q, int P, int L, const int32_t *ids, int B,
+                                                const float *ring, const int32_t *seen, const int64_t *rows,
+                                                const int32_t *gt_center, int gt_tol, void *acc_place,
+                                                void *acc_query, void *acc_multi, void *stream)
+{
+    return stream_accumulate_launch<true>("lens_seqpr_stream_accumulate_ids", S, n, Q, P, L, ids, B, ring, seen, 0,
+                                          rows, gt_center, gt_tol, acc_place, acc_query, acc_multi, stream);
 }
 
 extern "C" int lens_seqpr_stream_histogram(const void *acc, int B, int P, int L, int mode, uint64_t *hist,

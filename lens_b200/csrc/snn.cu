@@ -694,6 +694,33 @@ __global__ void __launch_bounds__(256) reset_streams_kernel(const uint8_t *__res
     }
 }
 
+// lens_snn_forward_streams: rows ids[i] of v0 / v1 / v2 <-> rows i of the workspace (kScatter: back to the state).
+// One CTA per (stream, layer) at a time, 16-byte copies when the rows allow them; ids outside [0, maxB) are skipped.
+template <bool kScatter>
+__global__ void __launch_bounds__(256) state_rows_kernel(const int32_t *__restrict__ ids, int n, int maxB, int I, int F,
+                                                         int P, float *__restrict__ v0, float *__restrict__ v1,
+                                                         float *__restrict__ v2, float *__restrict__ ws, int ws_cap)
+{
+    for (long long w = blockIdx.x; w < 3LL * n; w += gridDim.x) {
+        const int layer = (int)(w / n), i = (int)(w - (long long)layer * n);
+        const int b = ids[i];
+        if ((unsigned)b >= (unsigned)maxB) continue;                // block-uniform
+        const int len = layer == 0 ? I : layer == 1 ? F : P;
+        float *state = (layer == 0 ? v0 : layer == 1 ? v1 : v2) + (size_t)b * len;
+        float *work = ws + (layer == 0 ? 0 : layer == 1 ? (size_t)ws_cap * I : (size_t)ws_cap * (I + F)) +
+                      (size_t)i * len;
+        const float *src = kScatter ? work : state;
+        float *dst = kScatter ? state : work;
+        if ((len & 3) == 0 && ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0) {
+            const float4 *s4 = reinterpret_cast<const float4 *>(src);
+            float4 *d4 = reinterpret_cast<float4 *>(dst);
+            for (int k = threadIdx.x; k < len / 4; k += blockDim.x) d4[k] = s4[k];
+        } else {
+            for (int k = threadIdx.x; k < len; k += blockDim.x) dst[k] = src[k];
+        }
+    }
+}
+
 }  // namespace lens
 
 using namespace lens;
@@ -764,7 +791,7 @@ extern "C" int lens_snn_destroy(void *handle)
     snn_tc_release(h);
     cudaFree(h->Wf_fx); cudaFree(h->Wf_scale); cudaFree(h->Wo_fx); cudaFree(h->Wo_scale);
     cudaFree(h->U); cudaFree(h->Uq); cudaFree(h->v0); cudaFree(h->v1); cudaFree(h->v2);
-    cudaFree(h->counters); cudaFree(h->S1);
+    cudaFree(h->counters); cudaFree(h->S1); cudaFree(h->ws);
     delete h;
     return 0;
 }
@@ -843,6 +870,46 @@ extern "C" int lens_snn_forward_range(void *handle, const uint8_t *pooled, int b
     LENS_CHECK_ARG((int64_t)Q * h->T <= 2147483647LL, "lens_snn_forward_range: too many steps");
     return forward_common(h, pooled, nullptr, nb, Q * h->T, counts, nullptr, hidden_steps, out_steps, mode,
                           as_stream(stream), b0);
+}
+
+extern "C" int lens_snn_forward_streams(void *handle, const uint8_t *pooled, const int32_t *ids, int n, int Q,
+                                        float *counts, int mode, void *stream)
+{
+    LENS_CHECK_ARG(handle, "lens_snn_forward_streams: NULL handle");
+    SnnHandle *h = static_cast<SnnHandle *>(handle);
+    LENS_CHECK_ARG(h->U != nullptr, "lens_snn_forward_streams: handle was created without the raster matrix U");
+    LENS_CHECK_ARG(n >= 0 && Q >= 0, "lens_snn_forward_streams: bad sizes n=%d Q=%d", n, Q);
+    LENS_CHECK_ARG(mode >= LENS_SNN_AUTO && mode <= LENS_SNN_TC, "lens_snn_forward_streams: bad mode %d", mode);
+    if (n == 0 || Q == 0) return 0;
+    LENS_CHECK_ARG(pooled && ids && counts, "lens_snn_forward_streams: NULL buffer");
+    LENS_CHECK_ARG((int64_t)Q * h->T <= 2147483647LL, "lens_snn_forward_streams: too many steps");
+    cudaStream_t st = as_stream(stream);
+    const int need = n + (n & 1);                     // streams are tiled in pairs
+    if (need > h->ws_cap) {
+        if (h->ws) LENS_CUDA(cudaFree(h->ws));
+        h->ws = nullptr; h->ws_cap = 0;
+        const size_t bytes = (size_t)need * (h->I + h->F + h->P) * sizeof(float);
+        LENS_CUDA(cudaMalloc(&h->ws, bytes));
+        LENS_CUDA(cudaMemsetAsync(h->ws, 0, bytes, st));   // the pad row of an odd n is read as a stream's state
+        h->ws_cap = need;
+    }
+    const int blocks = (int)std::min<long long>(3LL * n, (long long)std::max(sm_count(), 1) * 16);
+    state_rows_kernel<false><<<blocks, 256, 0, st>>>(ids, n, h->maxB, h->I, h->F, h->P, h->v0, h->v1, h->v2, h->ws,
+                                                     h->ws_cap);
+    LENS_LAUNCH_CHECK();
+    // forward_common reads and writes the state through h->v0 / v1 / v2 (plain kernel parameters): point them at the
+    // workspace for the call
+    float *v[3] = {h->v0, h->v1, h->v2};
+    h->v0 = h->ws;
+    h->v1 = h->ws + (size_t)h->ws_cap * h->I;
+    h->v2 = h->ws + (size_t)h->ws_cap * (h->I + h->F);
+    const int rc = forward_common(h, pooled, nullptr, n, Q * h->T, counts, nullptr, nullptr, nullptr, mode, st);
+    h->v0 = v[0]; h->v1 = v[1]; h->v2 = v[2];
+    if (rc) return rc;                                // the state is left as it was
+    state_rows_kernel<true><<<blocks, 256, 0, st>>>(ids, n, h->maxB, h->I, h->F, h->P, h->v0, h->v1, h->v2, h->ws,
+                                                    h->ws_cap);
+    LENS_LAUNCH_CHECK();
+    return 0;
 }
 
 extern "C" int lens_snn_forward_float(void *handle, const float *x, int B, int steps,

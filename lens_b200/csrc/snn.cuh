@@ -69,6 +69,8 @@ struct SnnHandle {
     bool feature_smem_optin = false, output_smem_optin = false;  // CUDA-core kernels opted in to > 48 KB
     int8_t *S1 = nullptr;         // scratch hidden spikes [streams][steps][Fp]
     size_t S1_cap = 0;
+    float *ws = nullptr;          // lens_snn_forward_streams: v0 | v1 | v2 of the pushing streams, [ws_cap][I|F|P] each
+    int ws_cap = 0;
     // tensor-core operands (built lazily by snn_tc.cu)
     int8_t *Wo_planes = nullptr;  // [P_tiles][kPlanes][Fp/16][128][16] canonical UMMA layout
     int *Wo_npl = nullptr;        // [P_tiles] digit planes in use per place tile (5 or 6)

@@ -189,6 +189,22 @@ class B200Network:
                                                 None, None, int(mode), stream_ptr()), "lens_snn_forward_range")
         return counts
 
+    @_on_device
+    def run_streams_ids(self, pooled, ids, mode=MODE_AUTO):
+        """`run_streams` for the streams ids of the handle only, in any order: pooled u8 [n, Q, I] -> counts f32
+        [n, Q, P], row i = stream ids[i] (i32 [n] on the device, distinct, in [0, max_streams)).  Each of them
+        advances from its own state; every other stream's state is untouched, and the handle is never resized."""
+        require_cuda(pooled, ids)
+        if pooled.dtype != torch.uint8 or pooled.dim() != 3 or pooled.shape[2] != self.I:
+            raise LensError(f"pooled must be u8 [n, Q, {self.I}]")
+        n, Q, _ = pooled.shape
+        if ids.dtype != torch.int32 or tuple(ids.shape) != (n,):
+            raise LensError(f"ids must be i32 [{n}]")
+        counts = torch.empty((n, Q, self.P), dtype=torch.float32, device=pooled.device)
+        check(_lib.lib().lens_snn_forward_streams(self._h, ptr(pooled), ptr(ids), n, Q, ptr(counts), int(mode),
+                                                  stream_ptr()), "lens_snn_forward_streams")
+        return counts
+
     def ensure_streams(self, B):
         self._ensure_streams(B)
 

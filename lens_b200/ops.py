@@ -136,6 +136,26 @@ def seqmatch_topk_stream(S, L, N, ring, seen, t):
     return tv, ti
 
 
+def seqmatch_topk_stream_ids(S, L, N, ids, ring, seen, rows):
+    """seqmatch_topk_stream for any subset of a fleet of B streams, in any order: S f32 [n, Q, P] = the Q new rows of
+    the streams ids i32 [n] (device, distinct, in [0, B)) -> (top_val [n, Q, N], top_idx [n, Q, N]) by position.
+
+    ring f32 [B, L - 1, P] (None iff L == 1), seen i32 [B] and rows i64 [B] (rows pushed to each stream, which replaces
+    the scalar t) are the fleet's device state, updated in place for the pushed streams only.  See
+    lens_seqmatch_topk_stream_ids in include/lens_b200.h."""
+    require_cuda(S, ids, ring, seen, rows)
+    assert S.dtype == torch.float32 and S.dim() == 3 and seen.dtype == torch.int32 and rows.dtype == torch.int64
+    n, Q, P = S.shape
+    B = seen.shape[0]
+    assert ids.dtype == torch.int32 and ids.shape == (n,) and seen.shape == (B,) and rows.shape == (B,)
+    assert ring is None or (ring.dtype == torch.float32 and ring.shape == (B, L - 1, P))
+    tv = torch.empty((n, Q, N), dtype=torch.float32, device=S.device)
+    ti = torch.empty((n, Q, N), dtype=torch.int32, device=S.device)
+    check(_lib.lib().lens_seqmatch_topk_stream_ids(ptr(S), n, Q, P, L, N, ptr(ids), B, ptr(ring), ptr(seen), ptr(rows),
+                                                   ptr(tv), ptr(ti), stream_ptr()), "lens_seqmatch_topk_stream_ids")
+    return tv, ti
+
+
 def recall_counts(top_idx, Po, gt_dense=None, gt_center=None, gt_tol=0, ns=RECALL_NS,
                   hits=None, n_valid=None):
     """Accumulate Recall@N hit counters (device int64) for top_idx [B, Qo, N].
@@ -279,6 +299,38 @@ def seqpr_stream_accumulate(S, L, ring, seen, t, gt_center, gt_tol=0, acc_place=
     check(_lib.lib().lens_seqpr_stream_accumulate(ptr(S), B, Q, P, L, ptr(ring), ptr(seen), int(t), ptr(gt_center),
                                                   int(gt_tol), *(ptr(a) for a in accs), stream_ptr()),
           "lens_seqpr_stream_accumulate")
+
+
+def seqpr_stream_accumulate_ids(S, L, ids, ring, seen, rows, gt_center, gt_tol=0, acc_place=None, acc_query=None,
+                                acc_multi=None):
+    """seqpr_stream_accumulate for the push of seqmatch_topk_stream_ids: S f32 [n, Q, P] and gt_center i32 [n, Q] of the
+    streams ids i32 [n] of a fleet of B, with the ring / seen / rows that call is about to use; the accumulators are
+    the fleet's (seqpr_stream_bytes(B, ...))."""
+    accs = (acc_place, acc_query, acc_multi)
+    if not torch.is_tensor(seen) or seen.dtype != torch.int32 or seen.dim() != 1:
+        raise ValueError("seen must be i32 [B]")
+    B = seen.shape[0]
+    if not torch.is_tensor(S) or S.dtype != torch.float32 or S.dim() != 3:
+        raise ValueError("S must be f32 [n, Q, P]")
+    n, Q, P = S.shape
+    if not torch.is_tensor(ids) or ids.dtype != torch.int32 or tuple(ids.shape) != (n,):
+        raise ValueError(f"ids must be i32 [{n}]")
+    if not torch.is_tensor(rows) or rows.dtype != torch.int64 or tuple(rows.shape) != (B,):
+        raise ValueError(f"rows must be i64 [{B}]")
+    if not 1 <= L <= P:
+        raise ValueError(f"need 1 <= L <= P = {P}, got L={L}")
+    if L > 1 and (ring is None or ring.dtype != torch.float32 or tuple(ring.shape) != (B, L - 1, P)):
+        raise ValueError(f"ring must be f32 [{B}, {L - 1}, {P}]")
+    if not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32 or tuple(gt_center.shape) != (n, Q):
+        raise ValueError(f"gt_center must be i32 [{n}, {Q}]")
+    for mode, acc in enumerate(accs):
+        if acc is not None and (acc.dtype != torch.uint8 or acc.numel() != seqpr_stream_bytes(B, P, L, mode)):
+            raise ValueError(f"the {SEQPR_STREAM_MODES[mode]} accumulator must be u8 "
+                             f"[{seqpr_stream_bytes(B, P, L, mode)}] (seqpr_stream_bytes)")
+    require_cuda(S, ids, ring, seen, rows, gt_center, *accs)
+    check(_lib.lib().lens_seqpr_stream_accumulate_ids(ptr(S), n, Q, P, L, ptr(ids), B, ptr(ring), ptr(seen), ptr(rows),
+                                                      ptr(gt_center), int(gt_tol), *(ptr(a) for a in accs),
+                                                      stream_ptr()), "lens_seqpr_stream_accumulate_ids")
 
 
 def seqpr_stream_histogram(acc, B, P, L, mode, packed=None):

@@ -7,6 +7,7 @@ thousands: every stage is a call into liblens_b200.so; torch only owns the buffe
 GPU, no data-path collective) and the Recall@N counters are summed with one all-reduce
 (SURVEY.md 8e).
 """
+import numpy as np
 import torch
 
 from . import ops
@@ -236,16 +237,20 @@ class StreamingPipeline(InferencePipeline):
     """The hot path for live cameras: a fixed fleet of `n_streams` streams that deliver a few query windows at a
     time (one 250 ms timebin per push, typically), with sequence matching that spans the pushes.
 
-    Every push carries Q >= 1 new windows for each stream (all streams advance in lockstep).  Number a stream's
-    rows g = 0, 1, 2, ... since its last reset: new row g yields the top-N of the sequence that ends at it, once
-    the stream has seen L rows (g >= L - 1); earlier (warm-up) rows are -inf / -1.  However the windows are split
-    into pushes, the valid rows equal, bit for bit, the columns of one `step` over all of them (column g - L + 1).
+    A push carries Q >= 1 new windows for every stream (the fleet in lockstep), or for any subset of the streams in
+    any order (`push(..., streams=...)`: cameras that start late, deliver at their own rate or drop out for a while);
+    a stream outside a push keeps all of its state.  Number a stream's rows g = 0, 1, 2, ... since its last reset: new
+    row g yields the top-N of the sequence that ends at it, once the stream has seen L rows (g >= L - 1); earlier
+    (warm-up) rows are -inf / -1.  However a stream's windows are split into pushes, its valid rows equal, bit for
+    bit, the columns of one `step` over all of them (column g - L + 1).
 
     The object owns the device state that makes this work: the SNN membrane potentials (as any pipeline), `ring`
-    f32 [n_streams, L - 1, P] (the last L - 1 spike-count rows of every stream, row g at slot g mod (L - 1)),
-    `seen` i32 [n_streams] (rows since each stream's reset, saturating at L - 1) and `t` (rows pushed).  Under
-    torch.distributed every rank builds one for its own shard of streams; the Recall@N counters are all-reduced
-    like `step`'s.
+    f32 [n_streams, L - 1, P] (the last L - 1 spike-count rows of every stream, row g at slot g mod (L - 1), g counted
+    by `rows`), `seen` i32 [n_streams] (rows since each stream's reset, saturating at L - 1) and `rows` i64
+    [n_streams] (rows pushed to each stream since construction or `reset()`; `reset_streams` leaves it alone).  `t`
+    counts the rows pushed while the fleet moves in lockstep and equals every entry of `rows` until the first subset
+    push; from then on it no longer describes the session (use `rows`) until `reset()`.  Under torch.distributed
+    every rank builds one for its own shard of streams; the Recall@N counters are all-reduced like `step`'s.
 
     `track_pr` (any of "place", "query", "multi") also accumulates createPR's precision-recall curve of the session
     on the GPU, push by push, in bounded memory: see `session_precision_recall`.  The "place" accumulator holds
@@ -267,22 +272,53 @@ class StreamingPipeline(InferencePipeline):
                      if self.L > 1 else None)
         self.seen = torch.zeros((self.n_streams,), dtype=torch.int32, device=self.device)
         self.t = 0
+        # per-stream row counters: kept by the indexed kernels once a push has carried a subset of the streams (the
+        # session is then no longer lockstep); until then every stream has t rows and the lockstep kernels run
+        self._rows = torch.zeros((self.n_streams,), dtype=torch.int64, device=self.device)
+        self._indexed = False
+        self._all_ids = None
         # session accumulators of the tracked precision-recall modes (zeroed = empty session)
         self._pr_acc = {m: torch.zeros((ops.seqpr_stream_bytes(self.n_streams, self.net.P, self.L, i),),
                                        dtype=torch.uint8, device=self.device)
                         for i, m in enumerate(ops.SEQPR_STREAM_MODES) if m in track_pr}
 
+    @property
+    def rows(self):
+        """i64 [n_streams] on the device: rows pushed to each stream since construction or `reset()`."""
+        if not self._indexed:
+            self._rows.fill_(self.t)
+        return self._rows
+
     def _check_streams(self, B):
         if B != self.n_streams:
             raise LensError(f"this pipeline serves {self.n_streams} streams; the push has {B}")
 
-    def _check_gt(self, gt_center, Q, gt_tol):
-        if self._pr_acc and (gt_center is None or gt_tol < 0):
+    def _check_gt(self, gt_center, Q, gt_tol, n=None):
+        n = self.n_streams if n is None else n
+        if self._pr_acc and n and (gt_center is None or gt_tol < 0):
             raise LensError(f"precision-recall tracking ({', '.join(self._pr_acc)}) needs gt_center and gt_tol >= 0 "
                             "on every push")
         if gt_center is not None and (not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32
-                                      or tuple(gt_center.shape) != (self.n_streams, Q)):
-            raise LensError(f"gt_center must be i32 [{self.n_streams}, {Q}]")
+                                      or tuple(gt_center.shape) != (n, Q)):
+            raise LensError(f"gt_center must be i32 [{n}, {Q}]")
+
+    def _stream_indices(self, streams):
+        """A bool mask [n_streams] or integer stream indices (a host sequence, numpy array or tensor) -> list of int
+        indices in [0, n_streams): the indices in the order given, or the mask's True entries in ascending order."""
+        if isinstance(streams, np.ndarray):
+            streams = torch.from_numpy(streams)
+        is_tensor = torch.is_tensor(streams)
+        items = streams.reshape(-1).tolist() if is_tensor else list(streams)
+        if (streams.dtype == torch.bool) if is_tensor else (items and all(isinstance(v, bool) for v in items)):
+            if len(items) != self.n_streams:
+                raise LensError(f"a mask must have {self.n_streams} entries, got {len(items)}")
+            return [b for b, v in enumerate(items) if v]
+        if (is_tensor and (streams.dtype == torch.uint8 or streams.dtype.is_floating_point)) or \
+                any(isinstance(v, bool) or not isinstance(v, int) for v in items):
+            raise LensError("give a bool mask or integer stream indices (a u8 tensor is ambiguous)")
+        if any(v < 0 or v >= self.n_streams for v in items):
+            raise LensError(f"stream indices must lie in [0, {self.n_streams})")
+        return items
 
     def _offline(self, *args, **kwargs):
         # the batch entry points advance the SNN state without the sequence history (and a different stream count
@@ -297,25 +333,104 @@ class StreamingPipeline(InferencePipeline):
         raise LensError("StreamingPipeline is a live session: construct it with track_pr=(...) and call "
                         "session_precision_recall for the curve of the rows pushed so far")
 
-    def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True):
+    def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True, streams=None):
         """Q new windows of every stream: frames u8 [B, Q, roi, roi] or pooled u8 [B, Q, I], B = n_streams.
         -> `step`'s dict with top_val / top_idx [B, Q, N] (row q = the sequence ending at new row q), S [B, Q, P],
         and hits / n_valid for this push.  gt_center i32 [B, Q] (optional; required with track_pr) is the expected
         place of the sequence ending at each new row (band ground truth, |idx - center| <= gt_tol, -1 = none);
         warm-up rows never count.  With track_pr the valid new rows also join the precision-recall session; what
-        the push returns is the same as without tracking."""
+        the push returns is the same as without tracking.
+
+        `streams` (a bool mask [n_streams] or distinct integer indices, as a host sequence, numpy array or CPU
+        tensor, in any order, possibly empty) makes it a push of those streams only: row i of frames / pooled /
+        gt_center and of the results belongs to stream streams[i] (a mask: its True entries in ascending order), B =
+        their number.  Each of them advances exactly as in a lockstep push of that one stream; every other stream
+        keeps its SNN state, ring rows, seen, row counter and precision-recall records.  An empty push may omit
+        frames / pooled (and gt_center, also with track_pr) and launches no kernel of this library; under
+        torch.distributed with reduce=True, a rank with nothing to push calls it so that it takes part in the
+        all-reduce of the counters."""
         x = frames if frames is not None else pooled
-        if x is None or (frames is not None and pooled is not None):
+        if frames is not None and pooled is not None:
             raise LensError("give exactly one of frames / pooled")
-        self._check_streams(x.shape[0])
-        self._check_gt(gt_center, x.shape[1], gt_tol)
+        if streams is None:
+            if x is None:
+                raise LensError("give exactly one of frames / pooled")
+            self._check_streams(x.shape[0])
+            self._check_gt(gt_center, x.shape[1], gt_tol)
+            if self._indexed:
+                return self._push_ids(frames, pooled, None, gt_center, gt_tol, reduce)
+            with torch.cuda.device(self.device):
+                S = self.similarity(frames=frames, pooled=pooled)
+                if self._pr_acc:      # before the match, which advances seen and overwrites ring slots
+                    ops.seqpr_stream_accumulate(S, self.L, self.ring, self.seen, self.t, gt_center, gt_tol,
+                                                **{"acc_" + m: a for m, a in self._pr_acc.items()})
+                tv, ti = ops.seqmatch_topk_stream(S, self.L, self.n_top, self.ring, self.seen, self.t)
+                self.t += S.shape[1]
+            return self._finish(S, tv, ti, gt_center, gt_tol, reduce)
+        ids = self._stream_indices(streams)
+        if len(set(ids)) != len(ids):
+            raise LensError("a push names every stream at most once")
+        n = len(ids)
+        if x is None and n:
+            raise LensError("give exactly one of frames / pooled")
+        if x is not None and x.shape[0] != n:
+            raise LensError(f"the push names {n} streams but carries rows for {x.shape[0]}")
+        if n == 0:
+            return self._push_none(x.shape[1] if x is not None else None, gt_center, reduce)
+        self._check_gt(gt_center, x.shape[1], gt_tol, n)
+        net = self.net
+        want = (n, x.shape[1], net.I) if pooled is not None else (n, x.shape[1], net.roi, net.roi)
+        if not torch.is_tensor(x) or not x.is_cuda or x.dtype != torch.uint8 or tuple(x.shape) != want:
+            raise LensError(f"{'pooled' if pooled is not None else 'frames'} must be a u8 CUDA tensor {list(want)}")
+        return self._push_ids(frames, pooled, ids, gt_center, gt_tol, reduce)
+
+    def _push_ids(self, frames, pooled, ids, gt_center, gt_tol, reduce):
+        """The push on the indexed kernels: ids = the pushing streams (host list), None = all of them in order."""
         with torch.cuda.device(self.device):
-            S = self.similarity(frames=frames, pooled=pooled)
-            if self._pr_acc:      # before the match, which advances seen and overwrites ring slots
-                ops.seqpr_stream_accumulate(S, self.L, self.ring, self.seen, self.t, gt_center, gt_tol,
-                                            **{"acc_" + m: a for m, a in self._pr_acc.items()})
-            tv, ti = ops.seqmatch_topk_stream(S, self.L, self.n_top, self.ring, self.seen, self.t)
-            self.t += S.shape[1]
+            if not self._indexed:                  # the session leaves lockstep: every stream has t rows so far
+                self._rows.fill_(self.t)
+                self._indexed = True
+            if ids is None:
+                if self._all_ids is None:
+                    self._all_ids = torch.arange(self.n_streams, dtype=torch.int32, device=self.device)
+                dev_ids = self._all_ids
+                S = self.similarity(frames=frames, pooled=pooled)
+            else:
+                dev_ids = torch.tensor(ids, dtype=torch.int32).pin_memory().to(self.device, non_blocking=True)
+                if pooled is None:
+                    n, Q = frames.shape[:2]
+                    pooled = ops.pool_frames(frames.reshape(n * Q, self.net.roi, self.net.roi),
+                                             self.net.k).reshape(n, Q, self.net.I)
+                S = self.net.run_streams_ids(pooled, dev_ids, mode=self.mode)
+            if self._pr_acc:          # before the match, which advances seen / rows and overwrites ring slots
+                ops.seqpr_stream_accumulate_ids(S, self.L, dev_ids, self.ring, self.seen, self._rows, gt_center, gt_tol,
+                                                **{"acc_" + m: a for m, a in self._pr_acc.items()})
+            tv, ti = ops.seqmatch_topk_stream_ids(S, self.L, self.n_top, dev_ids, self.ring, self.seen, self._rows)
+        return self._finish(S, tv, ti, gt_center, gt_tol, reduce)
+
+    def _push_none(self, Q, gt_center, reduce):
+        """A push that carries no stream (Q windows each; None: as gt_center says, else 0): empty results, zero
+        counters when the other ranks count (gt_center given or precision-recall tracked)."""
+        if gt_center is not None and (not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32
+                                      or gt_center.dim() != 2 or gt_center.shape[0] != 0
+                                      or (Q is not None and gt_center.shape[1] != Q)):
+            raise LensError("gt_center of an empty push must be i32 [0, Q]")
+        if Q is None:
+            Q = gt_center.shape[1] if gt_center is not None else 0
+        dev = self.device
+        out = dict(top_val=torch.empty((0, Q, self.n_top), dtype=torch.float32, device=dev),
+                   top_idx=torch.empty((0, Q, self.n_top), dtype=torch.int32, device=dev), D=None, hits=None,
+                   n_valid=None, S=torch.empty((0, Q, self.net.P), dtype=torch.float32, device=dev),
+                   overflow=self.net.overflow_tensor())
+        if gt_center is not None or self._pr_acc:
+            out["hits"] = torch.zeros((len(self.ns),), dtype=torch.int64, device=dev)
+            out["n_valid"] = torch.zeros((1,), dtype=torch.int64, device=dev)
+        if reduce:
+            self._all_reduce_hits(out)
+        return out
+
+    def _finish(self, S, tv, ti, gt_center, gt_tol, reduce):
+        with torch.cuda.device(self.device):
             out = dict(top_val=tv, top_idx=ti, D=None, hits=None, n_valid=None, S=S,
                        overflow=self.net.overflow_tensor())
             if gt_center is not None:
@@ -327,47 +442,51 @@ class StreamingPipeline(InferencePipeline):
         return out
 
     def push_events(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0=0, roi_y0=0, gt_center=None, gt_tol=0,
-                    reduce=True):
+                    reduce=True, streams=None):
         """`push` fed from raw events: the next Q windows of every stream, window q of stream b covering
         [t0_us[b] + q * window_us, + window_us) of its events [offsets[b], offsets[b+1]) (as in `step_events`).
-        Returns `push`'s dict plus "events_per_window" i32 [B, Q]."""
-        self._check_streams(offsets.numel() - 1)
-        self._check_gt(gt_center, int(Q), gt_tol)
+        Returns `push`'s dict plus "events_per_window" i32 [B, Q].  With `streams` (as in `push`), offsets / t0_us
+        describe the pushing streams in that order, B = their number."""
+        if streams is None:
+            self._check_streams(offsets.numel() - 1)
+            self._check_gt(gt_center, int(Q), gt_tol)
+        else:
+            ids = self._stream_indices(streams)
+            if len(set(ids)) != len(ids):
+                raise LensError("a push names every stream at most once")
+            if offsets.numel() - 1 != len(ids):
+                raise LensError(f"the push names {len(ids)} streams but offsets describe {offsets.numel() - 1}")
+            if not ids:
+                out = self._push_none(int(Q), gt_center, reduce)
+                out["events_per_window"] = torch.empty((0, int(Q)), dtype=torch.int32, device=self.device)
+                return out
+            self._check_gt(gt_center, int(Q), gt_tol, len(ids))
+            streams = ids
         with torch.cuda.device(self.device):
             pooled, n_ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
-            out = self.push(pooled=pooled, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce)
+            out = self.push(pooled=pooled, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce, streams=streams)
         out["events_per_window"] = n_ev
         return out
 
     def reset_streams(self, streams):
         """Restart some streams (a camera that rebooted or dropped out): their SNN state and their sequence
         history.  `streams` is a bool mask [n_streams] (tensor or sequence of bools) or integer stream indices
-        (tensor or sequence).  Their next L - 1 rows are warm-up rows again; the other streams are untouched."""
-        is_tensor = torch.is_tensor(streams)
-        items = streams.reshape(-1).tolist() if is_tensor else list(streams)
-        if (streams.dtype == torch.bool) if is_tensor else (items and all(isinstance(v, bool) for v in items)):
-            if len(items) != self.n_streams:
-                raise LensError(f"a mask must have {self.n_streams} entries, got {len(items)}")
-            mask = torch.tensor(items, dtype=torch.bool)
-        else:
-            if (is_tensor and (streams.dtype == torch.uint8 or streams.dtype.is_floating_point)) or \
-                    any(isinstance(v, bool) or not isinstance(v, int) for v in items):
-                raise LensError("give a bool mask or integer stream indices (a u8 tensor is ambiguous)")
-            if any(v < 0 or v >= self.n_streams for v in items):
-                raise LensError(f"stream indices must lie in [0, {self.n_streams})")
-            mask = torch.zeros((self.n_streams,), dtype=torch.bool)
-            mask[torch.tensor(items, dtype=torch.int64)] = True
+        (tensor, numpy array or sequence).  Their next L - 1 rows are warm-up rows again; the other streams are
+        untouched.  Row counters (`rows`) are not reset."""
+        mask = torch.zeros((self.n_streams,), dtype=torch.bool)
+        mask[torch.tensor(self._stream_indices(streams), dtype=torch.int64)] = True
         with torch.cuda.device(self.device):
             mask = mask.to(self.device)
             self.net.reset_streams(mask)
             self.seen.masked_fill_(mask, 0)
 
     def reset(self):
-        """Every stream from scratch: SNN state (and the overflow counter), sequence history, t, and a new
-        precision-recall session."""
+        """Every stream from scratch: SNN state (and the overflow counter), sequence history, t and rows (the fleet is
+        in lockstep again), and a new precision-recall session."""
         self.net.reset_states()
         self.seen.zero_()
         self.t = 0
+        self._indexed = False
         self.reset_precision_recall()
 
     def reset_precision_recall(self):
