@@ -33,6 +33,8 @@
  *                          n * (I + F + P) * 4 bytes of handle-owned workspace (n rounded up to even), kept for the
  *                          largest n seen; ids outside [0, max_streams) are skipped, duplicates unspecified
  *   lens_recall / _bounds  at most 8 values of N per call
+ *   lens_seq_recall_bounds*
+ *                          at most 8 values of N, ascending, each >= 1; L and B * Q as the match of the same form
  *   lens_pr_counts         Qo <= 8192 (one CTA, shared-memory resident)
  *   lens_seqpr_scan / _counts
  *                          1 <= L <= min(Q, P), 2 <= n_thresh <= 4096 (table and histograms in 48 KB of shared memory)
@@ -283,6 +285,41 @@ int lens_topn_merge(const float *val, const int32_t *idx, int W, int64_t M, int 
  * D, GT [Po][Qo] (rows = database, the matrices recallAtK receives), ns host ints ascending.          */
 int lens_recall_bounds(const float *D, const uint8_t *GT, int Po, int Qo, const int *ns, int n_ns,
                        int64_t *lo, int64_t *hi, int64_t *n_valid, void *stream);
+
+/* The same bounds for whole fleets and live sessions, straight from the spike counts: D is recomputed exactly as
+ * lens_seqmatch_topk computes it (terms j = 0 .. L-1, one IEEE division) and never written, so the bounds bracket
+ * that kernel's own ranking (and lens_recall's hits) for any finite S.  In one column let vg be the largest D among
+ * its positives, A the places with D > vg and E the non-positive places with D == vg: a hit in the top K is possible
+ * iff A < K and certain iff A + E < K.  A column is read once after vg is known, and no further than the place
+ * where A reaches max(ns).
+ *   ns      [n_ns] host ints, ascending, each >= 1 (K > Po is allowed), 1 <= n_ns <= 8
+ *   lo, hi  [n_ns] i64 device, ACCUMULATED: columns that hit in the top ns[i] for every / for some order of ties
+ *   n_valid [1] i64 device, ACCUMULATED: the columns lens_recall counts for the same input
+ * Three launches per call, never more with the number of streams; stream-ordered scratch of 12 bytes per row.  No
+ * stream (B = 0, n = 0) returns 0 without launching.  Finite S only.
+ *
+ * lens_seq_recall_bounds: S [B][Q][P] f32 of B streams, 1 <= L <= min(Q, P), columns (b, q) for q < Qo = Q-L+1.
+ * Ground truth as lens_recall: gt_dense [B or 1][Po][Qo] u8 (gt_stream_stride = Po*Qo, or 0 to share one matrix;
+ * a column counts when it has a positive) or gt_center [B][Qo] i32 with gt_tol (positives |p - c| <= gt_tol; a
+ * column counts when c >= 0, even if its band lies outside [0, Po): it can then never hit), exactly one non-NULL.
+ *
+ * lens_seq_recall_bounds_stream: the new rows of one lens_seqmatch_topk_stream push (S, B, Q, P, L, ring, seen and
+ * t as for that call, which must come AFTER this one: it advances seen and overwrites ring slots).  A column is a
+ * valid new row (its stream has seen L rows) with gt_center [B][Q] >= 0; 1 <= L <= P, B * Q <= 2^31 - 1.
+ *
+ * lens_seq_recall_bounds_stream_ids: the same for the push of lens_seqmatch_topk_stream_ids (S, n, ids, B, ring,
+ * seen, rows as for that call, which must come AFTER this one); gt_center [n][Q] by position.  An id outside [0, B)
+ * is skipped.                                                                                                     */
+int lens_seq_recall_bounds(const float *S, int B, int Q, int P, int L, const uint8_t *gt_dense,
+                           int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, const int *ns, int n_ns,
+                           int64_t *lo, int64_t *hi, int64_t *n_valid, void *stream);
+int lens_seq_recall_bounds_stream(const float *S, int B, int Q, int P, int L, const float *ring, const int32_t *seen,
+                                  int64_t t, const int32_t *gt_center, int gt_tol, const int *ns, int n_ns, int64_t *lo,
+                                  int64_t *hi, int64_t *n_valid, void *stream);
+int lens_seq_recall_bounds_stream_ids(const float *S, int n, int Q, int P, int L, const int32_t *ids, int B,
+                                      const float *ring, const int32_t *seen, const int64_t *rows,
+                                      const int32_t *gt_center, int gt_tol, const int *ns, int n_ns, int64_t *lo,
+                                      int64_t *hi, int64_t *n_valid, void *stream);
 
 /* Precision-recall counters of lens/src/metrics.py:21-139 (createPR, matching='single'), used by
  * lens/run_model.py:319-327 with n_thresh = 100.  S and GT are [Po][Qo] (rows = database), exactly the

@@ -57,6 +57,11 @@ def _declare(L):
         "lens_pr_counts_multi": (i32, [vp, vp, i32, i32, i32, vp, vp, vp, vp, i32]),
         "lens_recall": (i32, [vp, i32, i32, i32, i32, vp, i64, vp, i32, pi32, i32, vp, vp, vp]),
         "lens_recall_bounds": (i32, [vp, vp, i32, i32, pi32, i32, vp, vp, vp, vp]),
+        "lens_seq_recall_bounds": (i32, [vp, i32, i32, i32, i32, vp, i64, vp, i32, pi32, i32, vp, vp, vp, vp]),
+        "lens_seq_recall_bounds_stream": (i32, [vp, i32, i32, i32, i32, vp, vp, i64, vp, i32, pi32, i32, vp, vp, vp,
+                                                vp]),
+        "lens_seq_recall_bounds_stream_ids": (i32, [vp, i32, i32, i32, i32, vp, i32, vp, vp, vp, vp, i32, pi32, i32, vp,
+                                                    vp, vp, vp]),
         "lens_topn_merge": (i32, [vp, vp, i32, i64, i32, vp, vp, vp]),
         "lens_seqpr_records_bytes": (i32, [i32, i32, i32, i32, i32, pi64]),
         "lens_seqpr_scan": (i32, [vp, i32, i32, i32, i32, i32, vp, i64, vp, i32, vp, vp, vp, vp]),

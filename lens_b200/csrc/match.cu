@@ -1288,6 +1288,209 @@ __global__ void __launch_bounds__(1024) seqpr_stream_bin_kernel(const unsigned l
     }
 }
 
+// ---- tie-aware Recall@N bounds straight from S (lens_seq_recall_bounds*) -------------------------------------------
+// The rule of recall_bounds_kernel without its level walk.  In one column (one sequence end of one stream) let vg be
+// the largest D among its positives, A the places with D > vg (none of them positive) and E the non-positive places
+// with D == vg.  Then for every K: a hit is possible iff A < K, and certain iff A + E < K.  So a column needs vg, then
+// one pass over its places counting two predicates, with D recomputed exactly as K4 computes it (terms j = 0 .. L - 1,
+// one __fdiv_rn); the bounds then bracket K4's own ranking for any finite S.  Once A >= max(ns) every K is a miss and
+// the pass stops; a place segment that stops there still adds >= max(ns) to the row's A, so the sum stays exact.
+// Three kernels per call, whatever the number of streams: peak (vg and validity per row), count (A, E, places split
+// into segments when rows are few), finish (per-K lo / hi / n_valid).  kStream / kIdx as in the streaming match:
+// batch (rows of S), lockstep streaming (StreamRows with t) and indexed streaming (fleet_stream<true>).
+constexpr unsigned kRbSkip = 0u;        // row key: not a column (warm-up row, skipped id, no positive in dense GT)
+constexpr unsigned kRbNoPositive = 1u;  // row key: a column whose band lies outside [0, Po): valid, never a hit
+                                        // (any finite vg has an orderable key above both)
+
+struct RecallBoundsArgs {
+    const float *S, *ring;
+    const int32_t *seen;
+    long long t;
+    const int32_t *ids;
+    const int64_t *rows;
+    int n_fleet;
+    int B, Q, P, L, Qr, Po;             // Qr: rows per stream, Qo (batch) or Q (streaming)
+    const uint8_t *gt_dense;            // [B or 1][Po][Qo] (batch only)
+    int64_t gt_stride;
+    const int32_t *gt_center;           // [B][Qr] by position
+    int gt_tol;
+    int ns[8];
+    int n_ns;
+    unsigned *key;                      // [B * Qr] orderable(vg), kRbSkip or kRbNoPositive
+    unsigned long long *ae;             // [B * Qr] A << 32 | E, summed over the row's place segments
+    unsigned long long *lo, *hi, *n_valid;
+};
+
+// The diagonal terms of batch row q of stream b: term j is row q + j of S.
+struct BatchRows {
+    const float *Sq;
+    size_t P;
+    __device__ __forceinline__ const float *row(int j) const { return Sq + (size_t)j * P; }
+};
+
+template <bool kStream>
+__device__ __forceinline__ auto rbounds_rows(const RecallBoundsArgs &a, int b, int fb, int q, long long tb)
+{
+    if constexpr (kStream) return StreamRows(a.S, a.ring, b, fb, a.Q, q, a.P, a.L, tb);
+    else return BatchRows{a.S + ((size_t)b * a.Q + q) * a.P, (size_t)a.P};
+}
+
+// Row g = b * Qr + q of the call -> (b, q, fleet stream fb, its row counter tb); false when g is not a sequence end.
+template <bool kStream, bool kIdx>
+__device__ __forceinline__ bool rbounds_row(const RecallBoundsArgs &a, int g, int &b, int &q, int &fb, long long &tb)
+{
+    b = g / a.Qr;
+    q = g - b * a.Qr;
+    if (!fleet_stream<kIdx>(a.ids, a.rows, a.n_fleet, b, a.t, fb, tb)) return false;
+    return !kStream || stream_row_valid(a.seen, fb, q, a.L);
+}
+
+__device__ __forceinline__ bool rbounds_positive(const RecallBoundsArgs &a, int b, int p, int q, int c)
+{
+    if (a.gt_dense) return __ldg(a.gt_dense + (size_t)b * a.gt_stride + (size_t)p * a.Qr + q) != 0;
+    return c >= 0 && abs(p - c) <= a.gt_tol;
+}
+
+// One warp per row: vg over the positives only (a band: at most 2 * tol + 1 places of L loads; dense GT: the lanes
+// walk the GT column and compute D at its positives), merged as order-preserving keys.
+template <bool kStream, bool kIdx>
+__global__ void __launch_bounds__(256, 1) rbounds_peak_kernel(RecallBoundsArgs a)
+{
+    const int lane = threadIdx.x & 31;
+    const int n = a.B * a.Qr;                                       // < 2^31 (checked on the host)
+    const float fl = (float)a.L;
+    const int warp0 = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
+    for (int g = warp0; g < n; g += n_warps) {
+        int b, q, fb;
+        long long tb;
+        unsigned key = kRbSkip;
+        if (rbounds_row<kStream, kIdx>(a, g, b, q, fb, tb)) {          // warp-uniform
+            const auto rr = rbounds_rows<kStream>(a, b, fb, q, tb);
+            int p0 = 0, p1 = a.Po, c = 0;
+            if (!a.gt_dense) {
+                c = __ldg(a.gt_center + g);
+                p0 = (int)max(0ll, (long long)c - a.gt_tol);
+                p1 = c >= 0 ? (int)min((long long)a.Po, (long long)c + a.gt_tol + 1) : 0;
+            }
+            unsigned best = 0u;
+            for (int p = p0 + lane; p < p1; p += 32) {
+                if (a.gt_dense && !rbounds_positive(a, b, p, q, c)) continue;
+                float acc = 0.0f;
+                for (int j = 0; j < a.L; ++j) acc += __ldg(rr.row(j) + (p + j));
+                best = max(best, f32_orderable(__fdiv_rn(acc, fl)));
+            }
+            best = __reduce_max_sync(0xffffffffu, best);
+            key = best ? best : (!a.gt_dense && c >= 0 ? kRbNoPositive : kRbSkip);
+        }
+        if (lane == 0) a.key[g] = key;
+    }
+}
+
+// One warp per (row, place segment), rows with a positive only: A and E over the segment's places with K4's coalesced
+// diagonal loads, kUnrollR batches of 32 places in flight; stops once the warp's A reaches max(ns).
+template <bool kStream, bool kIdx>
+__global__ void __launch_bounds__(256) rbounds_count_kernel(RecallBoundsArgs a, int kmax, int n_seg, int seg_len)
+{
+    const int lane = threadIdx.x & 31;
+    const float fl = (float)a.L;
+    const long long n_rows = (long long)a.B * a.Qr;
+    const long long warp0 = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+    const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
+    for (long long w = warp0; w < n_rows * n_seg; w += n_warps) {
+        const int seg = (int)(w / n_rows);
+        const int g = (int)(w - (long long)seg * n_rows);
+        const unsigned key = a.key[g];
+        if (key <= kRbNoPositive) continue;                                     // warp-uniform
+        const float vg = f32_from_orderable(key);
+        int b, q, fb;
+        long long tb;
+        rbounds_row<kStream, kIdx>(a, g, b, q, fb, tb);                         // true: the peak kernel found a positive
+        const auto rr = rbounds_rows<kStream>(a, b, fb, q, tb);
+        const int c = a.gt_dense ? 0 : __ldg(a.gt_center + g);
+        const int pe = min(a.Po, (seg + 1) * seg_len);
+        unsigned n_above = 0, n_tied = 0;                                        // per lane: A, E
+        for (int r0 = seg * seg_len; r0 < pe; r0 += 32 * kUnrollR) {
+            float acc[kUnrollR];
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) acc[u] = 0.0f;
+            if (r0 + 32 * kUnrollR <= pe) {
+                for (int j = 0; j < a.L; ++j) {
+                    const float *row = rr.row(j) + (r0 + lane + j);
+#pragma unroll
+                    for (int u = 0; u < kUnrollR; ++u) acc[u] += __ldg(row + 32 * u);
+                }
+            } else {
+                for (int j = 0; j < a.L; ++j) {
+                    const float *row = rr.row(j) + (r0 + lane + j);
+#pragma unroll
+                    for (int u = 0; u < kUnrollR; ++u)
+                        if (r0 + 32 * u + lane < pe) acc[u] += __ldg(row + 32 * u);
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < kUnrollR; ++u) {
+                const int p = r0 + 32 * u + lane;
+                if (p >= pe) continue;
+                const float d = __fdiv_rn(acc[u], fl);
+                n_above += d > vg;
+                if (d == vg && !rbounds_positive(a, b, p, q, c)) ++n_tied;
+            }
+            if (__reduce_add_sync(0xffffffffu, n_above) >= (unsigned)kmax) break;     // every K is a miss
+        }
+        n_above = __reduce_add_sync(0xffffffffu, n_above);
+        n_tied = __reduce_add_sync(0xffffffffu, n_tied);
+        if (lane == 0 && (n_above | n_tied))
+            atomicAdd(a.ae + g, (unsigned long long)n_above << 32 | n_tied);
+    }
+}
+
+// One thread per row: n_valid, and lo / hi per K, added to the caller's counters once per block.
+__global__ void __launch_bounds__(256) rbounds_finish_kernel(RecallBoundsArgs a)
+{
+    __shared__ unsigned s_lo[8], s_hi[8], s_valid;
+    if (threadIdx.x < 8) s_lo[threadIdx.x] = s_hi[threadIdx.x] = 0u;
+    if (threadIdx.x == 0) s_valid = 0u;
+    __syncthreads();
+    const int n = a.B * a.Qr;
+    unsigned lo[8], hi[8], valid = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) lo[i] = hi[i] = 0u;
+    for (int g = blockIdx.x * blockDim.x + threadIdx.x; g < n; g += gridDim.x * blockDim.x) {
+        const unsigned key = a.key[g];
+        if (key == kRbSkip) continue;
+        ++valid;
+        if (key == kRbNoPositive) continue;
+        const unsigned long long ae = a.ae[g];
+        const unsigned long long above = ae >> 32, tied = ae & 0xffffffffull;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            if (i >= a.n_ns) break;
+            hi[i] += above < (unsigned long long)a.ns[i];
+            lo[i] += above + tied < (unsigned long long)a.ns[i];
+        }
+    }
+    valid = __reduce_add_sync(0xffffffffu, valid);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        lo[i] = __reduce_add_sync(0xffffffffu, lo[i]);
+        hi[i] = __reduce_add_sync(0xffffffffu, hi[i]);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (valid) atomicAdd(&s_valid, valid);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            if (lo[i]) atomicAdd(&s_lo[i], lo[i]);
+            if (hi[i]) atomicAdd(&s_hi[i], hi[i]);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < a.n_ns) {
+        if (s_lo[threadIdx.x]) atomicAdd(a.lo + threadIdx.x, (unsigned long long)s_lo[threadIdx.x]);
+        if (s_hi[threadIdx.x]) atomicAdd(a.hi + threadIdx.x, (unsigned long long)s_hi[threadIdx.x]);
+    }
+    if (threadIdx.x == 0 && s_valid) atomicAdd(a.n_valid, (unsigned long long)s_valid);
+}
+
 // SAD baseline (lens/src/sad.py:38): one warp per (query, reference) pair, 16 pixels per lane-iteration
 // with byte-wise SIMD sum of absolute differences; integer accumulation (exact), stored as fp32.
 __global__ void __launch_bounds__(256) sad_kernel(const uint8_t *__restrict__ a, const uint8_t *__restrict__ b,
@@ -1909,4 +2112,122 @@ extern "C" int lens_seqpr_hist_counts(const uint64_t *hist, int L, int n_thresh,
     LENS_LAUNCH_CHECK();
     LENS_CUDA(cudaFreeAsync(binned, st));
     return 0;
+}
+
+// Place segments of the bounds count: as in plan_segments, few rows against many places (one camera, 100 000 places)
+// are split so that every SM gets warps.  Nothing is merged afterwards (the partial A, E of a row just add up), so a
+// segment may be as short as 1 024 places.
+static void plan_bounds_segments(long long n_rows, int Po, int &n_seg, int &seg_len, long long &blocks)
+{
+    const long long sms = std::max(sm_count(), 1), want_warps = sms * 32;
+    n_seg = 1;
+    if (n_rows < want_warps && Po >= 2048)
+        n_seg = (int)std::min<long long>(ceil_div64(want_warps, n_rows), Po / 1024);
+    n_seg = std::max(n_seg, 1);
+    seg_len = ceil_div(ceil_div(Po, n_seg), 32 * kUnrollR) * (32 * kUnrollR);
+    n_seg = ceil_div(Po, seg_len);
+    blocks = std::min<long long>(ceil_div64(n_rows * n_seg, 8), sms * 16);
+}
+
+// Host side of the three bounds calls, after each has checked its own arguments and filled a's inputs: checks ns and
+// the counters, then peak, count and finish on stream-ordered scratch of 12 bytes per row.
+template <bool kStream, bool kIdx>
+static int rbounds_launch(const char *fn, RecallBoundsArgs &a, const int *ns, int n_ns, int64_t *lo, int64_t *hi,
+                          int64_t *n_valid, void *stream)
+{
+    LENS_CHECK_ARG(ns && n_ns >= 1 && n_ns <= 8, "%s: n_ns must be in [1, 8]", fn);
+    for (int i = 0; i < 8; ++i) a.ns[i] = 0;
+    for (int i = 0; i < n_ns; ++i) {
+        LENS_CHECK_ARG(ns[i] >= 1 && (i == 0 || ns[i] > ns[i - 1]), "%s: ns must be ascending and >= 1", fn);
+        a.ns[i] = ns[i];
+    }
+    LENS_CHECK_ARG(lo && hi && n_valid, "%s: NULL lo / hi / n_valid", fn);
+    a.n_ns = n_ns;
+    a.lo = reinterpret_cast<unsigned long long *>(lo);
+    a.hi = reinterpret_cast<unsigned long long *>(hi);
+    a.n_valid = reinterpret_cast<unsigned long long *>(n_valid);
+    const long long n_rows = (long long)a.B * a.Qr;
+    if (n_rows == 0) return 0;
+    cudaStream_t st = as_stream(stream);
+    LENS_CUDA(cudaMallocAsync(&a.ae, (size_t)n_rows * (sizeof(unsigned long long) + sizeof(unsigned)), st));
+    a.key = reinterpret_cast<unsigned *>(a.ae + n_rows);
+    LENS_CUDA(cudaMemsetAsync(a.ae, 0, (size_t)n_rows * sizeof(unsigned long long), st));
+    const long long sms = std::max(sm_count(), 1);
+    const unsigned row_blocks = (unsigned)std::min<long long>(ceil_div64(n_rows, 256), sms * 8);
+    rbounds_peak_kernel<kStream, kIdx><<<(unsigned)std::min<long long>(ceil_div64(n_rows, 8), sms * 16), 256, 0, st>>>(a);
+    LENS_LAUNCH_CHECK();
+    int n_seg, seg_len;
+    long long blocks;
+    plan_bounds_segments(n_rows, a.Po, n_seg, seg_len, blocks);
+    rbounds_count_kernel<kStream, kIdx><<<(unsigned)blocks, 256, 0, st>>>(a, a.ns[n_ns - 1], n_seg, seg_len);
+    LENS_LAUNCH_CHECK();
+    rbounds_finish_kernel<<<row_blocks, 256, 0, st>>>(a);
+    LENS_LAUNCH_CHECK();
+    LENS_CUDA(cudaFreeAsync(a.ae, st));
+    return 0;
+}
+
+extern "C" int lens_seq_recall_bounds(const float *S, int B, int Q, int P, int L, const uint8_t *gt_dense,
+                                      int64_t gt_stream_stride, const int32_t *gt_center, int gt_tol, const int *ns,
+                                      int n_ns, int64_t *lo, int64_t *hi, int64_t *n_valid, void *stream)
+{
+    const char *fn = "lens_seq_recall_bounds";
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "%s: bad sizes", fn);
+    LENS_CHECK_ARG(L >= 1 && L <= Q && L <= P, "%s: need 1 <= L <= min(Q, P), got L=%d", fn, L);
+    LENS_CHECK_ARG((gt_dense != nullptr) != (gt_center != nullptr),
+                   "%s: exactly one of gt_dense / gt_center must be given", fn);
+    LENS_CHECK_ARG(gt_stream_stride >= 0 && gt_tol >= 0, "%s: gt_stream_stride and gt_tol must be >= 0", fn);
+    LENS_CHECK_ARG(B == 0 || S != nullptr, "%s: NULL S", fn);
+    LENS_CHECK_ARG((int64_t)B * (Q - L + 1) <= 2147483647LL, "%s: too many (stream, query) pairs", fn);
+    RecallBoundsArgs a{};
+    a.S = S; a.B = B; a.Q = Q; a.P = P; a.L = L; a.Qr = Q - L + 1; a.Po = P - L + 1;
+    a.gt_dense = gt_dense; a.gt_stride = gt_stream_stride; a.gt_center = gt_center; a.gt_tol = gt_tol;
+    return rbounds_launch<false, false>(fn, a, ns, n_ns, lo, hi, n_valid, stream);
+}
+
+// Checks shared by both streaming forms (B = the pushing streams, n_fleet = the fleet's size when kIdx).
+template <bool kIdx>
+static int rbounds_stream_args(RecallBoundsArgs &a, const char *fn, const float *S, int B, int Q, int P, int L,
+                               const int32_t *ids, int n_fleet, const float *ring, const int32_t *seen, int64_t t,
+                               const int64_t *rows, const int32_t *gt_center, int gt_tol)
+{
+    LENS_CHECK_ARG(B >= 0 && Q > 0 && P > 0, "%s: bad sizes", fn);
+    LENS_CHECK_ARG(L >= 1 && L <= P, "%s: need 1 <= L <= P, got L=%d", fn, L);
+    LENS_CHECK_ARG(t >= 0 && gt_tol >= 0, "%s: t and gt_tol must be >= 0", fn);
+    LENS_CHECK_ARG((int64_t)B * Q <= 2147483647LL, "%s: too many (stream, row) pairs", fn);
+    LENS_CHECK_ARG(B == 0 || (S && seen && gt_center), "%s: NULL S / seen / gt_center", fn);
+    LENS_CHECK_ARG(B == 0 || L == 1 || ring, "%s: NULL ring needs L == 1, got L=%d", fn, L);
+    if constexpr (kIdx) {
+        LENS_CHECK_ARG(n_fleet >= 0, "%s: bad fleet size %d", fn, n_fleet);
+        LENS_CHECK_ARG(B == 0 || (ids && rows), "%s: NULL ids / rows", fn);
+    }
+    a = RecallBoundsArgs{};
+    a.S = S; a.ring = ring; a.seen = seen; a.t = t; a.ids = ids; a.rows = rows; a.n_fleet = n_fleet;
+    a.B = B; a.Q = Q; a.P = P; a.L = L; a.Qr = Q; a.Po = P - L + 1;
+    a.gt_center = gt_center; a.gt_tol = gt_tol;
+    return 0;
+}
+
+extern "C" int lens_seq_recall_bounds_stream(const float *S, int B, int Q, int P, int L, const float *ring,
+                                             const int32_t *seen, int64_t t, const int32_t *gt_center, int gt_tol,
+                                             const int *ns, int n_ns, int64_t *lo, int64_t *hi, int64_t *n_valid,
+                                             void *stream)
+{
+    const char *fn = "lens_seq_recall_bounds_stream";
+    RecallBoundsArgs a;
+    if (int rc = rbounds_stream_args<false>(a, fn, S, B, Q, P, L, nullptr, B, ring, seen, t, nullptr, gt_center, gt_tol))
+        return rc;
+    return rbounds_launch<true, false>(fn, a, ns, n_ns, lo, hi, n_valid, stream);
+}
+
+extern "C" int lens_seq_recall_bounds_stream_ids(const float *S, int n, int Q, int P, int L, const int32_t *ids, int B,
+                                                 const float *ring, const int32_t *seen, const int64_t *rows,
+                                                 const int32_t *gt_center, int gt_tol, const int *ns, int n_ns,
+                                                 int64_t *lo, int64_t *hi, int64_t *n_valid, void *stream)
+{
+    const char *fn = "lens_seq_recall_bounds_stream_ids";
+    RecallBoundsArgs a;
+    if (int rc = rbounds_stream_args<true>(a, fn, S, n, Q, P, L, ids, B, ring, seen, 0, rows, gt_center, gt_tol))
+        return rc;
+    return rbounds_launch<true, true>(fn, a, ns, n_ns, lo, hi, n_valid, stream);
 }

@@ -399,6 +399,81 @@ def recall_bounds(D, gt_dense, ns=RECALL_NS):
     return lo, hi, n_valid
 
 
+def _bounds_counters(ns, device, lo, hi, n_valid):
+    """ns checks of the seq_recall_bounds calls and their (possibly given) i64 counters."""
+    ns = tuple(int(k) for k in ns)
+    if not 1 <= len(ns) <= 8 or ns[0] < 1 or any(b <= a for a, b in zip(ns, ns[1:])):
+        raise ValueError(f"ns must be 1 to 8 ascending values >= 1, got {ns}")
+    for name, t, n in (("lo", lo, len(ns)), ("hi", hi, len(ns)), ("n_valid", n_valid, 1)):
+        if t is not None and (not torch.is_tensor(t) or t.dtype != torch.int64 or tuple(t.shape) != (n,)):
+            raise ValueError(f"{name} must be i64 [{n}]")
+    zeros = (lambda n: torch.zeros((n,), dtype=torch.int64, device=device))
+    return ((C.c_int * len(ns))(*ns), len(ns), lo if lo is not None else zeros(len(ns)),
+            hi if hi is not None else zeros(len(ns)), n_valid if n_valid is not None else zeros(1))
+
+
+def seq_recall_bounds(S, L, gt_dense=None, gt_center=None, gt_tol=0, ns=RECALL_NS, lo=None, hi=None, n_valid=None):
+    """Tie-aware Recall@N bounds of a fleet straight from its spike counts S f32 [B, Q, P] (lens_seq_recall_bounds):
+    the sequence-matched matrices are recomputed as seqmatch_topk computes them, never stored.  Ground truth as in
+    `recall_counts`.  -> (lo [len(ns)], hi [len(ns)], n_valid [1]) i64 on the device, accumulated when given:
+    lo <= the hits of seqmatch_topk + recall_counts (and of any other order of equal similarities) <= hi, and n_valid
+    is recall_counts' own."""
+    B, Q, P, stride = _seqpr_check(S, L, SEQPR_MODES[("single", "place")], gt_dense, gt_center)
+    if gt_tol < 0:
+        raise ValueError(f"gt_tol must be >= 0, got {gt_tol}")
+    ns_arr, n_ns, lo, hi, n_valid = _bounds_counters(ns, S.device, lo, hi, n_valid)
+    require_cuda(S, gt_dense, gt_center, lo, hi, n_valid)
+    check(_lib.lib().lens_seq_recall_bounds(ptr(S), B, Q, P, L, ptr(gt_dense), stride, ptr(gt_center), int(gt_tol),
+                                            ns_arr, n_ns, ptr(lo), ptr(hi), ptr(n_valid), stream_ptr()),
+          "lens_seq_recall_bounds")
+    return lo, hi, n_valid
+
+
+def seq_recall_bounds_stream(S, L, ring, seen, t, gt_center, gt_tol=0, ns=RECALL_NS, lo=None, hi=None, n_valid=None):
+    """seq_recall_bounds over the valid new rows of one lockstep push: S f32 [B, Q, P] with the ring / seen / t that
+    the push's seqmatch_topk_stream call is about to use (so this comes first), gt_center i32 [B, Q] (-1 = none).
+    -> (lo, hi, n_valid) as seq_recall_bounds; n_valid equals what recall_counts gives for the push."""
+    B, Q, P = _seqpr_stream_check(S, L, ring, seen, gt_center, ())
+    if gt_tol < 0 or t < 0:
+        raise ValueError("gt_tol and t must be >= 0")
+    ns_arr, n_ns, lo, hi, n_valid = _bounds_counters(ns, S.device, lo, hi, n_valid)
+    require_cuda(S, ring, seen, gt_center, lo, hi, n_valid)
+    check(_lib.lib().lens_seq_recall_bounds_stream(ptr(S), B, Q, P, L, ptr(ring), ptr(seen), int(t), ptr(gt_center),
+                                                   int(gt_tol), ns_arr, n_ns, ptr(lo), ptr(hi), ptr(n_valid),
+                                                   stream_ptr()), "lens_seq_recall_bounds_stream")
+    return lo, hi, n_valid
+
+
+def seq_recall_bounds_stream_ids(S, L, ids, ring, seen, rows, gt_center, gt_tol=0, ns=RECALL_NS, lo=None, hi=None,
+                                 n_valid=None):
+    """seq_recall_bounds_stream for the push of seqmatch_topk_stream_ids: S f32 [n, Q, P] and gt_center i32 [n, Q] of
+    the streams ids i32 [n] of a fleet of B, with the ring / seen / rows that call is about to use."""
+    if not torch.is_tensor(seen) or seen.dtype != torch.int32 or seen.dim() != 1:
+        raise ValueError("seen must be i32 [B]")
+    B = seen.shape[0]
+    if not torch.is_tensor(S) or S.dtype != torch.float32 or S.dim() != 3:
+        raise ValueError("S must be f32 [n, Q, P]")
+    n, Q, P = S.shape
+    if not torch.is_tensor(ids) or ids.dtype != torch.int32 or tuple(ids.shape) != (n,):
+        raise ValueError(f"ids must be i32 [{n}]")
+    if not torch.is_tensor(rows) or rows.dtype != torch.int64 or tuple(rows.shape) != (B,):
+        raise ValueError(f"rows must be i64 [{B}]")
+    if not 1 <= L <= P:
+        raise ValueError(f"need 1 <= L <= P = {P}, got L={L}")
+    if L > 1 and (ring is None or ring.dtype != torch.float32 or tuple(ring.shape) != (B, L - 1, P)):
+        raise ValueError(f"ring must be f32 [{B}, {L - 1}, {P}]")
+    if not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32 or tuple(gt_center.shape) != (n, Q):
+        raise ValueError(f"gt_center must be i32 [{n}, {Q}]")
+    if gt_tol < 0:
+        raise ValueError(f"gt_tol must be >= 0, got {gt_tol}")
+    ns_arr, n_ns, lo, hi, n_valid = _bounds_counters(ns, S.device, lo, hi, n_valid)
+    require_cuda(S, ids, ring, seen, rows, gt_center, lo, hi, n_valid)
+    check(_lib.lib().lens_seq_recall_bounds_stream_ids(ptr(S), n, Q, P, L, ptr(ids), B, ptr(ring), ptr(seen), ptr(rows),
+                                                       ptr(gt_center), int(gt_tol), ns_arr, n_ns, ptr(lo), ptr(hi),
+                                                       ptr(n_valid), stream_ptr()), "lens_seq_recall_bounds_stream_ids")
+    return lo, hi, n_valid
+
+
 def sad_matrix(query_frames, reference_frames):
     """u8 [Q, npix], u8 [R, npix] -> L1 distances f32 [Q, R] (torch.cdist(a, b, 1) of lens/src/sad.py:38)."""
     require_cuda(query_frames, reference_frames)

@@ -46,18 +46,28 @@ class InferencePipeline:
         """u8 frames [B, Q, roi, roi] (or pooled [B, Q, I]) -> spike counts f32 [B, Q, P]."""
         return self.net.run_streams(frames=frames, pooled=pooled, mode=self.mode)
 
-    def match(self, S, gt_dense=None, gt_center=None, gt_tol=0, want_D=False):
-        """S [B, Q, P] -> dict(top_val, top_idx, D, hits, n_valid); hits are per-rank counters."""
+    def match(self, S, gt_dense=None, gt_center=None, gt_tol=0, want_D=False, bounds=False):
+        """S [B, Q, P] -> dict(top_val, top_idx, D, hits, n_valid); hits are per-rank counters.
+
+        bounds=True (with ground truth) adds hits_lo / hits_hi i64 [len(ns)]: the tie-aware bounds of the hits over
+        every order of equal similarities (the reference ranks with numpy's unstable argsort, so its own Recall@N is
+        defined only up to that order), computed straight from S (ops.seq_recall_bounds): hits_lo <= hits <=
+        hits_hi."""
         tv, ti, D = ops.seqmatch_topk(S, self.L, self.n_top, want_D=want_D)
         out = dict(top_val=tv, top_idx=ti, D=D, hits=None, n_valid=None)
         if gt_dense is not None or gt_center is not None:
             Po = S.shape[2] - self.L + 1
             out["hits"], out["n_valid"] = ops.recall_counts(ti, Po, gt_dense=gt_dense,
                                                             gt_center=gt_center, gt_tol=gt_tol, ns=self.ns)
+            if bounds:
+                out["hits_lo"], out["hits_hi"], _ = ops.seq_recall_bounds(S, self.L, gt_dense=gt_dense,
+                                                                          gt_center=gt_center, gt_tol=gt_tol,
+                                                                          ns=self.ns)
         return out
 
-    def step(self, frames=None, pooled=None, gt_dense=None, gt_center=None, gt_tol=0, reduce=True):
-        """One pass of the hot path over this rank's shard; Recall counters all-reduced if distributed."""
+    def step(self, frames=None, pooled=None, gt_dense=None, gt_center=None, gt_tol=0, reduce=True, bounds=False):
+        """One pass of the hot path over this rank's shard; Recall counters all-reduced if distributed.  bounds=True
+        adds the tie-aware hits_lo / hits_hi (see `match`)."""
         ev = None
         if self.stage_timing:
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
@@ -65,7 +75,7 @@ class InferencePipeline:
         S = self.similarity(frames=frames, pooled=pooled)
         if ev:
             ev[1].record()
-        out = self.match(S, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol)
+        out = self.match(S, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol, bounds=bounds)
         if ev:
             ev[2].record()
             self._stage_events.append(ev)
@@ -79,9 +89,13 @@ class InferencePipeline:
     def _all_reduce_hits(out):
         if out["hits"] is not None and torch.distributed.is_available() \
                 and torch.distributed.is_initialized() and torch.distributed.get_world_size() > 1:
-            packed = torch.cat([out["hits"], out["n_valid"]])
-            torch.distributed.all_reduce(packed)          # sum of 6 hit counters + valid count
-            out["hits"], out["n_valid"] = packed[:-1], packed[-1:]
+            keys = ["hits"] + [k for k in ("hits_lo", "hits_hi") if k in out]
+            packed = torch.cat([out[k] for k in keys] + [out["n_valid"]])
+            torch.distributed.all_reduce(packed)          # sum of the hit counters (and bounds) + valid count
+            n = out["hits"].numel()
+            for i, k in enumerate(keys):
+                out[k] = packed[i * n:(i + 1) * n]
+            out["n_valid"] = packed[-1:]
 
     def _bin_streams(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0):
         net = self.net
@@ -90,7 +104,7 @@ class InferencePipeline:
         return pooled, n_ev
 
     def step_events(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0=0, roi_y0=0, gt_dense=None,
-                    gt_center=None, gt_tol=0, reduce=True):
+                    gt_center=None, gt_tol=0, reduce=True, bounds=False):
         """The step fed from raw event streams: stream b is events [offsets[b], offsets[b+1]) of the device
         arrays t_us / x / y, and query q of stream b is its window [t0_us[b] + q * window_us, + window_us)
         (see ops.bin_event_streams).  The events are binned straight to pooled pixels (no frames are
@@ -102,12 +116,13 @@ class InferencePipeline:
         (collect_data.frames_from_events is the single-stream path that reproduces that)."""
         with torch.cuda.device(self.device):
             pooled, n_ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
-            out = self.step(pooled=pooled, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce)
+            out = self.step(pooled=pooled, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce,
+                            bounds=bounds)
         out["events_per_window"] = n_ev
         return out
 
     def step_event_groups(self, groups, B, Q, window_us, roi_x0=0, roi_y0=0, gt_dense=None, gt_center=None,
-                          gt_tol=0, reduce=True):
+                          gt_tol=0, reduce=True, bounds=False):
         """`step_events` for fleets whose events do not fit in device memory together.
 
         `groups` yields (b0, t_us, x, y, offsets, t0_us) for consecutive ranges of streams that cover
@@ -135,7 +150,7 @@ class InferencePipeline:
                 b_next = b0 + nb
             if b_next != B:
                 raise LensError(f"event groups cover streams [0, {b_next}) of {B}")
-            out = self.match(S, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol)
+            out = self.match(S, gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol, bounds=bounds)
             out["S"] = S
             out["overflow"] = net.overflow_tensor()
         out["events_per_window"] = n_ev
@@ -143,7 +158,8 @@ class InferencePipeline:
             self._all_reduce_hits(out)
         return out
 
-    def step_host(self, frames_host, gt_dense=None, gt_center=None, gt_tol=0, next_frames=None, reduce=True):
+    def step_host(self, frames_host, gt_dense=None, gt_center=None, gt_tol=0, next_frames=None, reduce=True,
+                  bounds=False):
         """The same step fed from PINNED HOST frames u8 [B, Q, roi, roi].
 
         The host->device copy runs on a side stream into one of two staging buffers.  Passing the
@@ -178,7 +194,7 @@ class InferencePipeline:
         slot, ev = self._pending.pop(frames_host.data_ptr())
         main.wait_event(ev)
         out = self.step(frames=self._stage[slot], gt_dense=gt_dense, gt_center=gt_center, gt_tol=gt_tol,
-                        reduce=reduce)
+                        reduce=reduce, bounds=bounds)
         self._stage_free[slot] = torch.cuda.Event()
         self._stage_free[slot].record(main)
         if next_frames is not None:
@@ -333,7 +349,7 @@ class StreamingPipeline(InferencePipeline):
         raise LensError("StreamingPipeline is a live session: construct it with track_pr=(...) and call "
                         "session_precision_recall for the curve of the rows pushed so far")
 
-    def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True, streams=None):
+    def push(self, frames=None, pooled=None, gt_center=None, gt_tol=0, reduce=True, streams=None, bounds=False):
         """Q new windows of every stream: frames u8 [B, Q, roi, roi] or pooled u8 [B, Q, I], B = n_streams.
         -> `step`'s dict with top_val / top_idx [B, Q, N] (row q = the sequence ending at new row q), S [B, Q, P],
         and hits / n_valid for this push.  gt_center i32 [B, Q] (optional; required with track_pr) is the expected
@@ -348,7 +364,11 @@ class StreamingPipeline(InferencePipeline):
         keeps its SNN state, ring rows, seen, row counter and precision-recall records.  An empty push may omit
         frames / pooled (and gt_center, also with track_pr) and launches no kernel of this library; under
         torch.distributed with reduce=True, a rank with nothing to push calls it so that it takes part in the
-        all-reduce of the counters."""
+        all-reduce of the counters.
+
+        bounds=True (with gt_center) adds hits_lo / hits_hi i64 [len(ns)]: the tie-aware bounds of this push's hits
+        over every order of equal similarities (see InferencePipeline.match), from S and the sequence history;
+        an empty push returns zeros for them."""
         x = frames if frames is not None else pooled
         if frames is not None and pooled is not None:
             raise LensError("give exactly one of frames / pooled")
@@ -358,15 +378,19 @@ class StreamingPipeline(InferencePipeline):
             self._check_streams(x.shape[0])
             self._check_gt(gt_center, x.shape[1], gt_tol)
             if self._indexed:
-                return self._push_ids(frames, pooled, None, gt_center, gt_tol, reduce)
+                return self._push_ids(frames, pooled, None, gt_center, gt_tol, reduce, bounds)
             with torch.cuda.device(self.device):
                 S = self.similarity(frames=frames, pooled=pooled)
                 if self._pr_acc:      # before the match, which advances seen and overwrites ring slots
                     ops.seqpr_stream_accumulate(S, self.L, self.ring, self.seen, self.t, gt_center, gt_tol,
                                                 **{"acc_" + m: a for m, a in self._pr_acc.items()})
+                lohi = None
+                if bounds and gt_center is not None:     # before the match, too
+                    lohi = ops.seq_recall_bounds_stream(S, self.L, self.ring, self.seen, self.t, gt_center, gt_tol,
+                                                        ns=self.ns)[:2]
                 tv, ti = ops.seqmatch_topk_stream(S, self.L, self.n_top, self.ring, self.seen, self.t)
                 self.t += S.shape[1]
-            return self._finish(S, tv, ti, gt_center, gt_tol, reduce)
+            return self._finish(S, tv, ti, gt_center, gt_tol, reduce, lohi)
         ids = self._stream_indices(streams)
         if len(set(ids)) != len(ids):
             raise LensError("a push names every stream at most once")
@@ -376,15 +400,15 @@ class StreamingPipeline(InferencePipeline):
         if x is not None and x.shape[0] != n:
             raise LensError(f"the push names {n} streams but carries rows for {x.shape[0]}")
         if n == 0:
-            return self._push_none(x.shape[1] if x is not None else None, gt_center, reduce)
+            return self._push_none(x.shape[1] if x is not None else None, gt_center, reduce, bounds)
         self._check_gt(gt_center, x.shape[1], gt_tol, n)
         net = self.net
         want = (n, x.shape[1], net.I) if pooled is not None else (n, x.shape[1], net.roi, net.roi)
         if not torch.is_tensor(x) or not x.is_cuda or x.dtype != torch.uint8 or tuple(x.shape) != want:
             raise LensError(f"{'pooled' if pooled is not None else 'frames'} must be a u8 CUDA tensor {list(want)}")
-        return self._push_ids(frames, pooled, ids, gt_center, gt_tol, reduce)
+        return self._push_ids(frames, pooled, ids, gt_center, gt_tol, reduce, bounds)
 
-    def _push_ids(self, frames, pooled, ids, gt_center, gt_tol, reduce):
+    def _push_ids(self, frames, pooled, ids, gt_center, gt_tol, reduce, bounds=False):
         """The push on the indexed kernels: ids = the pushing streams (host list), None = all of them in order."""
         with torch.cuda.device(self.device):
             if not self._indexed:                  # the session leaves lockstep: every stream has t rows so far
@@ -405,10 +429,14 @@ class StreamingPipeline(InferencePipeline):
             if self._pr_acc:          # before the match, which advances seen / rows and overwrites ring slots
                 ops.seqpr_stream_accumulate_ids(S, self.L, dev_ids, self.ring, self.seen, self._rows, gt_center, gt_tol,
                                                 **{"acc_" + m: a for m, a in self._pr_acc.items()})
+            lohi = None
+            if bounds and gt_center is not None:         # before the match, too
+                lohi = ops.seq_recall_bounds_stream_ids(S, self.L, dev_ids, self.ring, self.seen, self._rows, gt_center,
+                                                        gt_tol, ns=self.ns)[:2]
             tv, ti = ops.seqmatch_topk_stream_ids(S, self.L, self.n_top, dev_ids, self.ring, self.seen, self._rows)
-        return self._finish(S, tv, ti, gt_center, gt_tol, reduce)
+        return self._finish(S, tv, ti, gt_center, gt_tol, reduce, lohi)
 
-    def _push_none(self, Q, gt_center, reduce):
+    def _push_none(self, Q, gt_center, reduce, bounds=False):
         """A push that carries no stream (Q windows each; None: as gt_center says, else 0): empty results, zero
         counters when the other ranks count (gt_center given or precision-recall tracked)."""
         if gt_center is not None and (not torch.is_tensor(gt_center) or gt_center.dtype != torch.int32
@@ -425,11 +453,14 @@ class StreamingPipeline(InferencePipeline):
         if gt_center is not None or self._pr_acc:
             out["hits"] = torch.zeros((len(self.ns),), dtype=torch.int64, device=dev)
             out["n_valid"] = torch.zeros((1,), dtype=torch.int64, device=dev)
+            if bounds:
+                out["hits_lo"] = torch.zeros((len(self.ns),), dtype=torch.int64, device=dev)
+                out["hits_hi"] = torch.zeros((len(self.ns),), dtype=torch.int64, device=dev)
         if reduce:
             self._all_reduce_hits(out)
         return out
 
-    def _finish(self, S, tv, ti, gt_center, gt_tol, reduce):
+    def _finish(self, S, tv, ti, gt_center, gt_tol, reduce, lohi=None):
         with torch.cuda.device(self.device):
             out = dict(top_val=tv, top_idx=ti, D=None, hits=None, n_valid=None, S=S,
                        overflow=self.net.overflow_tensor())
@@ -437,12 +468,14 @@ class StreamingPipeline(InferencePipeline):
                 gt = torch.where(ti[..., 0] >= 0, gt_center, -1)      # warm-up rows: no ground truth
                 out["hits"], out["n_valid"] = ops.recall_counts(ti, S.shape[2] - self.L + 1, gt_center=gt,
                                                                 gt_tol=gt_tol, ns=self.ns)
+                if lohi is not None:
+                    out["hits_lo"], out["hits_hi"] = lohi
         if reduce:
             self._all_reduce_hits(out)
         return out
 
     def push_events(self, t_us, x, y, offsets, t0_us, window_us, Q, roi_x0=0, roi_y0=0, gt_center=None, gt_tol=0,
-                    reduce=True, streams=None):
+                    reduce=True, streams=None, bounds=False):
         """`push` fed from raw events: the next Q windows of every stream, window q of stream b covering
         [t0_us[b] + q * window_us, + window_us) of its events [offsets[b], offsets[b+1]) (as in `step_events`).
         Returns `push`'s dict plus "events_per_window" i32 [B, Q].  With `streams` (as in `push`), offsets / t0_us
@@ -457,14 +490,15 @@ class StreamingPipeline(InferencePipeline):
             if offsets.numel() - 1 != len(ids):
                 raise LensError(f"the push names {len(ids)} streams but offsets describe {offsets.numel() - 1}")
             if not ids:
-                out = self._push_none(int(Q), gt_center, reduce)
+                out = self._push_none(int(Q), gt_center, reduce, bounds)
                 out["events_per_window"] = torch.empty((0, int(Q)), dtype=torch.int32, device=self.device)
                 return out
             self._check_gt(gt_center, int(Q), gt_tol, len(ids))
             streams = ids
         with torch.cuda.device(self.device):
             pooled, n_ev = self._bin_streams(t_us, x, y, offsets, t0_us, window_us, Q, roi_x0, roi_y0)
-            out = self.push(pooled=pooled, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce, streams=streams)
+            out = self.push(pooled=pooled, gt_center=gt_center, gt_tol=gt_tol, reduce=reduce, streams=streams,
+                            bounds=bounds)
         out["events_per_window"] = n_ev
         return out
 
