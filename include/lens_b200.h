@@ -222,6 +222,8 @@ int lens_snn_forward_float(void *handle, const float *x, int B, int steps, float
  *   top_val [B][Qo][N] f32, top_idx [B][Qo][N] i32: the N largest D[b][.][q],
  *           ordered by (value desc, index desc) == np.argsort(kind='stable')[-N:][::-1];
  *           missing entries (N > Po) are -inf / -1.
+ *   Any S is ranked as numpy sorts it: -0.0 ties with +0.0 and every NaN (any sign or payload, and the NaN of
+ *   +inf + -inf in a sum) ties with every other NaN above +inf.  top_val holds such values as +0.0 and 0x7fffffff.
  * L >= 1 (the reference's L == 0 branch returns S itself and is handled by the caller). */
 int lens_seqmatch_topk(const float *S, int B, int Q, int P, int L, int N, float *D_out,
                        float *top_val, int32_t *top_idx, void *stream);
@@ -273,7 +275,7 @@ int lens_recall(const int32_t *top_idx, int B, int Qo, int Po, int N, const uint
  * W per-shard lists of a query are gathered, and the global list is the N best of their union under the
  * same order as lens/src/metrics.py:218 under the deterministic rule (value desc, place index desc).
  *   val, idx [W][M][N] device (idx = GLOBAL place index, -1 = empty slot), M = streams * queries,
- *   out_val, out_idx [M][N] device.  W * N <= 512.                                                       */
+ *   out_val, out_idx [M][N] device.  W * N <= 512.  Non-finite values rank as in lens_seqmatch_topk.       */
 int lens_topn_merge(const float *val, const int32_t *idx, int W, int64_t M, int N, float *out_val,
                     int32_t *out_idx, void *stream);
 
@@ -282,7 +284,8 @@ int lens_topn_merge(const float *val, const int32_t *idx, int W, int64_t M, int 
  *   lo [n_ns] i64 device, ACCUMULATED: queries that hit in the top ns[i] whatever the order,
  *   hi [n_ns] i64 device, ACCUMULATED: queries that hit for some order,
  *   n_valid [1] i64 device, ACCUMULATED: queries with at least one positive (metrics.py:214-216).
- * D, GT [Po][Qo] (rows = database, the matrices recallAtK receives), ns host ints ascending.          */
+ * D, GT [Po][Qo] (rows = database, the matrices recallAtK receives), ns host ints ascending.  Ties as numpy's sort
+ * sees them: -0.0 == +0.0, and all NaNs are one tie class above +inf.                                           */
 int lens_recall_bounds(const float *D, const uint8_t *GT, int Po, int Qo, const int *ns, int n_ns,
                        int64_t *lo, int64_t *hi, int64_t *n_valid, void *stream);
 
@@ -327,14 +330,15 @@ int lens_seq_recall_bounds_stream_ids(const float *S, int n, int Q, int P, int L
  * row attaining the maximum (np.argmax); thresholds are np.linspace(max, min, n_thresh) over the best
  * similarities, evaluated like numpy (>= 2.0) in the dtype of the caller's matrix: thresh_f64 = 0 for a
  * float32 matrix (float32 arithmetic and comparison), 1 for float64, integer or bool matrices (float64;
- * exact when every value is representable in float32, the type S is read in).
+ * exact when every value is representable in float32, the type S is read in).  NaN as in numpy: a column's best
+ * match is its first NaN, and one NaN best makes max and min NaN, so every threshold is NaN and tp = fp = 0.
  *   tp, fp [n_thresh] i64 device: true / false positives with best >= threshold
  *   gtp    [1] i64 device: number of queries that have a positive at all (GT.any(0))             */
 int lens_pr_counts(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
                    int64_t *fp, int64_t *gtp, void *stream, int thresh_f64);
 /* The same for matching='multi' (lens/src/metrics.py:63-91): every entry of S counts, thresholds are
  * np.linspace(S.max(), S.min(), n_thresh) (thresh_f64 as above), gtp = count_nonzero(GT).  tp, fp, gtp are
- * overwritten.                                                                                              */
+ * overwritten.  One NaN in S makes every threshold NaN (tp = fp = 0), as numpy's max / min do.               */
 int lens_pr_counts_multi(const float *S, const uint8_t *GT, int Po, int Qo, int n_thresh, int64_t *tp,
                          int64_t *fp, int64_t *gtp, void *stream, int thresh_f64);
 

@@ -10,7 +10,7 @@
 // (spike counts), exact in fp32 in any order; the one division is IEEE (__fdiv_rn),
 // like numpy's float32 / int.  Selection order is (value desc, index desc) -- the
 // order np.argsort(kind='stable')[-N:][::-1] produces -- implemented as a 64-bit max
-// over keys (orderable(value) << 32 | index).
+// over keys (rank key(value) << 32 | index), NaN and signed zeros included (f32_rank_key).
 #include "common.cuh"
 
 #include <algorithm>
@@ -31,6 +31,15 @@ __device__ __forceinline__ uint32_t f32_orderable(float v)
 __device__ __forceinline__ float f32_from_orderable(uint32_t u)
 {
     return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
+}
+
+// numpy's sort order as a key, for matrices a caller may fill with anything: -0.0 ranks as +0.0 (equal values tie)
+// and every NaN, whatever its sign and payload, as one value above +inf (np.sort puts NaNs last).  The key of a NaN
+// decodes (f32_from_orderable) to 0x7fffffff; no value has the key 0, which marks an empty top-N slot.  Finite
+// non-negative sums (spike counts) get the key f32_orderable gives them.
+__device__ __forceinline__ uint32_t f32_rank_key(float v)
+{
+    return isnan(v) ? 0xffffffffu : f32_orderable(__fadd_rn(v, 0.0f));
 }
 
 // One top-N slot from its key (0 = empty slot: -inf / -1).
@@ -112,7 +121,7 @@ seqmatch_topk_kernel(const float *__restrict__ S, int Q, int P, int L, int N,
             for (int j = 0; j < L; ++j) acc += __ldg(Sb + (size_t)(q + j) * P + (r + j));
             const float d = __fdiv_rn(acc, fl);
             if (D_out) D_out[((size_t)b * Po + r) * Qo + q] = d;
-            cand[i] = ((unsigned long long)f32_orderable(d) << 32) | (uint32_t)r;
+            cand[i] = ((unsigned long long)f32_rank_key(d) << 32) | (uint32_t)r;
         }
         __syncthreads();
         cta_merge_chunk(cand, best, next_best, warp_best, s_winner, nr, N, tid, lane, warp);
@@ -212,7 +221,7 @@ seqmatch_topk_warp_kernel(const float *__restrict__ S, long long n_queries, int 
                 if (r < Po) {
                     const float d = __fdiv_rn(acc[u], fl);
                     if (D_out) D_out[((size_t)b * Po_all + r) * Qo + q] = d;
-                    key = ((unsigned long long)f32_orderable(d) << 32) | (uint32_t)r;
+                    key = ((unsigned long long)f32_rank_key(d) << 32) | (uint32_t)r;
                 }
                 const unsigned long long kth = shfl_u64(best, 31);          // current 32nd largest
                 if (!__any_sync(0xffffffffu, key > kth)) continue;          // nothing in this batch can enter
@@ -477,7 +486,7 @@ __global__ void __launch_bounds__(256) topn_merge_kernel(const float *__restrict
             const int w = c / N, n = c - w * N;
             const size_t o = ((size_t)w * M + m) * N + n;
             const int32_t i = idx[o];
-            if (i >= 0) key[s] = ((unsigned long long)f32_orderable(val[o]) << 32) | (uint32_t)i;
+            if (i >= 0) key[s] = ((unsigned long long)f32_rank_key(val[o]) << 32) | (uint32_t)i;
         }
     }
     for (int n = 0; n < N; ++n) {
@@ -583,26 +592,27 @@ __global__ void __launch_bounds__(256) recall_bounds_kernel(BoundsParams p)
     for (int r = lane; r < p.Po; r += 32) any |= p.GT[(size_t)r * p.Qo + q] != 0;
     if (!__any_sync(0xffffffffu, any)) return;                   // metrics.py:214-216: no positive, dropped
     const int kmax = p.ns[p.n_ns - 1];
-    float cur = INFINITY;
+    // the levels are the distinct rank keys (f32_rank_key: all NaNs one level above +inf, -0.0 == +0.0), walked
+    // from the top; no value has the key 0, so m = 0 below means that no entry is left
+    unsigned long long cur = 1ull << 32;                          // above every key
     int g = 0, gpos = 0, next_k = 0;                              // next_k: first K not decided yet
     unsigned lo_mask = 0u, hi_mask = 0u;
     while (next_k < p.n_ns) {
-        // largest value strictly below `cur`, its multiplicity and its positives
-        float m = -INFINITY;
+        // largest key strictly below `cur`, its multiplicity and its positives
+        unsigned m = 0u;
         for (int r = lane; r < p.Po; r += 32) {
-            const float v = p.D[(size_t)r * p.Qo + q];
-            if (v < cur) m = fmaxf(m, v);
+            const unsigned k = f32_rank_key(p.D[(size_t)r * p.Qo + q]);
+            if (k < cur) m = max(m, k);
         }
-        for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+        m = __reduce_max_sync(0xffffffffu, m);
         int c = 0, cpos = 0;
         for (int r = lane; r < p.Po; r += 32) {
-            const float v = p.D[(size_t)r * p.Qo + q];
-            if (v == m && v < cur) { ++c; cpos += p.GT[(size_t)r * p.Qo + q] != 0; }
+            if (f32_rank_key(p.D[(size_t)r * p.Qo + q]) == m) { ++c; cpos += p.GT[(size_t)r * p.Qo + q] != 0; }
         }
         c = __reduce_add_sync(0xffffffffu, c);
         cpos = __reduce_add_sync(0xffffffffu, cpos);
         if (c == 0) {
-            // the column is exhausted (K > Po, or only NaNs are left): everything ranked so far is certain
+            // the column is exhausted (K > Po): everything ranked so far is certain
             for (; next_k < p.n_ns; ++next_k)
                 if (gpos > 0) { lo_mask |= 1u << next_k; hi_mask |= 1u << next_k; }
             break;
@@ -664,18 +674,21 @@ __global__ void __launch_bounds__(256) pr_counts_kernel(const float *__restrict_
     __syncthreads();
     float vmax = -INFINITY, vmin = INFINITY;
     unsigned int my_gtp = 0;
+    bool my_nan = false;
     for (int q = threadIdx.x; q < Qo; q += blockDim.x) {
         float best = -INFINITY;
         int arg = 0;
         bool any = false;
         for (int r = 0; r < Po; ++r) {
             const float v = S[(size_t)r * Qo + q];
-            if (v > best) { best = v; arg = r; }             // strict: first maximum wins (np.argmax)
+            // strict: the first maximum wins, and the first NaN beats everything (np.argmax / np.max)
+            if (v > best || (isnan(v) && !isnan(best))) { best = v; arg = r; }
             any |= GT[(size_t)r * Qo + q] != 0;
         }
         s_best[q] = best;
         s_hit[q] = GT[(size_t)arg * Qo + q] != 0;
         my_gtp += any;
+        my_nan |= isnan(best);
         vmax = fmaxf(vmax, best); vmin = fminf(vmin, best);
     }
     for (int o = 16; o > 0; o >>= 1) {
@@ -684,8 +697,9 @@ __global__ void __launch_bounds__(256) pr_counts_kernel(const float *__restrict_
         my_gtp += __shfl_xor_sync(0xffffffffu, my_gtp, o);
     }
     if ((threadIdx.x & 31) == 0) { s_max[threadIdx.x >> 5] = vmax; s_min[threadIdx.x >> 5] = vmin; atomicAdd(&s_gtp, my_gtp); }
-    __syncthreads();
+    const bool any_nan = __syncthreads_or(my_nan);
     for (int i = 0; i < 8; ++i) { vmax = fmaxf(vmax, s_max[i]); vmin = fminf(vmin, s_min[i]); }
+    if (any_nan) vmax = vmin = __int_as_float(0x7fffffff);     // np.max / np.min of the best values: NaN
     for (int i = threadIdx.x; i < n_thresh; i += blockDim.x) {
         const double t = pr_threshold(i, n_thresh, vmax, vmin, thresh_f64 != 0);
         unsigned long long a = 0, b = 0;
@@ -729,7 +743,10 @@ __global__ void __launch_bounds__(256) pr_multi_counts_kernel(const float *__res
                                                               unsigned long long *__restrict__ fp)
 {
     const int i = blockIdx.x;
-    const double t = pr_threshold(i, n_thresh, f32_from_orderable(mm[0]), f32_from_orderable(mm[1]), thresh_f64 != 0);
+    // np.max and np.min are NaN as soon as S holds a NaN.  A NaN is one of the two extremes (above +inf or below -inf by
+    // its sign bit); as the minimum it makes every threshold NaN by itself, as the maximum it needs this.
+    const float vmax = f32_from_orderable(mm[0]), vmin = isnan(vmax) ? vmax : f32_from_orderable(mm[1]);
+    const double t = pr_threshold(i, n_thresh, vmax, vmin, thresh_f64 != 0);
     const long long per = ceil_div64(n, gridDim.y), e0 = per * blockIdx.y, e1 = min(n, e0 + per);
     unsigned long long a = 0, b = 0;
     for (long long e = e0 + threadIdx.x; e < e1; e += blockDim.x)
